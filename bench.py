@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--scaling weak|strong] [--workload c5|c4] [--impl reference]
     torchrun --nproc-per-node N ... bench.py --gpus N --steps K --warmup W      (N > 1: one process per GPU)
     python bench.py --gpus N --single-process                                   (N > 1: one host thread drives N GPUs)
+    python bench.py ... --dump-outputs DIR      (DIR/tnonlin.npy: the smoothed field of the last timed step, seeded sample)
 
 Workload (BASELINE.json configs[4], SURVEY 8(d) "c5"): synthetic semi-structured triangle mesh, kp = 4 (256 parents per
 super-triangle), n_split = 8 -> 16 777 216 P1 DG elements = 50.3 M DOFs.  Weak scaling (default): every GPU holds one
@@ -29,8 +30,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark leaves the source tree untouched (it may be read-only)
 
 KP, NSMOOTH = 4, 4
+DUMP_VALUES = 1 << 22                # float64 values --dump-outputs writes per run (32 MB)
 NSPLIT_OF = {"c5": 8, "c4": 7}
 BYTES_PER_DOF_JACOBI = 24.0      # read T, read b, write T' (SURVEY 8(d))
 METRIC = "DG DOF-updates/s per smoother sweep"
@@ -238,6 +241,17 @@ def seeded_parent_field(gids, C_children, seed):
     return out
 
 
+def dump_sample(field, nvalues):
+    """The whole field when it has at most nvalues entries, else the entries at a fixed, seeded set of flat indices
+    (sorted, depending only on the field size), so that two builds can be compared value for value."""
+    flat = field.reshape(-1)
+    if flat.size <= nvalues:
+        return flat.copy()
+    keep = np.zeros(flat.size, bool)
+    keep[np.random.Generator(np.random.MT19937(4242)).integers(0, flat.size, nvalues)] = True
+    return flat[keep]
+
+
 def parity_check(pkg, orc, g, mesh, first, U_local, nsplit, gather, part_first, nshare):
     """One Jacobi sweep from a seeded field: the parents along the GPU cuts (or the first 8 parents on one GPU) and their
     halo strips against the CPU oracle run on those parents plus all their neighbours."""
@@ -295,7 +309,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-vcycle", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the other kernels of the path (GS, residual, unstructured)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the level-1 field after the last timed step to DIR/tnonlin.npy (float64; a fixed, seeded "
+                         "sample of at most 32 MB; with several ranks one file per rank, tnonlin_rank<R>.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -305,6 +324,8 @@ def main():
         import faulthandler
         faulthandler.dump_traceback_later(wd, exit=True)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the CUDA path, not to --impl reference")
         run_reference(args, rank)
         return
     single = args.single_process and world == 1 and args.gpus > 1
@@ -416,6 +437,11 @@ def main():
     kern_ms, kern_n = g.profile_read()
     g.profile(False)
     value = ndof_job * NSMOOTH * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        # what a caller of the timed smoother receives: the swept level-1 field (this rank's parents)
+        out = dump_sample(g.download(pkg.TNONLIN, 1), DUMP_VALUES // world)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "tnonlin.npy" if world == 1 else f"tnonlin_rank{rank}.npy"), out)
 
     # ---- end to end through the C ABI with HOST buffers ---------------------------------------------------
     # (a) the headline e2e: one reference-facing smoother call per step with pinned HOST fields - upload of the field,
