@@ -199,6 +199,15 @@ int pamg_halo_peer_info(const pamg_handle* h, int idx, int* peer_part, int* nfac
 int pamg_set_unstructured(pamg_handle* h, int E, const double* X, const int32_t* neig, const int32_t* fneig);
 int pamg_unstr_upload(pamg_handle* h, const double* tnew /* (3,E) */);
 int pamg_unstr_download(pamg_handle* h, double* tnew);
+/* u_ele(2,3,E) of transport_tri_unstr.F90 in the reference's layout: flat index (e*3 + iloc)*2 + d, HOST array.
+ * NULL returns to the uniform velocity.  While a field is set, the u_x, u_y arguments of pamg_explicit_step,
+ * pamg_implicit_assemble(_diffusion) and pamg_unstr_stab are not used: in the reference they only fill u_ele.
+ * Needs pamg_set_unstructured first (else PAMG_ERR_STATE); pamg_set_unstructured clears the field.  Setting or clearing it
+ * makes the assembled operator stale: pamg_implicit_step, _apply, _get_bsr and _set_stab return PAMG_ERR_STATE until the
+ * next pamg_implicit_assemble*.  The face flux takes its upwind choice per Gauss point from the two traces
+ * (income(s) = 1/2 + 1/2 sign(1, -n.(u + u2)/2)); where n.u changes sign along a face, the inflow point's part goes into the
+ * neighbour's columns and the outflow point's into the element's own (HEAD picks one block per face from income(1)). */
+int pamg_unstr_set_velocity(pamg_handle* h, const double* u_ele);
 /* ntime x nits nonlinear iterations; njac_its Jacobi iterations on M x = M told + dt rhs, or the exact
  * register-resident local inverse when use_exact_minv != 0 (transport_rect.F90:277-291) */
 int pamg_explicit_step(pamg_handle* h, double dt, double u_x, double u_y, double t_bc, int ntime, int nits,

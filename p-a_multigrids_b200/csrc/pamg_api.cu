@@ -2128,6 +2128,18 @@ int pamg_set_unstructured(pamg_handle* h, int E, const double* X, const int32_t*
   return PAMG_OK;
 }
 
+int pamg_unstr_set_velocity(pamg_handle* h, const double* u_ele) {
+  ON_PART0(h);
+  if (!h) return PAMG_ERR_ARG;
+  if (h->un.E < 1) return fail(h, PAMG_ERR_STATE, "pamg_set_unstructured has not been called");
+  CK(cudaSetDevice(h->device));
+  std::string e;
+  int rc = unstr_set_velocity(h->un, u_ele, h->nsm, h->stream, e);
+  h->launches += u_ele ? 1 : 0;
+  if (rc) return fail(h, rc, e);
+  return PAMG_OK;
+}
+
 int pamg_unstr_upload(pamg_handle* h, const double* tnew) {
   ON_PART0(h);
   if (!h || !tnew || h->un.E < 1) return PAMG_ERR_ARG;
@@ -2253,8 +2265,10 @@ int pamg_unstr_stab(pamg_handle* h, const double* told, double dt, double u_x, d
   StabArgs sa;
   sa.X = h->un.X; sa.tnew = h->un.T[h->un.cur]; sa.told = d_old; sa.diff_coe = d_out + E * 9; sa.stab = d_out; sa.diag0 = nullptr;
   sa.val = nullptr; sa.dinv = nullptr; sa.dt = dt; sa.ux = u_x; sa.uy = u_y; sa.ld = h->un.ld; sa.E = h->un.E; sa.mode = 0;
+  sa.U = h->un.U;
   const int grid = std::max(1, std::min((h->un.E + TPB - 1) / TPB, h->nsm * 8));
-  k_unstr_stab<<<grid, TPB, 0, h->stream>>>(sa);
+  if (h->un.U) k_unstr_stab<true><<<grid, TPB, 0, h->stream>>>(sa);
+  else k_unstr_stab<false><<<grid, TPB, 0, h->stream>>>(sa);
   h->launches++;
   cudaError_t e1 = cudaGetLastError();
   if (stab) cudaMemcpyAsync(stab, d_out, E * 9 * sizeof(double), cudaMemcpyDeviceToHost, h->stream);

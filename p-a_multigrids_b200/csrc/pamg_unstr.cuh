@@ -31,6 +31,8 @@ struct UnstrDev {
                               // to DRAM in k_assemble_bsr (lines evicted half written); with an odd number of lines between
                               // planes the streams spread over the sets
   double* X = nullptr;        // [6][ld] planes x1, y1, x2, y2, x3, y3
+  double* U = nullptr;        // [6][ld] planes u1x, u1y, u2x, u2y, u3x, u3y of the nodal velocity field u_ele(2,3,E)
+                              //         (transport_tri_unstr.F90:504-511); null = the uniform velocity of the call
   int32_t* neig = nullptr;    // [3][ld] 1-based, 0 = boundary
   int32_t* nside = nullptr;   // [3][ld] fNeig | swap<<2 (swap: geometric pairing differs from get_unstr_sn2)
   double* pen = nullptr;      // [3][ld] (L/2) / dx of the diffusion face term: half the face length over the centroid distance
@@ -56,6 +58,7 @@ struct UnstrDev {
   double* xfer = nullptr; size_t xfer_bytes = 0;   // staging for the [E][..] <-> [..][E] conversions at the ABI
   int occ_explicit = 0, occ_assemble = 0, occ_spmv = 0, occ_apply = 0, occ_stab = 0, occ_kry[6] = {0, 0, 0, 0, 0, 0};   // resident CTAs
                               // per SM of the streaming kernels (this device)
+  int occ_explicit_f = 0, occ_assemble_f = 0, occ_stab_f = 0;   // the same for the velocity-field instantiations
 };
 
 inline size_t plane_stride(int E) {
@@ -114,12 +117,47 @@ __device__ __forceinline__ double face_flux(const TriEdges& g, int l1, int l2, i
   return (ey * mx - ex * my < 0.0) ? -c : c;
 }
 
+// ---- nodal velocity field u_ele(2,3,E) ------------------------------------------------------------------------------
+// Own velocity: six coalesced plane loads.  The neighbour's velocity at its two face nodes (m1, m2) is a gather through L2
+// like its T.  Gauss point s of a face weighs (l1, l2) with sn(s, :) = (al, be) at s = 0 and (be, al) at s = 1.
+__device__ __forceinline__ void load_vel(const double* __restrict__ U, size_t ld, size_t e, double ux[3], double uy[3]) {
+#pragma unroll
+  for (int l = 0; l < 3; ++l) { ux[l] = __ldg(U + (size_t)(2 * l) * ld + e); uy[l] = __ldg(U + (size_t)(2 * l + 1) * ld + e); }
+}
+// Neighbour trace velocity at the face nodes, as the (m1, m2) pair of its T: (x, y) of node m1, then of node m2.  Nside = 0
+// (sn2 = 0): zero.  npos = 0 with Nside >= 1: flagged by own = true - the trace is the element's own (sum2 u in the
+// uniform form, u_bc = u_ele in trans_rec).
+struct FaceVel2 { double ax, ay, bx, by; bool own; };
+__device__ __forceinline__ FaceVel2 neighbour_vel(const double* __restrict__ U, size_t ld, int q, int ns, int m1, int m2) {
+  FaceVel2 v = {0.0, 0.0, 0.0, 0.0, false};
+  if (ns >= 1 && q != 0) {
+    const size_t n = (size_t)(q - 1);
+    v.ax = __ldg(U + (size_t)(2 * m1) * ld + n); v.ay = __ldg(U + (size_t)(2 * m1 + 1) * ld + n);
+    v.bx = __ldg(U + (size_t)(2 * m2) * ld + n); v.by = __ldg(U + (size_t)(2 * m2 + 1) * ld + n);
+  } else if (ns >= 1) {
+    v.own = true;
+  }
+  return v;
+}
+// sdetwei n.u of both traces at Gauss point s and the upwind choice income(s) = 1/2 + 1/2 sign(1, -n.(us + us2)/2), the
+// sign taken from the element's own trace alone where sn2 = 0
+struct GaussFlux { double c, c2; bool in; };
+__device__ __forceinline__ GaussFlux gauss_flux(const TriEdges& g, int l1, int l2, int l3, double a1, double a2,
+                                                const double ux[3], const double uy[3], const FaceVel2& v, int ns) {
+  GaussFlux r;
+  r.c = face_flux(g, l1, l2, l3, a1 * ux[l1] + a2 * ux[l2], a1 * uy[l1] + a2 * uy[l2]);
+  r.c2 = v.own ? r.c : face_flux(g, l1, l2, l3, a1 * v.ax + a2 * v.bx, a1 * v.ay + a2 * v.by);
+  r.in = signbit(-(ns >= 1 ? r.c + r.c2 : r.c)) == 0;
+  return r;
+}
+
 struct UnstrArgs {
   const double* X; const int32_t* neig; const int32_t* nside;
   const double* Tin; const double* told; double* Tout;
   double dt, ux, uy, t_bc;
   size_t ld;
   int E, njac, exact, use_dir;
+  const double* U;   // velocity planes (FIELD instantiation only); last, so the uniform kernel's parameter offsets stay put
 };
 
 // unstr_explicit element loop (transport_tri_unstr.F90:600-791).  One warp = 32 consecutive elements per trip: all the
@@ -137,7 +175,14 @@ struct UnstrArgs {
 #else
 #define ASM_ST(p, v) (*(p) = (v))
 #endif
-__global__ void __launch_bounds__(TPB, PAMG_OCC_EXPLICIT) k_unstr_explicit(UnstrArgs a) {
+// FIELD: the velocity is the nodal field a.U (u_ele); the volume term takes ugi(g) = sum_i n(g,i) u(:,i) at the three
+// Gauss points and every face Gauss point its own upwind choice from the two traces.  The uniform instantiation is the
+// kernel as it was before the field existed.
+#ifndef PAMG_OCC_EXPLICIT_FIELD
+#define PAMG_OCC_EXPLICIT_FIELD 2
+#endif
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OCC_EXPLICIT) k_unstr_explicit(UnstrArgs a) {
   __shared__ double smw[TPB / 32][2][96];
   const double al = 0.78867513459481288, be = 0.21132486540518712;  // sn_orig, ShapFun.F90:1100-1111
   // weights of int sn_c * trace over the face: (2/3, 1/3) -- exact products of the 2-point Gauss rule
@@ -169,6 +214,9 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_EXPLICIT) k_unstr_explicit(Unstr
     // ---- neighbour values paired with sn_orig(:,1), sn_orig(:,2): get_unstr_sn2 (ShapFun_unstruc.F90:205-222),
     // Nside 1 -> nodes (3,1), 2 -> (1,2), 3 -> (2,3); use_dir: the geometric pairing
     double T2a[3], T2b[3];
+    double ux[3], uy[3];
+    FaceVel2 v2[3];
+    if constexpr (FIELD) load_vel(a.U, ld, (size_t)e, ux, uy);
 #pragma unroll
     for (int f = 0; f < 3; ++f) {
       const int ns = enc[f] & 3;
@@ -176,6 +224,9 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_EXPLICIT) k_unstr_explicit(Unstr
       if (a.use_dir && (enc[f] >> 2)) { const int t = m1; m1 = m2; m2 = t; }
       T2a[f] = a.t_bc; T2b[f] = a.t_bc;
       if (ns >= 1 && q[f] != 0) { const double* nb = a.Tin + (size_t)(q[f] - 1) * 3; T2a[f] = __ldg(nb + m1); T2b[f] = __ldg(nb + m2); }
+      // with the neighbour's T, before anything is used: gathered face by face inside the flux loop instead they cost 14 %
+      // more time on a B200 (the gathers then wait one after the other)
+      if constexpr (FIELD) v2[f] = neighbour_vel(a.U, ld, q[f], ns, m1, m2);
     }
 #pragma unroll
     for (int k = 0; k < 3; ++k) { smT[lane + 32 * k] = ra[k]; smO[lane + 32 * k] = rb[k]; }
@@ -185,11 +236,36 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_EXPLICIT) k_unstr_explicit(Unstr
     __syncwarp();
     const double sumT = T[0] + T[1] + T[2];
     double rhs[3];
+    const int L1[3] = {0, 1, 2}, L2[3] = {2, 0, 1}, L3[3] = {1, 2, 0};
+    if constexpr (FIELD) {
+      // sum_g (grad(phi_i) . ugi(g)) T(g) detwei(g), ugi and T(g) at the edge midpoints n(g,:) = (1/2,1/2,0), (0,1/2,1/2), (1/2,0,1/2)
+      double px = 0.0, py = 0.0;
+#pragma unroll
+      for (int gq = 0; gq < 3; ++gq) {
+        const int i0 = gq == 2 ? 0 : gq, i1 = gq == 2 ? 2 : gq + 1;
+        const double tg = 0.5 * (T[i0] + T[i1]);
+        px += 0.5 * (ux[i0] + ux[i1]) * tg; py += 0.5 * (uy[i0] + uy[i1]) * tg;
+      }
+      rhs[0] = g.sgn * (g.D * px - g.C * py) * sixth;
+      rhs[1] = g.sgn * (g.A * py - g.B * px) * sixth;
+      rhs[2] = -(rhs[0] + rhs[1]);
+#pragma unroll
+      for (int f = 0; f < 3; ++f) {
+        const int l1 = L1[f], l2 = L2[f], ns = enc[f] & 3;
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const double a1 = s == 0 ? al : be, a2 = s == 0 ? be : al;
+          const GaussFlux r = gauss_flux(g, l1, l2, L3[f], a1, a2, ux, uy, v2[f], ns);
+          // Nside = 0: c2 = 0, the inflow trace carries nothing (sn2 = 0)
+          const double fl = r.in ? r.c2 * (a1 * T2a[f] + a2 * T2b[f]) : r.c * (a1 * T[l1] + a2 * T[l2]);
+          rhs[l1] -= a1 * fl; rhs[l2] -= a2 * fl;
+        }
+      }
+    } else {
     // (grad(phi_i) . u) (A/3) sum(T)  (:668-672)
     rhs[0] = g.sgn * (g.D * a.ux - g.C * a.uy) * sixth * sumT;
     rhs[1] = g.sgn * (g.A * a.uy - g.B * a.ux) * sixth * sumT;
     rhs[2] = -(rhs[0] + rhs[1]);
-    const int L1[3] = {0, 1, 2}, L2[3] = {2, 0, 1}, L3[3] = {1, 2, 0};
 #pragma unroll
     for (int f = 0; f < 3; ++f) {
       const int l1 = L1[f], l2 = L2[f];
@@ -201,6 +277,7 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_EXPLICIT) k_unstr_explicit(Unstr
       if (in) { const double f2 = has2 ? c : 0.0; ca = f2 * (w2 * T2a[f] + w1 * T2b[f]); cb = f2 * (w1 * T2a[f] + w2 * T2b[f]); }
       else { ca = c * (w2 * T[l1] + w1 * T[l2]); cb = c * (w1 * T[l1] + w2 * T[l2]); }
       rhs[l1] -= ca; rhs[l2] -= cb;                     // :742-746
+    }
     }
     const double area = 0.5 * fabs(g.detj);
     const double m12 = area * (1.0 / 12.0);
@@ -251,7 +328,7 @@ __global__ void __launch_bounds__(TPB) k_from_planes(const Tp* __restrict__ soa,
 }
 
 inline void unstr_free(UnstrDev& u) {
-  cudaFree(u.X); cudaFree(u.neig); cudaFree(u.nside); cudaFree(u.pen); cudaFree(u.T[0]); cudaFree(u.T[1]); cudaFree(u.told);
+  cudaFree(u.X); cudaFree(u.U); cudaFree(u.neig); cudaFree(u.nside); cudaFree(u.pen); cudaFree(u.T[0]); cudaFree(u.T[1]); cudaFree(u.told);
   cudaFree(u.bsr_val); cudaFree(u.bsr_col); cudaFree(u.dinv); cudaFree(u.mdt); cudaFree(u.work); cudaFree(u.dots); cudaFree(u.diag0); cudaFree(u.stab);
   cudaFree(u.xfer);
   if (u.dots_host) cudaFreeHost(u.dots_host);
@@ -336,17 +413,43 @@ inline int unstr_setup(UnstrDev& u, int E, const double* X, const int32_t* neig,
   return PAMG_OK;
 }
 
+// u_ele(2,3,E) in the reference's layout ([E][6] doubles, host) -> 6 planes; null clears the field.  The operator assembled
+// with the previous velocity is stale either way: the implicit entries refuse to run until the next assembly.
+inline int unstr_set_velocity(UnstrDev& u, const double* u_ele, int nsm, cudaStream_t st, std::string& err) {
+  u.assembled = false;
+  u.with_stab = false;
+  if (!u_ele) { cudaFree(u.U); u.U = nullptr; return PAMG_OK; }
+  const size_t E = (size_t)u.E;
+  if (!u.U) UCK(cudaMalloc(&u.U, u.ld * 6 * sizeof(double)));
+  // on any failure below the planes hold no valid field: drop them, so that later calls run the uniform path, not garbage
+  int rc = unstr_xfer(u, E * 6 * sizeof(double), err);
+  if (rc == PAMG_OK) {
+    cudaError_t e1 = cudaMemcpyAsync(u.xfer, u_ele, E * 6 * sizeof(double), cudaMemcpyHostToDevice, st);
+    if (e1 == cudaSuccess) {
+      k_to_planes<double><<<std::max(1, std::min((u.E + TPB - 1) / TPB, nsm * 8)), TPB, 0, st>>>(u.xfer, u.U, 6, u.E, u.ld);
+      e1 = cudaGetLastError();
+    }
+    if (e1 == cudaSuccess) e1 = cudaStreamSynchronize(st);
+    if (e1 != cudaSuccess) { err = std::string("pamg_unstr_set_velocity: ") + cudaGetErrorString(e1); rc = PAMG_ERR_CUDA; }
+  }
+  if (rc != PAMG_OK) { cudaFree(u.U); u.U = nullptr; }
+  return rc;
+}
+
 // time loop of unstr_explicit (:588-795): told = tnew ; nits x { tnew = tnew_nonlin ; element loop }
 inline int unstr_step(UnstrDev& u, double dt, double ux, double uy, double t_bc, int ntime, int nits, int njac,
                       int exact, int use_dir, int nsm, cudaStream_t st, long long& nlaunch, std::string& err) {
-  const int grid = stream_grid(k_unstr_explicit, u.occ_explicit, u.E, nsm);
+  const int grid = u.U ? stream_grid(k_unstr_explicit<true>, u.occ_explicit_f, u.E, nsm)
+                       : stream_grid(k_unstr_explicit<false>, u.occ_explicit, u.E, nsm);
   for (int it = 0; it < ntime; ++it) {
     UCK(cudaMemcpyAsync(u.told, u.T[u.cur], (size_t)u.E * 3 * sizeof(double), cudaMemcpyDeviceToDevice, st));
     for (int k = 0; k < nits; ++k) {
       UnstrArgs a;
       a.X = u.X; a.neig = u.neig; a.nside = u.nside; a.Tin = u.T[u.cur]; a.told = u.told; a.Tout = u.T[u.cur ^ 1];
       a.dt = dt; a.ux = ux; a.uy = uy; a.t_bc = t_bc; a.ld = u.ld; a.E = u.E; a.njac = njac; a.exact = exact; a.use_dir = use_dir;
-      k_unstr_explicit<<<grid, TPB, 0, st>>>(a);
+      a.U = u.U;
+      if (u.U) k_unstr_explicit<true><<<grid, TPB, 0, st>>>(a);
+      else k_unstr_explicit<false><<<grid, TPB, 0, st>>>(a);
       nlaunch++;
       UCK(cudaGetLastError());
       u.cur ^= 1;
@@ -374,9 +477,18 @@ struct BsrArgs {
   double inv24dt, ux, uy, kdiff;
   size_t ld;
   int E, use_dir;
+  const double* U;   // velocity planes (FIELD only)
 };
 
-__global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs a) {
+// FIELD: stiff(i,j) = sum_g (grad(phi_i) . ugi(g)) n(g,j) detwei(g) (no longer the same for every j) and the face flux split per
+// Gauss point: the sn(s,j) part of an outflow point into the own columns, the sn2(s,j) part of an inflow point into the
+// neighbour's.  (HEAD, :339, sends the whole face to one block chosen by income(1); for a uniform velocity both Gauss points
+// agree and the two rules coincide.)
+#ifndef PAMG_OCC_ASSEMBLE_FIELD
+#define PAMG_OCC_ASSEMBLE_FIELD 2
+#endif
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_ASSEMBLE_FIELD : PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs a) {
   const double al = 0.78867513459481288, be = 0.21132486540518712;
   const double w2 = al * al + be * be, w1 = 2.0 * al * be;
   const size_t ld = a.ld;
@@ -395,7 +507,27 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs
     const double adet = fabs(g.detj);
     const double m12 = adet * a.inv24dt;                    // A / (12 dt)
     double d[9];
-    {
+    double ux[3], uy[3];
+    if constexpr (FIELD) {
+      load_vel(a.U, ld, (size_t)e, ux, uy);
+      // a(i,g) = (grad(phi_i) . ugi(g)) A/3 ; stiff(i,j) = sum_g a(i,g) n(g,j): g = 0 holds nodes (0,1), 1 (1,2), 2 (0,2)
+      double gx[3], gy[3];
+#pragma unroll
+      for (int gq = 0; gq < 3; ++gq) {
+        const int i0 = gq == 2 ? 0 : gq, i1 = gq == 2 ? 2 : gq + 1;
+        gx[gq] = 0.5 * (ux[i0] + ux[i1]); gy[gq] = 0.5 * (uy[i0] + uy[i1]);
+      }
+      const double Gx[3] = {g.D, -g.B, g.B - g.D}, Gy[3] = {-g.C, g.A, g.C - g.A};
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        double ag[3];
+#pragma unroll
+        for (int gq = 0; gq < 3; ++gq) ag[gq] = g.sgn * (Gx[i] * gx[gq] + Gy[i] * gy[gq]) * sixth;
+        const double st[3] = {0.5 * (ag[0] + ag[2]), 0.5 * (ag[0] + ag[1]), 0.5 * (ag[1] + ag[2])};
+#pragma unroll
+        for (int j = 0; j < 3; ++j) d[i * 3 + j] = m12 * (i == j ? 2.0 : 1.0) - st[j];
+      }
+    } else {
       // stiff(i,j) = (grad(phi_i) . u) A/3: the same for every j (:281-283)
       double st[3];
       st[0] = g.sgn * (g.D * a.ux - g.C * a.uy) * sixth;
@@ -405,6 +537,8 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs
       for (int i = 0; i < 3; ++i)
 #pragma unroll
         for (int j = 0; j < 3; ++j) d[i * 3 + j] = m12 * (i == j ? 2.0 : 1.0) - st[i];
+    }
+    {
       if (a.kdiff != 0.0) {
         // k A grad(phi_i) . grad(phi_j) = k / (2 |detj|) G_i . G_j with the unnormalised gradients G = (D,-C), (-B,A), -(sum)
         const double kk = a.kdiff * 0.5 / adet;
@@ -427,8 +561,35 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs
       int m1 = (ns == 1) ? 2 : (ns == 2 ? 0 : 1), m2 = (ns == 1) ? 0 : (ns == 2 ? 1 : 2);
       if (a.use_dir && (enc[f] >> 2)) { const int t = m1; m1 = m2; m2 = t; }
       double o11 = 0.0, o12 = 0.0;     // the face block: rows (l1, l2) x columns (m1, m2) = [[o11, o12], [o12, o11]]
+      double o21 = 0.0, o22 = 0.0;     // FIELD: [[o11, o12], [o21, o22]]
       int colf = -1;
-      if (!in) {                       // outflow: own columns
+      if constexpr (FIELD) {
+        const FaceVel2 v2 = neighbour_vel(a.U, ld, q[f], ns, m1, m2);
+        // the own face-node velocities again (L1 hits): not holding all six across the face loop keeps the kernel in 128
+        // registers without spilling
+        double fx[3] = {0.0, 0.0, 0.0}, fy[3] = {0.0, 0.0, 0.0};
+        fx[l1] = __ldg(a.U + (size_t)(2 * l1) * ld + e); fy[l1] = __ldg(a.U + (size_t)(2 * l1 + 1) * ld + e);
+        fx[l2] = __ldg(a.U + (size_t)(2 * l2) * ld + e); fy[l2] = __ldg(a.U + (size_t)(2 * l2 + 1) * ld + e);
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const double a1 = s == 0 ? al : be, a2 = s == 0 ? be : al;
+          const GaussFlux r = gauss_flux(g, l1, l2, L3[f], a1, a2, fx, fy, v2, ns);
+          if (!r.in) {
+            d[l1 * 3 + l1] += r.c * a1 * a1; d[l1 * 3 + l2] += r.c * a1 * a2;
+            d[l2 * 3 + l1] += r.c * a2 * a1; d[l2 * 3 + l2] += r.c * a2 * a2;
+          } else if (ns >= 1) {
+            const double p11 = r.c2 * a1 * a1, p12 = r.c2 * a1 * a2, p21 = r.c2 * a2 * a1, p22 = r.c2 * a2 * a2;
+            if (q[f] != 0) { o11 += p11; o12 += p12; o21 += p21; o22 += p22; colf = q[f] - 1; }
+            else {                     // target_ele == 0: the element's own columns at (m1, m2) (:340-342)
+#pragma unroll
+              for (int j = 0; j < 3; ++j) {
+                d[l1 * 3 + j] += (j == m1) ? p11 : ((j == m2) ? p12 : 0.0);
+                d[l2 * 3 + j] += (j == m1) ? p21 : ((j == m2) ? p22 : 0.0);
+              }
+            }
+          }
+        }
+      } else if (!in) {                // outflow: own columns
         d[l1 * 3 + l1] += c * w2; d[l1 * 3 + l2] += c * w1;
         d[l2 * 3 + l1] += c * w1; d[l2 * 3 + l2] += c * w2;
       } else if (ns >= 1) {            // inflow: the neighbour's columns, its nodes paired as in get_unstr_sn2
@@ -447,7 +608,10 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs
         const double kd = pn[f];
         d[l1 * 3 + l1] += kd * w2; d[l1 * 3 + l2] += kd * w1;
         d[l2 * 3 + l1] += kd * w1; d[l2 * 3 + l2] += kd * w2;
-        if (q[f] != 0 && ns >= 1) { o11 -= kd * w2; o12 -= kd * w1; colf = q[f] - 1; }
+        if (q[f] != 0 && ns >= 1) {
+          o11 -= kd * w2; o12 -= kd * w1; colf = q[f] - 1;
+          if constexpr (FIELD) { o21 -= kd * w1; o22 -= kd * w2; }
+        }
       }
       ASM_ST(a.col + (size_t)(1 + f) * ld + e, colf);
       double* v = a.val + (size_t)((1 + f) * 9) * ld + e;
@@ -457,7 +621,8 @@ __global__ void __launch_bounds__(TPB, PAMG_OCC_ASSEMBLE) k_assemble_bsr(BsrArgs
         for (int j = 0; j < 3; ++j) {
           double x = 0.0;
           if (i == l1) x = (j == m1) ? o11 : ((j == m2) ? o12 : 0.0);
-          if (i == l2) x = (j == m1) ? o12 : ((j == m2) ? o11 : 0.0);
+          if constexpr (FIELD) { if (i == l2) x = (j == m1) ? o21 : ((j == m2) ? o22 : 0.0); }
+          else { if (i == l2) x = (j == m1) ? o12 : ((j == m2) ? o11 : 0.0); }
           ASM_ST(v + (size_t)(i * 3 + j) * ld, x);
         }
     }
@@ -764,8 +929,10 @@ struct StabArgs {
   double dt, ux, uy;
   size_t ld;
   int E, mode;
+  const double* U;   // velocity planes (FIELD only): ugi(g) = sum_l n(g,l) u(:,l)
 };
 
+template <bool FIELD>
 __global__ void __launch_bounds__(TPB) k_unstr_stab(StabArgs a) {
   const double toler = 0.00000000001;
   const size_t E = a.ld;   // plane stride
@@ -786,12 +953,18 @@ __global__ void __launch_bounds__(TPB) k_unstr_stab(StabArgs a) {
     for (int l = 0; l < 3; ++l) { tx += gx[l] * tn[l]; ty += gy[l] * tn[l]; }
     const double g2 = tx * tx + ty * ty;
     const double N[3][3] = {{0.5, 0.5, 0.0}, {0.0, 0.5, 0.5}, {0.5, 0.0, 0.5}};   // n(gi, iloc), ShapFun.F90:1038-1040
+    double ux[3], uy[3];
+    if constexpr (FIELD) load_vel(a.U, E, (size_t)e, ux, uy);
     double dc[3];
 #pragma unroll
     for (int g = 0; g < 3; ++g) {
       double ugx = 0.0, ugy = 0.0, tgi = 0.0, togi = 0.0;
 #pragma unroll
-      for (int l = 0; l < 3; ++l) { ugx += N[g][l] * a.ux; ugy += N[g][l] * a.uy; tgi += N[g][l] * tn[l]; togi += N[g][l] * to[l]; }
+      for (int l = 0; l < 3; ++l) {
+        if constexpr (FIELD) { ugx += N[g][l] * ux[l]; ugy += N[g][l] * uy[l]; }
+        else { ugx += N[g][l] * a.ux; ugy += N[g][l] * a.uy; }
+        tgi += N[g][l] * tn[l]; togi += N[g][l] * to[l];
+      }
       const double rgi = (tgi - togi) / a.dt + (ugx * tx + ugy * ty);
       const double ac = rgi / fmax(toler, g2);
       const double as1 = ac * tx, as2 = ac * ty;
@@ -846,9 +1019,9 @@ inline int implicit_assemble(UnstrDev& u, double dt, double ux, double uy, doubl
   BsrArgs a;
   a.X = u.X; a.neig = u.neig; a.nside = u.nside; a.pen = u.pen; a.val = u.bsr_val; a.col = u.bsr_col; a.dinv = u.dinv;
   a.mdt = u.mdt;
-  a.inv24dt = 1.0 / (24.0 * dt); a.ux = ux; a.uy = uy; a.kdiff = kdiff; a.ld = ld; a.E = u.E; a.use_dir = use_dir;
-  const int grid = stream_grid(k_assemble_bsr, u.occ_assemble, u.E, nsm);
-  k_assemble_bsr<<<grid, TPB, 0, st>>>(a);
+  a.inv24dt = 1.0 / (24.0 * dt); a.ux = ux; a.uy = uy; a.kdiff = kdiff; a.ld = ld; a.E = u.E; a.use_dir = use_dir; a.U = u.U;
+  if (u.U) k_assemble_bsr<true><<<stream_grid(k_assemble_bsr<true>, u.occ_assemble_f, u.E, nsm), TPB, 0, st>>>(a);
+  else k_assemble_bsr<false><<<stream_grid(k_assemble_bsr<false>, u.occ_assemble, u.E, nsm), TPB, 0, st>>>(a);
   nlaunch++;
   UCK(cudaGetLastError());
   u.assembled = true; u.dt = dt; u.ux = ux; u.uy = uy; u.kdiff = kdiff;
@@ -863,7 +1036,8 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
                          int nsm, cudaStream_t st, long long& nlaunch, std::string& err, long long* host_syncs = nullptr) {
   const int E = u.E;
   const long long n = 3LL * E;
-  const int g_apply = stream_grid(k_block_apply, u.occ_apply, E, nsm), g_stab = stream_grid(k_unstr_stab, u.occ_stab, E, nsm);
+  const int g_apply = stream_grid(k_block_apply, u.occ_apply, E, nsm);
+  const int g_stab = u.U ? stream_grid(k_unstr_stab<true>, u.occ_stab_f, E, nsm) : stream_grid(k_unstr_stab<false>, u.occ_stab, E, nsm);
   const int g_init = stream_grid(k_kry_init, u.occ_kry[0], E, nsm), g_p = stream_grid(k_kry_p, u.occ_kry[1], E, nsm);
   const int g_v = stream_grid(k_kry_spmv<0>, u.occ_kry[2], E, nsm), g_s = stream_grid(k_kry_s, u.occ_kry[3], E, nsm);
   const int g_t = stream_grid(k_kry_spmv<1>, u.occ_kry[4], E, nsm), g_x = stream_grid(k_kry_x, u.occ_kry[5], E, nsm);
@@ -888,7 +1062,10 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
         StabArgs sa;
         sa.X = u.X; sa.tnew = a.x; sa.told = u.told; sa.diff_coe = u.stab + (size_t)E * 9; sa.stab = u.stab; sa.diag0 = u.diag0;
         sa.val = u.bsr_val; sa.dinv = u.dinv; sa.dt = u.dt; sa.ux = u.ux; sa.uy = u.uy; sa.ld = u.ld; sa.E = E; sa.mode = 1;
-        k_unstr_stab<<<g_stab, TPB, 0, st>>>(sa); nlaunch++;
+        sa.U = u.U;
+        if (u.U) k_unstr_stab<true><<<g_stab, TPB, 0, st>>>(sa);
+        else k_unstr_stab<false><<<g_stab, TPB, 0, st>>>(sa);
+        nlaunch++;
       }
       UCK(cudaMemcpyAsync(u.dots + KS_MAXIT, &maxit, sizeof(double), cudaMemcpyHostToDevice, st));
       k_kry_init<<<g_init, TPB, 0, st>>>(a, tol); nlaunch++;

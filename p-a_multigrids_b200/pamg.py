@@ -104,6 +104,7 @@ def lib():
         "pamg_halo_peer_count": (ci, [vp, pint]),
         "pamg_halo_peer_info": (ci, [vp, ci, pint, pint]),
         "pamg_set_unstructured": (ci, [vp, ci, _f64, _i32, _i32]),
+        "pamg_unstr_set_velocity": (ci, [vp, vp]),
         "pamg_unstr_upload": (ci, [vp, _f64]),
         "pamg_unstr_download": (ci, [vp, _f64]),
         "pamg_explicit_step": (ci, [vp, cd, cd, cd, cd, ci, ci, ci, ci, ci]),
@@ -473,6 +474,19 @@ class SemiImplicitIterative:
     def set_unstructured(self, mesh):
         self._ck(self.L.pamg_set_unstructured(self.h, mesh.U, mesh.X, mesh.neig, mesh.fneig))
         self._E = mesh.U
+
+    def set_velocity(self, u_ele):
+        """Nodal velocity field u_ele of the unstructured front-ends: shape (E, 3, 2) = (element, node, component), which in C
+        order is the reference's u_ele(2,3,E); None returns to the uniform velocity.  While a field is set, the u_x, u_y
+        arguments of unstr_explicit, implicit_assemble, unstr_stab and unstr_implicit are not used.  Call implicit_assemble
+        again before the implicit entries: the operator of the previous velocity is stale."""
+        if u_ele is None:
+            self._ck(self.L.pamg_unstr_set_velocity(self.h, None))
+            return
+        u = np.ascontiguousarray(u_ele, np.float64)
+        if hasattr(self, "_E") and u.shape != (self._E, 3, 2):      # (without a mesh the library answers ERR_STATE)
+            raise ValueError(f"u_ele must have shape (E, 3, 2) = ({self._E}, 3, 2), got {u.shape}")
+        self._ck(self.L.pamg_unstr_set_velocity(self.h, _ptr(u)))
 
     def unstr_explicit(self, tnew, dt, u_x, u_y, ntime=2, nits=2, njac_its=10, t_bc=0.0, exact_minv=False,
                        use_dir=False):

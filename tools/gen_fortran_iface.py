@@ -20,7 +20,8 @@ SCALAR_OUT = {"n", "U", "ndof", "l2", "linf", "conv", "cycles", "relres", "npeer
               "ntime", "ms", "total_ms", "launches"}
 # array arguments the header documents as optional (NULL allowed): passed as type(c_ptr) so that c_null_ptr can be given
 NULLABLE = {"part_first", "region", "devices", "bc_value", "val", "col", "diff_coe", "stab", "x_all", "analytical", "error",
-            "Minv", "status", "rhs", "x", "hist", "strip_of", "dst_strip", "rev", "hmap", "peers", "counts", "X_out", "bc_kind"}
+            "Minv", "status", "rhs", "x", "hist", "strip_of", "dst_strip", "rev", "hmap", "peers", "counts", "X_out", "bc_kind",
+            "u_ele"}
 NULLABLE_IN = {"pamg_mesh_get": {"X", "neig", "fneig", "dir", "region"},
                "pamg_halo_plan": {"part_first", "strip_of", "dst_strip", "rev", "hmap", "peers", "counts"},
                "pamg_halo_sources": {"part_first"},
@@ -31,7 +32,8 @@ NULLABLE_IN = {"pamg_mesh_get": {"X", "neig", "fneig", "dir", "region"},
                "pamg_unstr_stab": {"diff_coe", "stab"}, "pamg_output_fields": {"x_all", "analytical", "error"},
                "pamg_vcycle_solve": {"cycles", "hist"}, "pamg_residual": {"l2", "linf"},
                "pamg_timestep_host": {"cycles", "relres"}, "pamg_implicit_step": {"iters_total", "relres"},
-               "pamg_halo_peer_info": {"peer_part", "nfaces"}, "pamg_parent_table": {"bc_kind"}}
+               "pamg_halo_peer_info": {"peer_part", "nfaces"}, "pamg_parent_table": {"bc_kind"},
+               "pamg_unstr_set_velocity": {"u_ele"}}
 
 FTYPE = {"int": "integer(c_int)", "int32_t": "integer(c_int32_t)", "int64_t": "integer(c_int64_t)", "double": "real(c_double)",
          "float": "real(c_float)"}
