@@ -102,32 +102,17 @@ struct pamg_handle {
   // both halo-strip buffers of every level in ONE allocation, kept resident in L2 (access-policy window on the stream): the
   // strips are written by one sweep and read by the next, a whole field of streaming traffic later
   double* strip_arena = nullptr; size_t strip_arena_bytes = 0;
-  bool l2_persist = true;       // PAMG_L2_PERSIST=0 disables the window
   std::vector<LevelDev> lev;
   double* partial = nullptr; int npartial = 0; int last_partials = 0;
   double* out3 = nullptr;         // device
   double* out3_host = nullptr;    // pinned
   double* scratch = nullptr; size_t scratch_bytes = 0;  // L2 flush
-  int kernel_mode = 4;  // 4 window kernel (default; 1-D TMA tile ring, all neighbours from shared memory), 1 pipelined 1-D TMA tiles,
-                        // 3 branch-free direct; PAMG_KERNEL=win|tma1d|direct2 (A/B and the families used on small / deep levels)
-  // where a sweep takes the exterior values of faces between local parents from (PAMG_HALO=strips|direct|fused):
-  //   0 strips: one k_halo launch per sweep fills the halo strips (update_overlaps as a kernel of its own);
-  //   1 direct: out-of-place sweeps read the neighbour parent's boundary children straight from the start-of-sweep field;
-  //   2 fused (default): the producer warp of the window kernels writes the strips of the NEXT sweep from the finished
-  //     tiles, so no halo kernel runs between sweeps; kernels without a producer warp (small levels) read direct
-  int halo_mode = 2;
-  long long debug_gap_ns = 0;   // PAMG_DEBUG_GAP_NS (measurement aid): a one-warp kernel that idles this long before every sweep
   // resident CTAs per SM of the shared-memory kernels on THIS device ([face_terms]); set once per handle in configure_kernels
   struct KernelCfg { int win2[2] = {0, 0}, win2x = 0, win[2] = {0, 0}, tma[2] = {0, 0}, gs2 = 0, gs2x = 0, gs = 0, halo = 0; bool done = false; } kc;
   bool capturing = false;   // stream capture in progress: no synchronisation, no per-launch error polling
-  bool use_graph = true;    // replay the V-cycle as a CUDA graph from the second cycle on (PAMG_GRAPH=0 disables)
   struct VcGraph { long long key; std::vector<cudaGraphExec_t> exec; std::vector<long long> launches; };   // one graph per GPU of the group
   std::vector<VcGraph> vc_graphs;   // a few cached V-cycle graphs (solver / sweep counts / buffer parity)
-  bool graph_nccl = true;       // try to capture NCCL calls into the V-cycle graph (PAMG_GRAPH_NCCL=0 disables)
-  bool gs_tma = true;   // coloured GS pass through the TMA tile kernel (PAMG_GS=direct selects the direct kernel)
-  bool win_producer = true;  // window kernel with a producer warp (k_element_win2); PAMG_WIN=barrier: k_element_win
-  bool gs_fused = true; // both colours in one pass (k_gs_win); PAMG_GS=twopass keeps the two in-place passes
-  bool vc_norm_fuse = true;   // Jacobi V-cycles take their convergence norm out of the first pre-sweep of the next cycle (PAMG_VC_NORM=0: a residual evaluation per cycle)
+  bool graph_nccl = true;       // try to capture NCCL calls into the V-cycle graph (cleared when the library refuses)
   // per-kernel timing (element kernels only)
   bool profiling = false;
   std::vector<cudaEvent_t> pev;  // pairs
@@ -162,9 +147,6 @@ struct pamg_handle {
   unsigned long long* p2p_err_dev = nullptr;    // every host synchronisation point can check it without a copy
   uint4* p2p_stage = nullptr;               // flagged receive staging of ALL levels (IPC-exported): per level P2P_SLOTS slots x
   long long p2p_strips = 0;                 //   p2p_strips * 3 * S(level) words, levels one after the other
-  bool xchg_in_kernel = true;               // the producer warps of a sweep send the new cut-face values to the peers themselves and a
-                                            // small unpack launch runs between two sweeps (PAMG_XCHG=halo: k_halo copies, sends and
-                                            // receives between the sweeps instead)
   struct P2PPeer { int slot_at_peer = -1, strip_begin_at_peer = 0; long long recv_strips_at_peer = 0; uint4* stage = nullptr; };
   std::vector<P2PPeer> p2p_peers;      // same order as plan.peers
   std::vector<void*> p2p_opened;       // IPC mappings to close
@@ -563,17 +545,17 @@ int launch_halo(pamg_handle* h, int level, int what) {
 int ensure_strips(pamg_handle* h, int level, bool all = true) {
   LevelDev& L = h->lev[level - 1];
   if (!h->p.face_terms) return PAMG_OK;
-  if ((all || h->halo_mode == 0) && !L.strips_valid) return launch_halo(h, level, 3);
+  if (all && !L.strips_valid) return launch_halo(h, level, 3);
   if (L.cut_valid) return PAMG_OK;
   // the values a sweep's producer warps sent are waiting in the staging buffer: unpack them; else a full exchange
   return launch_halo(h, level, (L.stage_valid && h->p2p_ready) ? 4 : 2);
 }
 
-// the producer warps of this level's sweep kernel can send the cut-face values themselves
-bool xchg_kernel(const pamg_handle* h, const LevelDev& L) {
-  return h->xchg_in_kernel && h->p2p_ready && L.xsend && !h->plan.peers.empty() && h->p.face_terms &&
-         h->kernel_mode == 4 && h->win_producer && L.s >= 6 && L.s <= 8;
-}
+// the sweeps of this level run the window kernels with a producer warp (k_element_win2, k_gs_win2; with face terms the
+// producer warp also writes the next sweep's strips and sends the cut-face values).  Below s = 6 a parent has fewer than
+// 8 tiles, too few for k_element_win2's double-buffered per-parent coefficients; above s = 8 a row (up to 2^(s+1) - 1
+// children, the reach of a vertical neighbour) no longer fits the 8-tile ring.
+bool producer_level(const LevelDev& L) { return L.s >= 6 && L.s <= 8; }
 
 int add_old_time_terms(pamg_handle* h);
 
@@ -615,7 +597,8 @@ int configure_face(pamg_handle* h) {
   if ((rc = configure_one(h, k_element_win<MODE_JACOBI, FACE>, TPB, WIN_SMEM_BYTES, h->kc.win[f]))) return rc;
   if ((rc = configure_one(h, k_element_win<MODE_RESID, FACE>, TPB, WIN_SMEM_BYTES, dummy))) return rc;
   if ((rc = configure_one(h, k_element_win<MODE_RICH, FACE>, TPB, WIN_SMEM_BYTES, dummy))) return rc;
-  if ((rc = configure_one(h, k_element_win<MODE_GS, FACE>, TPB, WIN_SMEM_BYTES, dummy))) return rc;
+  // (the in-place GS pass runs with face terms only on s >= 9, in k_element_tma)
+  if (!FACE && (rc = configure_one(h, k_element_win<MODE_GS, false>, TPB, WIN_SMEM_BYTES, dummy))) return rc;
   if ((rc = configure_one(h, k_element_tma<MODE_JACOBI, FACE>, TPB, TMA_SMEM_BYTES, h->kc.tma[f]))) return rc;
   if ((rc = configure_one(h, k_element_tma<MODE_RESID, FACE>, TPB, TMA_SMEM_BYTES, dummy))) return rc;
   if ((rc = configure_one(h, k_element_tma<MODE_RICH, FACE>, TPB, TMA_SMEM_BYTES, dummy))) return rc;
@@ -646,7 +629,6 @@ int configure_kernels(pamg_handle* h) {
   CK(cudaFuncGetAttributes(&fa, k_fill));
   CK(cudaFuncGetAttributes(&fa, k_push));
   CK(cudaFuncGetAttributes(&fa, k_wait_flags));
-  CK(cudaFuncGetAttributes(&fa, k_spin));
   CK(cudaFuncGetAttributes(&fa, k_output_fields));
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_JACOBI, true>));
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_JACOBI, false>));
@@ -654,16 +636,9 @@ int configure_kernels(pamg_handle* h) {
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_RESID, false>));
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_RICH, true>));
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_RICH, false>));
-  CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_GS, true>));
   CK(cudaFuncGetAttributes(&fa, k_element_direct2<MODE_GS, false>));
   h->kc.done = true;
   return PAMG_OK;
-}
-
-// whether a sweep of this solver on this level runs a window kernel with a producer warp (which can write the next strips)
-bool producer_kernel(const pamg_handle* h, const LevelDev& L, bool gs) {
-  if (!(h->kernel_mode == 4 && h->win_producer && L.s >= 6 && L.s <= 8)) return false;
-  return !gs || (h->gs_fused && h->p.face_terms);
 }
 
 // use_strips: every strip of the level holds the start-of-sweep values (else: neighbour-field reads where possible);
@@ -685,9 +660,12 @@ int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout,
   a.colour = colour; a.partial_off = 0;
   if (ov) { a.ovl = ov->ovl; a.pc = ov->pc; a.rsign = ov->rsign; }
   const int f = h->p.face_terms ? 1 : 0;
+  // the in-place GS pass runs with face terms only on s >= 9 (do_smooth), so k_element_win and k_element_direct2 have
+  // no such instantiation
+  constexpr bool FACE_OK = MODE != MODE_GS;
   const bool prof = !ov && h->profiling && h->pev_used + 2 <= (int)h->pev.size();
   if (prof) CK(cudaEventRecord(h->pev[h->pev_used], h->stream));
-  if (MODE != MODE_GS && h->kernel_mode == 4 && h->win_producer && L.s >= 6 && L.s <= 8) {
+  if (MODE != MODE_GS && producer_level(L)) {
     // window kernel with a producer warp (no CTA-wide barrier between tiles)
     auto kern = xchg ? k_element_win2<MODE == MODE_RESID ? MODE_JACOBI : MODE, true, true>
                      : h->p.face_terms ? k_element_win2<MODE, true> : k_element_win2<MODE, false>;
@@ -697,14 +675,14 @@ int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout,
     const int tgrid = (int)std::max(1ll, std::min(L.nelem / TPB, (long long)h->nsm * (xchg ? h->kc.win2x : h->kc.win2[f])));
     kern<<<tgrid, WIN2_THREADS, WIN_SMEM_BYTES, h->stream>>>(a);
     if (MODE == MODE_RESID || norm) h->last_partials = tgrid;
-  } else if ((MODE != MODE_GS || h->gs_tma) && h->kernel_mode == 4 && L.C >= TPB && L.s <= 8) {
+  } else if (L.C >= TPB && L.s <= 8) {
     // (a vertical neighbour is up to 2^(s+1) children away: the 8-tile ring covers s <= 8)
     // window kernel: ring of 8 field tiles in shared memory, every neighbour value read from it
-    auto kern = h->p.face_terms ? k_element_win<MODE, true> : k_element_win<MODE, false>;
+    auto kern = h->p.face_terms && FACE_OK ? k_element_win<MODE, FACE_OK> : k_element_win<MODE, false>;
     const int tgrid = (int)std::max(1ll, std::min(L.nelem / TPB, (long long)h->nsm * h->kc.win[f]));
     kern<<<tgrid, TPB, WIN_SMEM_BYTES, h->stream>>>(a);
     if (MODE == MODE_RESID) h->last_partials = tgrid;
-  } else if ((MODE != MODE_GS || h->gs_tma) && (h->kernel_mode == 1 || h->kernel_mode == 4) && L.C >= TPB) {
+  } else if (L.C >= TPB) {
     // 1-D TMA tiles: contiguous 6 KB spans through shared memory; contiguous tile ranges per CTA, one wave of resident CTAs
     auto kern = h->p.face_terms ? k_element_tma<MODE, true> : k_element_tma<MODE, false>;
     const int tgrid = (int)std::max(1ll, std::min((L.nelem + TPB - 1) / TPB, (long long)h->nsm * h->kc.tma[f]));
@@ -713,7 +691,7 @@ int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout,
   } else {
     // branch-free direct kernel (all loads of a child in flight at once): levels with fewer than 256 children per parent
     if (MODE == MODE_RESID) h->last_partials = grid;
-    if (h->p.face_terms) k_element_direct2<MODE, true><<<grid, TPB, 0, h->stream>>>(a);
+    if (h->p.face_terms && FACE_OK) k_element_direct2<MODE, FACE_OK><<<grid, TPB, 0, h->stream>>>(a);
     else k_element_direct2<MODE, false><<<grid, TPB, 0, h->stream>>>(a);
   }
   if (prof) { CK(cudaEventRecord(h->pev[h->pev_used + 1], h->stream)); h->pev_used += 2; }
@@ -767,15 +745,9 @@ int add_old_time_terms(pamg_handle* h) {
 
 // coloured Gauss-Seidel sweep in one pass (k_gs_win / k_gs_win2), out of place
 // small levels (a CTA holds whole parents): both colours in one launch of k_gs_small
-bool gs_small_ok(const pamg_handle* h, const LevelDev& L) {
-  return h->gs_fused && h->kernel_mode == 4 && h->p.face_terms && L.C <= TPB;
-}
-bool gs_fused_ok(const pamg_handle* h, const LevelDev& L) {
-  if (gs_small_ok(h, L)) return true;
-  return h->gs_fused && h->kernel_mode == 4 && h->p.face_terms && L.C >= TPB && L.s <= 8;
-}
+bool gs_small_ok(const pamg_handle* h, const LevelDev& L) { return h->p.face_terms && L.C <= TPB; }
 
-int launch_gs_fused(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, bool use_strips, bool write_next, bool xchg) {
+int launch_gs_one_pass(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, bool use_strips, bool write_next, bool xchg) {
   ElemArgs a;
   a.xsend = L.xsend; a.xsync = h->p2p_sync ? h->p2p_sync + (size_t)(&L - h->lev.data()) * P2P_WORDS : nullptr;
   a.Tin = Tin; a.Tout = Tout; a.rhs = L.rhs; a.ovl = L.ovlb[L.ovl_cur]; a.pc = L.pc; a.strip_of = h->strip_of; a.hmap = h->hmap;
@@ -791,7 +763,7 @@ int launch_gs_fused(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout
     CK(cudaGetLastError());
     return PAMG_OK;
   }
-  const bool producer = h->win_producer && L.s >= 6;
+  const bool producer = producer_level(L);
   const int resident = producer ? (xchg ? h->kc.gs2x : h->kc.gs2) : h->kc.gs;
   const bool prof = h->profiling && h->pev_used + 2 <= (int)h->pev.size();
   if (prof) CK(cudaEventRecord(h->pev[h->pev_used], h->stream));
@@ -806,9 +778,7 @@ int launch_gs_fused(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout
 }
 
 // a Jacobi sweep of this level can hand out the residual norms of the iterate it starts from (k_element_win2<.., NORM>)
-bool norm_fusable(const pamg_handle* h, const LevelDev& L) {
-  return h->p.face_terms && h->kernel_mode == 4 && h->win_producer && L.s >= 6 && L.s <= 8;
-}
+bool norm_fusable(const pamg_handle* h, const LevelDev& L) { return h->p.face_terms && producer_level(L); }
 
 // norm_first: the first sweep (Jacobi on a norm_fusable level) also leaves the partial sums of the residual norms
 int do_smooth(pamg_handle* h, int level, int solver, int nsweeps, bool norm_first = false) {
@@ -821,14 +791,14 @@ int do_smooth(pamg_handle* h, int level, int solver, int nsweeps, bool norm_firs
     // the previous sweep's producer warps or by k_halo), or the sweep reads its neighbours' field directly.  Faces cut
     // by the GPU partition always go through their strips (the exchange step).
     L.tnew_alias = true;
-    if (h->debug_gap_ns > 0) { k_spin<<<1, 32, 0, h->stream>>>(h->debug_gap_ns); }   // experiment: idle time between sweeps
     const bool gs = solver == 3 || solver == 4;
-    const bool in_place = gs && !gs_fused_ok(h, L);
-    const bool fusedk = h->halo_mode == 2 && h->p.face_terms && !in_place && producer_kernel(h, L, gs);
-    const bool use_strips = in_place || fusedk || h->halo_mode == 0;
+    // GS without face terms (the literal head) or on a level too deep for the window ring: two in-place passes
+    const bool in_place = gs && !(h->p.face_terms && L.s <= 8);
+    const bool fusedk = h->p.face_terms && producer_level(L);
+    const bool use_strips = in_place || fusedk;
     // the producer warps of the sweep send the new cut-face values to the peers themselves (the strips it reads were
     // exchanged by k_halo or unpacked out of the staging buffer just before)
-    const bool xs = fusedk && xchg_kernel(h, L) && (!gs || (h->win_producer && L.s >= 6));
+    const bool xs = fusedk && h->p2p_ready && L.xsend && !h->plan.peers.empty();
     int rc = ensure_strips(h, level, use_strips);
     if (rc) return rc;
     if (solver == 1 || solver == 2) {
@@ -842,7 +812,7 @@ int do_smooth(pamg_handle* h, int level, int solver, int nsweeps, bool norm_firs
       // two-colour ordering of the reference's Gauss-Seidel sweep (all down children, then all up children; values across
       // parent faces stay lagged exactly as at :647-655), both colours in one pass over memory, written to the other
       // buffer (which then holds tracer%tnew, as for Jacobi)
-      rc = launch_gs_fused(h, L, L.T[L.cur], L.T[L.cur ^ 1], use_strips, fusedk, xs);
+      rc = launch_gs_one_pass(h, L, L.T[L.cur], L.T[L.cur ^ 1], use_strips, fusedk, xs);
       if (rc) return rc;
       L.cur ^= 1;
       L.tnew_alias = false;
@@ -887,7 +857,7 @@ int do_residual(pamg_handle* h, int level, double* l2, double* linf, double* sma
   if (2 * grid > h->npartial) return fail(h, PAMG_ERR_STATE, "partial buffer too small");
   // exterior values of faces between local parents come straight from TNEW (what update_overlaps copies); the strips of
   // faces cut by the GPU partition are refreshed here if something touched the field since the last exchange
-  const bool use_strips = L.strips_valid || h->halo_mode == 0;
+  const bool use_strips = L.strips_valid;
   int rc = ensure_strips(h, level, use_strips);
   if (rc) return rc;
   rc = launch_element<MODE_RESID>(h, L, tnew_ptr(L), L.res, 0, grid, use_strips);
@@ -1162,7 +1132,7 @@ int vcycle_body(const Group& G, pamg_handle* owner, int solver, int nu1, int nu2
 // the strips it read (local, unpacked cut faces) in the other strip buffer
 int undo_norm_sweep(pamg_handle* h) {
   LevelDev& L = h->lev[0];
-  const bool fusedk = h->halo_mode == 2 && h->p.face_terms && producer_kernel(h, L, false);
+  const bool fusedk = h->p.face_terms && producer_level(L);
   L.cur ^= 1;
   L.tnew_alias = true;
   if (fusedk) { L.ovl_cur ^= 1; L.strips_valid = true; L.cut_valid = true; }
@@ -1255,38 +1225,10 @@ int pamg_create(const pamg_params* p, int device, pamg_handle** out) {
   if (device < 0 || device >= ndev) return PAMG_ERR_ARG;
   pamg_handle* h = new pamg_handle();
   h->p = *p; h->device = device;
-  {
-    const char* e = getenv("PAMG_KERNEL");
-    if (e && !strcmp(e, "tma1d")) h->kernel_mode = 1;
-    else if (e && !strcmp(e, "direct2")) h->kernel_mode = 3;
-    else if (e && !strcmp(e, "win")) h->kernel_mode = 4;
-    const char* wp = getenv("PAMG_WIN");
-    if (wp && !strcmp(wp, "producer")) h->win_producer = true;
-    if (wp && !strcmp(wp, "barrier")) h->win_producer = false;
-    const char* pp = getenv("PAMG_P2P");
-    if (pp && pp[0] == '0') h->p2p_enabled = false;
-    const char* pt = getenv("PAMG_P2P_TIMEOUT_S");
-    if (pt && atof(pt) > 0.0) h->p2p_timeout_ns = (unsigned long long)(atof(pt) * 1e9);
-    const char* dg = getenv("PAMG_DEBUG_GAP_NS");
-    if (dg) h->debug_gap_ns = atoll(dg);
-    const char* lp = getenv("PAMG_L2_PERSIST");
-    if (lp && lp[0] == '0') h->l2_persist = false;
-    const char* vn = getenv("PAMG_VC_NORM");
-    if (vn && vn[0] == '0') h->vc_norm_fuse = false;
-    const char* xk = getenv("PAMG_XCHG");
-    if (xk && !strcmp(xk, "halo")) h->xchg_in_kernel = false;     // cut faces by a k_halo launch (copy, send, receive) between the sweeps
-    const char* hl = getenv("PAMG_HALO");
-    if (hl && !strcmp(hl, "strips")) h->halo_mode = 0;
-    if (hl && !strcmp(hl, "direct")) h->halo_mode = 1;
-    if (hl && !strcmp(hl, "fused")) h->halo_mode = 2;
-    const char* gr = getenv("PAMG_GRAPH");
-    if (gr && gr[0] == '0') h->use_graph = false;
-    const char* gn = getenv("PAMG_GRAPH_NCCL");
-    if (gn && gn[0] == '0') h->graph_nccl = false;
-    const char* g = getenv("PAMG_GS");
-    if (g && !strcmp(g, "direct")) { h->gs_tma = false; h->gs_fused = false; }
-    if (g && !strcmp(g, "twopass")) h->gs_fused = false;
-  }
+  const char* pp = getenv("PAMG_P2P");
+  if (pp && pp[0] == '0') h->p2p_enabled = false;
+  const char* pt = getenv("PAMG_P2P_TIMEOUT_S");
+  if (pt && atof(pt) > 0.0) h->p2p_timeout_ns = (unsigned long long)(atof(pt) * 1e9);
   if (cudaSetDevice(device) != cudaSuccess) { delete h; return PAMG_ERR_CUDA; }
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) h->nsm = prop.multiProcessorCount;
@@ -1356,7 +1298,7 @@ int pamg_create_multi(const pamg_params* p, int ngpus, const int* devices, pamg_
     q->in_group = true; q->nranks = ngpus; q->rank = i;
     root->parts.push_back(q);
   }
-  root->device = root->parts[0]->device; root->nsm = root->parts[0]->nsm; root->use_graph = root->parts[0]->use_graph;
+  root->device = root->parts[0]->device; root->nsm = root->parts[0]->nsm;
   *out = root;
   return PAMG_OK;
 }
@@ -1463,7 +1405,7 @@ int pamg_set_parents_partition(pamg_handle* h, int U_global, const double* X, co
     CK(cudaMalloc(&h->strip_arena, tot));
     CK(cudaMemsetAsync(h->strip_arena, 0, tot, h->stream));
     h->strip_arena_bytes = tot;
-    if (h->l2_persist && !h->shared_stream) {
+    if (!h->shared_stream) {
       // best effort: devices / driver modes without persisting L2 simply run without the window
       cudaDeviceProp prop;
       if (cudaGetDeviceProperties(&prop, h->device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
@@ -1549,8 +1491,8 @@ int pamg_set_parents_partition(pamg_handle* h, int U_global, const double* X, co
         ap.n_split = h->lev[lvl - 1].s;
         ap.multi_levels = h->p.multi_levels - lvl + 1;
         pamg_handle* g = new pamg_handle();
-        g->p = ap; g->device = h->device; g->nsm = h->nsm; g->kernel_mode = h->kernel_mode; g->gs_tma = h->gs_tma; g->gs_fused = h->gs_fused; g->win_producer = h->win_producer;
-        g->stream = h->stream; g->shared_stream = true; g->level_offset = lvl - 1; g->halo_mode = h->halo_mode;
+        g->p = ap; g->device = h->device; g->nsm = h->nsm;
+        g->stream = h->stream; g->shared_stream = true; g->level_offset = lvl - 1;
         g->bc_kind_h = h->bc_kind_h; g->bc_val_h = h->bc_val_h;
         h->agg = g;
         for (auto& ev : g->ev) CK(cudaEventCreate(&ev));
@@ -1847,8 +1789,8 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
   // replayed as one CUDA graph per GPU
   // Jacobi: no residual evaluation per cycle - the first pre-smoothing sweep of the next cycle reduces the norms of the iterate
   // it starts from (same numbers as get_residual's), and is taken back when the solve stops
-  bool fuse = solver == 1 && nu1 >= 1 && G[0]->vc_norm_fuse;
-  for (pamg_handle* q : G) fuse = fuse && norm_fusable(q, q->lev[0]) && q->halo_mode == 2;
+  bool fuse = solver == 1 && nu1 >= 1;
+  for (pamg_handle* q : G) fuse = fuse && norm_fusable(q, q->lev[0]);
   bool swept = false;                       // a fused body has run: its trailing norm sweep is pending
   auto finish = [&]() -> int {
     if (!fuse || !swept) return PAMG_OK;
@@ -1859,7 +1801,7 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
   const long long key0 = (((((long long)solver * 64 + nu1) * 64 + nu2) * 64 + ncoarse) * 2 + (fuse ? 1 : 0));
   // with NCCL in the cycle (halo exchange fallback, coarse gather/scatter) the capture is attempted once; if the library
   // refuses, the handle falls back to eager launches for good
-  bool graph_ok = h->use_graph;
+  bool graph_ok = true;
   for (pamg_handle* q : G) graph_ok = graph_ok && !q->profiling && (!q->comm || q->graph_nccl);
   for (int c = 1; c <= max_cycles; ++c) {
     if (c >= 2 && graph_ok) {

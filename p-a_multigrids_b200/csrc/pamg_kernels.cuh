@@ -1478,8 +1478,8 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
 // Branch-free direct kernel: thread per child, every load of the child (own values, rhs, the three
 // neighbours) is issued before the first use so that one memory latency is exposed per child instead of a
 // chain of two or three; children on a parent face patch their neighbour values from the halo strips in a
-// rare branch.  Coefficients come straight from the per-parent table (L1-resident).  Used for the coloured
-// Gauss-Seidel pass (in place) and selectable for the other modes (PAMG_KERNEL=direct2).
+// rare branch.  Coefficients come straight from the per-parent table (L1-resident).  Used on levels with fewer
+// than 256 children per parent (n_split <= 3) in every mode but the one-pass GS with face terms (k_gs_small).
 // one child, everything from global memory: used by the direct kernel and by the boundary fix-up kernel
 template <int MODE, bool FACE>
 __device__ __forceinline__ void child_update(const ElemArgs& a, int u, int r, int ipos, int ele, int len, double& acc_sum,
@@ -2011,12 +2011,6 @@ __global__ void __launch_bounds__(TPB) k_output_fields(OutArgs a) {
       if (a.error) a.error[g * 3 + i] = fabs(a.T[g * 3 + i] - an);
     }
   }
-}
-
-// measurement aid: one warp that does nothing for `ns` nanoseconds
-__global__ void k_spin(long long ns) {
-  const unsigned long long t0 = p2p_now();
-  while ((long long)(p2p_now() - t0) < ns) { }
 }
 
 __global__ void __launch_bounds__(TPB) k_fill(double* p, long long n, double v) {

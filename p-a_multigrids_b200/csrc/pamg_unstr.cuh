@@ -352,7 +352,6 @@ inline int stream_grid(K kernel, int& occ_cache, int E, int nsm) {
   if (occ_cache <= 0) {
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, TPB, 0) != cudaSuccess || occ < 1) occ = 2;
-    if (const char* ev = getenv("PAMG_UNSTR_CTAS_PER_SM")) occ = std::max(1, std::min(occ, atoi(ev)));   // experiments
     occ_cache = occ;
   }
   return std::max(1, std::min((E + TPB - 1) / TPB, nsm * std::min(occ_cache, 8)));   // (8: the Krylov partial sums are sized for it)

@@ -3,17 +3,14 @@
 Direct parity with the CPU oracle on the SAME seeded inputs (the oracle, OpenMP over parents, needs about a second per
 sweep at c5): one Jacobi sweep, one residual evaluation, one two-colour Gauss-Seidel sweep (rel-L2 <= 1e-12 each, the
 north-star tolerance) and the residual history of the first V-cycles (rtol 1e-6).  Size-independent properties follow:
-affinity of the sweep, transfer identities, mesh-independent convergence, and the fall-back kernel families against the
-oracle-checked default."""
+affinity of the sweep, transfer identities and mesh-independent convergence."""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 import oracle_api as orc
-from helpers import ROOT, rel_l2
+from helpers import rel_l2
 from pamg_pkg import pamg
 
 pytestmark = pytest.mark.gpu
@@ -82,7 +79,7 @@ def test_vcycle_history_matches_the_oracle_at_full_size(n, solver, cycles):
 
 
 @pytest.mark.parametrize("n", [7, 8])
-def test_sweep_is_affine_and_fallback_families_agree(n):
+def test_sweep_is_affine(n):
     g, _ = big_solver(n)
     shape = g.shape(1)
     T1, T2, Told = rnd(shape, 1), rnd(shape, 2), rnd(shape, 3)
@@ -97,29 +94,7 @@ def test_sweep_is_affine_and_fallback_families_agree(n):
         a = 0.3
         s1, s2, s12 = sweep(T1, solver), sweep(T2, solver), sweep(a * T1 + (1 - a) * T2, solver)
         assert rel_l2(s12, a * s1 + (1 - a) * s2) <= 1e-13          # S(aT1+(1-a)T2) = aS(T1)+(1-a)S(T2)
-    ref = sweep(T1, pamg.JACOBI)       # the default kernel, checked against the oracle above
     g.close()
-    # the same sweep through the families that serve the other level sizes, and with halo strips instead of
-    # neighbour-field reads (separate processes: the choice is read at handle creation)
-    code = ("import sys,numpy as np;sys.path.insert(0,'%s');from pamg_pkg import pamg;"
-            "m=pamg.Mesh.synthetic(4,1);p=pamg.default_params(n_split=%d,multi_levels=%d,u_x=0.9,u_y=0.3);"
-            "g=pamg.SemiImplicitIterative(p,m);r=lambda s:np.random.Generator(np.random.MT19937(s)).random(g.shape(1));"
-            "g.upload(pamg.TOLD,1,r(3));g.upload(pamg.TNONLIN,1,r(1));g.smoother(1,pamg.JACOBI,1);"
-            "np.save(sys.argv[1],g.download(pamg.TNONLIN,1))") % (os.path.join(ROOT, "tests"), n, n)
-    for fam in ("direct2", "tma1d", "win:barrier", "win:producer:strips", "win:producer:direct"):
-        out = os.path.join(os.environ.get("TMPDIR", "/tmp"), f"pamg_{fam.replace(':', '_')}_{n}.npy")
-        parts = fam.split(":")
-        env = dict(os.environ, PAMG_KERNEL=parts[0])
-        if len(parts) > 1:
-            env["PAMG_WIN"] = parts[1]
-        if len(parts) > 2:
-            env["PAMG_HALO"] = parts[2]
-        r = subprocess.run([sys.executable, "-c", code, out], env=env,
-                           capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stderr[-2000:]
-        other = np.load(out)
-        os.unlink(out)
-        assert rel_l2(other, ref) <= 1e-13, fam
 
 
 def test_transfer_identities_full_size():

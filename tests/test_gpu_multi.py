@@ -12,19 +12,18 @@ pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-@pytest.mark.parametrize("xchg", ["sweep", "halo", "deep", "theta"])
+@pytest.mark.parametrize("xchg", ["sweep", "deep", "theta"])
 @pytest.mark.parametrize("world", [2, 4])
 def test_partitioned_smoother_and_vcycle_match_single_gpu(world, xchg):
     """theta: the default exchange with theta = 1/2 (the told strips of the cut faces are exchanged for the old-time terms);
-    xchg = sweep: the producer warps of the sweeps send the cut-face values, an unpack launch runs between sweeps (default);
-    halo: k_halo copies, sends and receives between the sweeps (PAMG_XCHG=halo); deep: nearly no agglomeration
-    (PAMG_AGG_ELEMS=1024), so that every kernel family of the hierarchy runs partitioned with its own exchange."""
+    xchg = sweep: the producer warps of the sweeps send the cut-face values, an unpack launch runs between sweeps; k_halo
+    copies, sends and receives after uploads and prolongations and on the levels without a producer warp; deep: nearly
+    no agglomeration (PAMG_AGG_ELEMS=1024), so that every kernel family of the hierarchy runs partitioned with its own
+    exchange."""
     if pamg.device_count() < world:
         pytest.skip(f"needs {world} GPUs")
     env = dict(os.environ)
     env.setdefault("PAMG_P2P_TIMEOUT_S", "30")
-    if xchg == "halo":
-        env["PAMG_XCHG"] = "halo"
     if xchg == "deep":
         env["PAMG_AGG_ELEMS"] = "1024"
     if xchg == "theta":

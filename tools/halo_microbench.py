@@ -38,7 +38,7 @@ def main():
         allms = [None] * world
         dist.all_gather_object(allms, ms)
         if rank == 0:
-            print(f"{what}: {max(allms) * 1e3:.1f} us per call (PAMG_P2P={os.environ.get('PAMG_P2P', '1')}, PAMG_XCHG={os.environ.get('PAMG_XCHG', 'sweep')}, ranks {world})", flush=True)
+            print(f"{what}: {max(allms) * 1e3:.1f} us per call (PAMG_P2P={os.environ.get('PAMG_P2P', '1')}, ranks {world})", flush=True)
     g.close()
     dist.destroy_process_group()
 
