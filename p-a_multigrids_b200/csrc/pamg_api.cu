@@ -65,6 +65,12 @@ namespace { void p2p_close(pamg_handle* h); }
 enum { AGG_COUNTER = 0, AGG_EPOCH = 8, AGG_FLAGS = 40, AGG_EXPECT = 72, AGG_WORDS = 104 };
 
 // ------------------------------------------------------------------ handle
+// what the strips of the faces cut by the GPU partition hold.  CUT_STAGED: the values of the current iterate, sent by a
+// sweep's producer warps, wait in the level's flagged staging buffer under the current exchange number; an unpack is due.
+// The letters of the exchange-protocol model (tests/test_exchange_protocol_model.py) are the transitions next to
+// ensure_strips: H halo_exchanged, W sweep_done after a sweep that sent, U unpacked, X field_changed.
+enum CutState { CUT_STALE, CUT_STAGED, CUT_VALID };
+
 struct LevelDev {
   int s = 0, S = 0;
   long long C = 0, nelem = 0, ndof = 0;
@@ -75,8 +81,8 @@ struct LevelDev {
   double* ovlb[2] = {nullptr, nullptr};       // halo strips, double-buffered: (nstrips + nsend) * 3S doubles each
   int ovl_cur = 0;                            // ovlb[ovl_cur] holds the strips of the current iterate when strips_valid
   bool strips_valid = false;                  // strips of the faces between local parents hold the current iterate
-  bool cut_valid = false;                     // strips of the faces cut by the GPU partition hold the current iterate
-  bool stage_valid = false;                   // ... and the level's flagged staging buffer holds it under the current exchange number
+  CutState cut = CUT_STALE;                   // strips of the faces cut by the GPU partition
+  // (strips_valid and cut are written only by the transitions next to ensure_strips)
   ulonglong2* xsend = nullptr;                // [U*3] where a sweep's producer warp sends the values of a cut side (ElemArgs::xsend)
   double* ovl_old = nullptr;                  // told strips (update_overlaps as written only)
   double* pc = nullptr;               // [U][NPC]
@@ -190,15 +196,60 @@ int materialise_tnew(pamg_handle* h, LevelDev& L) {
   return PAMG_OK;
 }
 
+// ---- transitions of a level's strip state (LevelDev::strips_valid, LevelDev::cut)
+// X: something other than a sweep wrote the iterate (upload, fill, copy, prolongation, a coarse correction)
+void field_changed(LevelDev& L) { L.strips_valid = false; L.cut = CUT_STALE; }
+
+// H: a k_halo launch exchanged the cut faces of a field under a new exchange number, and copied the strips of every face
+// between parents unless it ran HALO_CUT.  Of the iterate: those strips are current.  Of TOLD: the staging buffer no
+// longer holds what a sweep's producer warps sent.
+void halo_exchanged(LevelDev& L, HaloMode mode, bool of_iterate) {
+  if (!of_iterate) { if (L.cut == CUT_STAGED) L.cut = CUT_STALE; return; }
+  if (mode != HALO_CUT) L.strips_valid = true;
+  L.cut = CUT_VALID;
+}
+
+// U: the staged cut-face values are in the strips
+void unpacked(LevelDev& L) { L.cut = CUT_VALID; }
+
+// W: the end of a sweep.  The producer warps of a fused sweep wrote the strips of the new iterate, except those of the
+// cut faces, whose values they sent to the peers when `sent`; any other sweep leaves no current strips.
+void sweep_done(const pamg_handle* h, LevelDev& L, bool fused, bool sent) {
+  if (!fused) { field_changed(L); return; }
+  L.strips_valid = true;
+  L.cut = h->plan.peers.empty() ? CUT_VALID : sent ? CUT_STAGED : CUT_STALE;
+}
+
+// undo_norm_sweep: the strips a fused sweep read are current again; what it sent to the peers belongs to the discarded
+// iterate
+void sweep_undone(LevelDev& L, bool fused) {
+  if (!fused) { field_changed(L); return; }
+  L.strips_valid = true; L.cut = CUT_VALID;
+}
+
+int launch_halo(pamg_handle* h, int level, HaloMode mode);
+
+// halo data of the current iterate, refreshed only if something touched the field since: `all` = the strips of every
+// face between parents (in-place sweeps and the kernels that do not read their neighbours' field), otherwise only the
+// strips of the faces cut by the GPU partition
+int ensure_strips(pamg_handle* h, int level, bool all = true) {
+  LevelDev& L = h->lev[level - 1];
+  if (!h->p.face_terms) return PAMG_OK;
+  if (all && !L.strips_valid) return launch_halo(h, level, HALO_SHARED);
+  if (L.cut == CUT_VALID) return PAMG_OK;
+  // the values a sweep's producer warps sent are waiting in the staging buffer: unpack them; else a full exchange
+  return launch_halo(h, level, (L.cut == CUT_STAGED && h->p2p_ready) ? HALO_UNPACK : HALO_CUT);
+}
+
 double* field_ptr(pamg_handle* h, int field, int level, bool for_write, int* rc) {
   *rc = PAMG_OK;
   LevelDev& L = h->lev[level - 1];
   switch (field) {
     case PAMG_TNEW:
-      if (for_write) { *rc = materialise_tnew(h, L); L.strips_valid = false; L.cut_valid = false; L.stage_valid = false; return L.T[L.cur ^ 1]; }
+      if (for_write) { *rc = materialise_tnew(h, L); field_changed(L); return L.T[L.cur ^ 1]; }
       return tnew_ptr(L);
     case PAMG_TNONLIN:
-      if (for_write) { *rc = materialise_tnew(h, L); L.strips_valid = false; L.cut_valid = false; L.stage_valid = false; }
+      if (for_write) { *rc = materialise_tnew(h, L); field_changed(L); }
       return L.T[L.cur];
     case PAMG_TOLD: if (for_write) L.rhs_valid = false; return L.told;
     case PAMG_RHS: if (for_write) L.rhs_valid = true; return L.rhs;
@@ -319,7 +370,6 @@ bool parent_coefficients(const pamg_params& p, const double* Xall, const int32_t
   return supported;
 }
 
-int launch_halo(pamg_handle* h, int level, int what = 0);
 int p2p_upload_args(pamg_handle* h);
 
 void p2p_close(pamg_handle* h) {
@@ -486,69 +536,58 @@ int exchange_halo_nccl(pamg_handle* h, LevelDev& L, double* ovl) {
   return PAMG_OK;
 }
 
-// what: 0 = update_overlaps as written (every face, tnew and told strips); 1 = Dirichlet faces only (static data,
-// written once per level); 2 = faces cut by the GPU partition only (the exchange step of a sweep that reads its local
-// neighbours straight from the field); 3 = every face between parents.
-int launch_halo(pamg_handle* h, int level, int what) {
-  LevelDev& L = h->lev[level - 1];
+// one k_halo launch on level L: `mode` applied to the strips of `src` in `ovl` (HALO_ALL: and to the told strips).  With
+// peers the cut faces are exchanged: inside the kernel through peer memory (set up at the first exchange), else by NCCL
+// after it.  Without peers there are no cut faces to exchange or unpack.
+int launch_halo_kernel(pamg_handle* h, LevelDev& L, HaloMode mode, const double* src, double* ovl) {
+  const bool cut = mode != HALO_DIRICHLET && !h->plan.peers.empty();
+  if ((mode == HALO_CUT || mode == HALO_UNPACK) && !cut) return PAMG_OK;
+  const int level = (int)(&L - h->lev.data()) + 1;
   HaloArgs a;
-  a.tnew = tnew_ptr(L); a.told = L.told; a.ovl = L.ovlb[L.ovl_cur]; a.ovl_old = L.ovl_old; a.xg = h->xg;
+  a.tnew = src; a.told = L.told; a.ovl = ovl; a.ovl_old = L.ovl_old; a.xg = h->xg;
   a.dst_strip = h->dst_strip; a.rev = h->rev; a.strip_of = h->strip_of;
   a.bc_scale = (h->p.coarse_bc_zero && level + h->level_offset > 1) ? 0.0 : 1.0;
-  a.U = h->U; a.s = L.s; a.with_old = (what == 0) ? 1 : 0; a.what = what; a.nstrips = h->plan.nstrips;
+  a.U = h->U; a.s = L.s; a.with_old = (mode == HALO_ALL) ? 1 : 0; a.what = mode; a.nstrips = h->plan.nstrips;
   a.cut_lf = h->cut_lf; a.ncut = (int)h->plan.cut_lf.size();
   a.bc_kind = h->bc_kind; a.bc_val = h->bc_val;
-  const bool cut = what != 1 && !h->plan.peers.empty();
-  if ((what == 2 || what == 4) && !cut) { L.cut_valid = true; return PAMG_OK; }
-  if (what == 4 && !(h->p2p_ready && L.stage_valid)) return fail(h, PAMG_ERR_STATE, "nothing staged to unpack");
-  const long long n = (what == 2 ? (long long)a.ncut : what == 4 ? (long long)a.ncut * 3 : (long long)h->U * 3) * L.S;
   a.x.npeers = 0;
   if (cut && h->comm && h->p2p_enabled && !h->p2p_ready && !h->p2p_failed && !h->capturing && h->level_offset == 0) {
     int rc = p2p_setup(h);      // collective, first exchange only
     if (rc) return rc;
   }
   const bool fused_x = cut && h->p2p_ready;
-  if (what == 0 && cut) {
-    // update_overlaps as written also fills t_overlap_old (splitting.F90:1259-1262): an exchange of its own carries the told
-    // values of the cut faces into the neighbours' old strips (the sweeps never read them; the entry point returns them).
-    // It goes FIRST, so that the staging buffers end up holding the tnew values under the current exchange number.
-    HaloArgs b = a;
-    b.tnew = L.told; b.ovl = L.ovl_old; b.with_old = 0; b.what = 2;
-    if (fused_x) { int rc = p2p_args(h, L, L.ovl_old, b.x); if (rc) return rc; }
-    const long long n2 = (long long)b.ncut * L.S;
-    int g2 = grid_for(h, n2);
-    if (fused_x) g2 = std::min(g2, h->nsm * std::min(std::max(h->kc.halo, 1), 4));
-    k_halo<<<g2, TPB, 0, h->stream>>>(b);
-    h->launches++;
-    CK(cudaGetLastError());
-    if (!fused_x) { int rc = exchange_halo_nccl(h, L, L.ovl_old); if (rc) return rc; }
-  }
-  if (fused_x) { int rc = p2p_args(h, L, L.ovlb[L.ovl_cur], a.x); if (rc) return rc; }
+  if (fused_x) { int rc = p2p_args(h, L, ovl, a.x); if (rc) return rc; }
+  const long long n = (mode == HALO_CUT ? (long long)a.ncut : mode == HALO_UNPACK ? (long long)a.ncut * 3 : (long long)h->U * 3) * L.S;
   // with the exchange fused in, blocks poll for remote data after their own work: keep the grid within one wave
-  int hgrid = grid_for(h, n);
-  if (fused_x) hgrid = std::min(hgrid, h->nsm * std::min(std::max(h->kc.halo, 1), 4));
-  k_halo<<<hgrid, TPB, 0, h->stream>>>(a);
+  int grid = grid_for(h, n);
+  if (fused_x) grid = std::min(grid, h->nsm * std::min(std::max(h->kc.halo, 1), 4));
+  k_halo<<<grid, TPB, 0, h->stream>>>(a);
   h->launches++;
   CK(cudaGetLastError());
-  if (what == 1) return PAMG_OK;
-  if (what == 4) { L.cut_valid = true; return PAMG_OK; }
-  if (cut && !fused_x) { int rc = exchange_halo_nccl(h, L, L.ovlb[L.ovl_cur]); if (rc) return rc; }
-  L.cut_valid = true;
-  if (fused_x) L.stage_valid = true;       // the same values sit in the staging buffers under the current exchange number
-  if (what != 2) L.strips_valid = true;
+  if (cut && !fused_x) return exchange_halo_nccl(h, L, ovl);
   return PAMG_OK;
 }
 
-// halo data of the current iterate, refreshed only if something touched the field since: `all` = the strips of every
-// face between parents (in-place sweeps and the kernels that do not read their neighbours' field), otherwise only the
-// strips of the faces cut by the GPU partition
-int ensure_strips(pamg_handle* h, int level, bool all = true) {
+// told values of the cut faces into the neighbours' told strips: the exchange update_overlaps as written makes for
+// t_overlap_old (splitting.F90:1259-1262).  The sweeps never read them; the old-time terms (theta != 1) and the entry
+// point do.
+int exchange_told(pamg_handle* h, LevelDev& L) {
+  int rc = launch_halo_kernel(h, L, HALO_CUT, L.told, L.ovl_old);
+  if (!rc) halo_exchanged(L, HALO_CUT, false);
+  return rc;
+}
+
+// the strips of the current iterate: HALO_ALL (pamg_update_overlaps) or what ensure_strips asks for
+int launch_halo(pamg_handle* h, int level, HaloMode mode) {
   LevelDev& L = h->lev[level - 1];
-  if (!h->p.face_terms) return PAMG_OK;
-  if (all && !L.strips_valid) return launch_halo(h, level, 3);
-  if (L.cut_valid) return PAMG_OK;
-  // the values a sweep's producer warps sent are waiting in the staging buffer: unpack them; else a full exchange
-  return launch_halo(h, level, (L.stage_valid && h->p2p_ready) ? 4 : 2);
+  if (mode == HALO_UNPACK && !(h->p2p_ready && L.cut == CUT_STAGED)) return fail(h, PAMG_ERR_STATE, "nothing staged to unpack");
+  int rc;
+  // the told exchange goes FIRST, so that the staging buffers end up holding the tnew values under the current exchange number
+  if (mode == HALO_ALL && (rc = exchange_told(h, L))) return rc;
+  if ((rc = launch_halo_kernel(h, L, mode, tnew_ptr(L), L.ovlb[L.ovl_cur]))) return rc;
+  if (mode == HALO_UNPACK) unpacked(L);
+  else halo_exchanged(L, mode, true);
+  return PAMG_OK;
 }
 
 // the sweeps of this level run the window kernels with a producer warp (k_element_win2, k_gs_win2; with face terms the
@@ -641,23 +680,30 @@ int configure_kernels(pamg_handle* h) {
   return PAMG_OK;
 }
 
-// use_strips: every strip of the level holds the start-of-sweep values (else: neighbour-field reads where possible);
-// write_next: the kernel's producer warp writes the strips of the next sweep into the other strip buffer
-// what a launch takes from somewhere else than the level's current state (the old-time pass of get_RHS, theta != 1)
-struct ElemOverride { const double* ovl; const double* pc; double rsign; };
-
-template <int MODE>
-int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, int colour, int grid, bool use_strips,
-                   bool write_next = false, bool xchg = false, bool norm = false, const ElemOverride* ov = nullptr) {
+// the arguments of a sweep-kernel launch.  use_strips: every strip of the level holds the start-of-sweep values (else:
+// neighbour-field reads where possible); write_next: the kernel's producer warp writes the strips of the next sweep into
+// the other strip buffer
+ElemArgs elem_args(const pamg_handle* h, const LevelDev& L, const double* Tin, double* Tout, int colour, bool use_strips,
+                   bool write_next) {
   ElemArgs a;
   a.xsend = L.xsend; a.xsync = h->p2p_sync ? h->p2p_sync + (size_t)(&L - h->lev.data()) * P2P_WORDS : nullptr;
-  if (MODE == MODE_RESID) xchg = false;     // a residual evaluation sends nothing
   a.Tin = Tin; a.Tout = Tout; a.rhs = L.rhs; a.ovl = L.ovlb[L.ovl_cur]; a.pc = L.pc; a.strip_of = h->strip_of; a.hmap = h->hmap;
   // (an in-place pass - the two-pass coloured GS - must see start-of-sweep values across parent faces: strips only)
   a.nsrc = (use_strips || Tin == Tout) ? nullptr : h->nsrc;
   a.ovl_next = write_next ? L.ovlb[L.ovl_cur ^ 1] : nullptr; a.dst_strip = h->dst_strip; a.rev = h->rev; a.nstrips = h->plan.nstrips;
   a.partial = h->partial; a.omega = h->p.omega; a.rsign = (double)h->p.residual_sign; a.nelem = L.nelem; a.s = L.s;
   a.colour = colour; a.partial_off = 0;
+  return a;
+}
+
+// what a launch takes from somewhere else than the level's current state (the old-time pass of get_RHS, theta != 1)
+struct ElemOverride { const double* ovl; const double* pc; double rsign; };
+
+template <int MODE>
+int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, int colour, int grid, bool use_strips,
+                   bool write_next = false, bool xchg = false, bool norm = false, const ElemOverride* ov = nullptr) {
+  ElemArgs a = elem_args(h, L, Tin, Tout, colour, use_strips, write_next);
+  if (MODE == MODE_RESID) xchg = false;     // a residual evaluation sends nothing
   if (ov) { a.ovl = ov->ovl; a.pc = ov->pc; a.rsign = ov->rsign; }
   const int f = h->p.face_terms ? 1 : 0;
   // the in-place GS pass runs with face terms only on s >= 9 (do_smooth), so k_element_win and k_element_direct2 have
@@ -700,41 +746,13 @@ int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout,
   return PAMG_OK;
 }
 
-// told values of the level-1 faces cut by the GPU partition into the neighbours' told strips (the exchange that
-// update_overlaps as written makes for t_overlap_old, splitting.F90:1259-1262; see launch_halo, what = 0)
-int exchange_told_cut(pamg_handle* h) {
-  LevelDev& L = h->lev[0];
-  if (h->plan.peers.empty()) return PAMG_OK;
-  HaloArgs b;
-  b.tnew = L.told; b.told = L.told; b.ovl = L.ovl_old; b.ovl_old = L.ovl_old; b.xg = h->xg;
-  b.dst_strip = h->dst_strip; b.rev = h->rev; b.strip_of = h->strip_of;
-  b.bc_scale = 1.0; b.U = h->U; b.s = L.s; b.with_old = 0; b.what = 2; b.nstrips = h->plan.nstrips;
-  b.cut_lf = h->cut_lf; b.ncut = (int)h->plan.cut_lf.size();
-  b.bc_kind = h->bc_kind; b.bc_val = h->bc_val;
-  b.x.npeers = 0;
-  if (h->comm && h->p2p_enabled && !h->p2p_ready && !h->p2p_failed && !h->capturing && h->level_offset == 0) {
-    int rc = p2p_setup(h);      // collective, first exchange only
-    if (rc) return rc;
-  }
-  const bool fused_x = h->p2p_ready;
-  if (fused_x) { int rc = p2p_args(h, L, L.ovl_old, b.x); if (rc) return rc; }
-  int g2 = grid_for(h, (long long)b.ncut * L.S);
-  if (fused_x) g2 = std::min(g2, h->nsm * std::min(std::max(h->kc.halo, 1), 4));
-  k_halo<<<g2, TPB, 0, h->stream>>>(b);
-  h->launches++;
-  CK(cudaGetLastError());
-  if (!fused_x) { int rc = exchange_halo_nccl(h, L, L.ovl_old); if (rc) return rc; }
-  if (fused_x) L.stage_valid = false;     // the staging buffers now hold told values under the current exchange number
-  return PAMG_OK;
-}
-
 // theta != 1: RHS -= (1 - theta)(-stiff + flux + diff_vol + diff_surf) told  (get_RHS :459-460).  One residual-mode pass of the
 // level-1 sweep kernel over TOLD with the old-time coefficient table: exterior values of faces between local parents straight
 // from TOLD, Dirichlet data and cut-face values from the told strips.  RES is the scratch field of the pass.
 int add_old_time_terms(pamg_handle* h) {
   LevelDev& L = h->lev[0];
   int rc;
-  if (h->p.face_terms && (rc = exchange_told_cut(h))) return rc;
+  if (h->p.face_terms && (rc = exchange_told(h, L))) return rc;
   const int grid = grid_for(h, L.nelem);
   if (2 * grid > h->npartial) return fail(h, PAMG_ERR_STATE, "partial buffer too small");
   const ElemOverride ov = {L.ovl_old, L.pc_old, -1.0};     // r = b - A_old told with b = the theta = 1 right-hand side
@@ -748,13 +766,7 @@ int add_old_time_terms(pamg_handle* h) {
 bool gs_small_ok(const pamg_handle* h, const LevelDev& L) { return h->p.face_terms && L.C <= TPB; }
 
 int launch_gs_one_pass(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, bool use_strips, bool write_next, bool xchg) {
-  ElemArgs a;
-  a.xsend = L.xsend; a.xsync = h->p2p_sync ? h->p2p_sync + (size_t)(&L - h->lev.data()) * P2P_WORDS : nullptr;
-  a.Tin = Tin; a.Tout = Tout; a.rhs = L.rhs; a.ovl = L.ovlb[L.ovl_cur]; a.pc = L.pc; a.strip_of = h->strip_of; a.hmap = h->hmap;
-  a.nsrc = use_strips ? nullptr : h->nsrc;
-  a.ovl_next = write_next ? L.ovlb[L.ovl_cur ^ 1] : nullptr; a.dst_strip = h->dst_strip; a.rev = h->rev; a.nstrips = h->plan.nstrips;
-  a.partial = h->partial; a.omega = h->p.omega; a.rsign = (double)h->p.residual_sign; a.nelem = L.nelem; a.s = L.s;
-  a.colour = 1; a.partial_off = 0;
+  const ElemArgs a = elem_args(h, L, Tin, Tout, 1, use_strips, write_next);
   if (gs_small_ok(h, L)) {
     const long long ppc = TPB / L.C, nparents = L.nelem / L.C;
     const int sgrid = (int)std::max(1ll, std::min((nparents + ppc - 1) / ppc, (long long)h->nsm * 8));
@@ -823,13 +835,8 @@ int do_smooth(pamg_handle* h, int level, int solver, int nsweeps, bool norm_firs
       rc = launch_element<MODE_GS>(h, L, L.T[L.cur], L.T[L.cur], 1, grid, true);   // all children on parent faces are "up"
       if (rc) return rc;
     }
-    if (fusedk) {
-      L.ovl_cur ^= 1;                        // the producer warps wrote the strips of the new iterate
-      L.strips_valid = true; L.cut_valid = h->plan.peers.empty();
-      L.stage_valid = xs;                    // ... and sent the cut-face values to the peers as the next exchange
-    } else {
-      L.strips_valid = false; L.cut_valid = false; L.stage_valid = false;
-    }
+    if (fusedk) L.ovl_cur ^= 1;              // the producer warps wrote the strips of the new iterate
+    sweep_done(h, L, fusedk, xs);
   }
   return PAMG_OK;
 }
@@ -907,7 +914,7 @@ int do_prolong(pamg_handle* h, int fine_level, bool keep_tnew = true) {
       F.tnew_alias = true;            // inside the V-cycle nothing reads the pre-correction field
     }
     a.src = Cc.T[Cc.cur]; a.dst = F.T[F.cur];
-    F.strips_valid = false; F.cut_valid = false; F.stage_valid = false;           // the iterate changes outside a sweep
+    field_changed(F);
     k_prolong_p1<<<grid_for(h, F.nelem), TPB, 0, h->stream>>>(a);
   }
   h->launches++;
@@ -991,7 +998,7 @@ int agg_coarse_solve(const Group& G, pamg_handle* owner, int solver, int nu1, in
       LevelDev& A = g->lev[0];
       CK(cudaMemcpyAsync(A.rhs, Lc.rhs, per_parent * h->U * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
       CK(cudaMemsetAsync(A.T[A.cur], 0, A.ndof * sizeof(double), h->stream));
-      A.tnew_alias = true; A.strips_valid = false; A.cut_valid = false; A.stage_valid = false; A.rhs_valid = true;
+      A.tnew_alias = true; field_changed(A); A.rhs_valid = true;
       const long long l0 = g->launches;
       int rc = vcycle_rec(Group{g}, g, 1, solver, nu1, nu2, ncoarse);
       h->launches += g->launches - l0;
@@ -1008,7 +1015,7 @@ int agg_coarse_solve(const Group& G, pamg_handle* owner, int solver, int nu1, in
       g_nccl.Recv(Lc.T[Lc.cur], per_parent * h->U, ncclFloat64, 0, h->comm, h->stream);
     }
     if (g_nccl.GroupEnd() != ncclSuccess) return fail(h, PAMG_ERR_CUDA, "ncclGroupEnd failed in coarse scatter");
-    Lc.tnew_alias = true; Lc.strips_valid = false; Lc.cut_valid = false; Lc.stage_valid = false;
+    Lc.tnew_alias = true; field_changed(Lc);
     return PAMG_OK;
   }
   // single process, several GPUs: the parts push their slices into part 0's memory (k_push), part 0 waits for the
@@ -1033,13 +1040,13 @@ int agg_coarse_solve(const Group& G, pamg_handle* owner, int solver, int nu1, in
     CK(cudaMemsetAsync(A.T[A.cur], 0, A.ndof * sizeof(double), h->stream));
     int rc = launch_wait(h, all);
     if (rc) return gfail(owner, h, rc);
-    A.tnew_alias = true; A.strips_valid = false; A.cut_valid = false; A.stage_valid = false; A.rhs_valid = true;
+    A.tnew_alias = true; field_changed(A); A.rhs_valid = true;
     const long long l0 = g->launches;
     rc = vcycle_rec(Group{g}, g, 1, solver, nu1, nu2, ncoarse);
     h->launches += g->launches - l0;
     if (rc) { h->err = g->err; return gfail(owner, h, rc); }
     CK(cudaMemcpyAsync(Lc.T[Lc.cur], A.T[A.cur], per_parent * h->U * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-    Lc.tnew_alias = true; Lc.strips_valid = false; Lc.cut_valid = false; Lc.stage_valid = false;
+    Lc.tnew_alias = true; field_changed(Lc);
     for (size_t p = 1; p < G.size(); ++p) {
       pamg_handle* q = G[p];
       LevelDev& Lq = q->lev[lvl - 1];
@@ -1054,7 +1061,7 @@ int agg_coarse_solve(const Group& G, pamg_handle* owner, int solver, int nu1, in
     int rc = launch_wait(q, 1u);
     if (rc) return gfail(owner, q, rc);
     LevelDev& Lq = q->lev[lvl - 1];
-    Lq.tnew_alias = true; Lq.strips_valid = false; Lq.cut_valid = false; Lq.stage_valid = false;
+    Lq.tnew_alias = true; field_changed(Lq);
   }
   return PAMG_OK;
 }
@@ -1097,7 +1104,7 @@ int vcycle_rec(const Group& G, pamg_handle* owner, int level, int solver, int nu
     int rc = do_fill(q, Cc.T[Cc.cur], Cc.ndof, 0.0);
     if (rc) return gfail(owner, q, rc);
     Cc.tnew_alias = true;
-    Cc.strips_valid = false; Cc.cut_valid = false; Cc.stage_valid = false;
+    field_changed(Cc);
   }
   int rc;
   if (G[0]->agg_level && level + 1 == G[0]->agg_level) {
@@ -1135,9 +1142,8 @@ int undo_norm_sweep(pamg_handle* h) {
   const bool fusedk = h->p.face_terms && producer_level(L);
   L.cur ^= 1;
   L.tnew_alias = true;
-  if (fusedk) { L.ovl_cur ^= 1; L.strips_valid = true; L.cut_valid = true; }
-  else { L.strips_valid = false; L.cut_valid = false; }
-  L.stage_valid = false;                    // (whatever the sweep sent to the peers belongs to the discarded iterate)
+  if (fusedk) L.ovl_cur ^= 1;
+  sweep_undone(L, fusedk);
   return PAMG_OK;
 }
 
@@ -1442,7 +1448,6 @@ int pamg_set_parents_partition(pamg_handle* h, int U_global, const double* X, co
     arena_off += 2 * obp;
     CK(cudaMalloc(&L.ovl_old, ob));
     CK(cudaMemsetAsync(L.ovl_old, 0, ob, h->stream));  // :207
-    L.ovl_cur = 0; L.strips_valid = false; L.cut_valid = false; L.stage_valid = false;
     for (int u = 0; u < U; ++u)
       if (!parent_coefficients(h->p, X, neig, bc_glob, first + u, L.s, &pc[(size_t)u * NPC], h->p.theta))
         return fail(h, PAMG_ERR_UNSUPPORTED, "open boundary face (kind 2) with inflow: give it Dirichlet data instead");
@@ -1458,23 +1463,13 @@ int pamg_set_parents_partition(pamg_handle* h, int U_global, const double* X, co
     }
     L.cur = 0; L.tnew_alias = true; L.rhs_valid = (il != 0);
   }
-  // Dirichlet data sin(x+y) on domain-boundary faces never changes: fill those strips once per level
-  for (int il = 1; il <= h->p.multi_levels; ++il)
-    for (int bsel = 0; bsel < 2; ++bsel) {
-      h->lev[il - 1].ovl_cur = bsel;
-      int rc2 = launch_halo(h, il, 1);
-      if (rc2) return rc2;
-    }
-  for (auto& Lv : h->lev) Lv.ovl_cur = 0;
-  if (h->lev[0].pc_old) {
-    // ... and in the told strips of level 1, which the old-time face terms read (theta != 1)
-    LevelDev& L1 = h->lev[0];
-    double* keep = L1.ovlb[0];
-    L1.ovlb[0] = L1.ovl_old;
-    int rc2 = launch_halo(h, 1, 1);
-    L1.ovlb[0] = keep;
-    if (rc2) return rc2;
-  }
+  // Dirichlet data sin(x+y) on domain-boundary faces never changes: fill those strips once per level, in both strip
+  // buffers, and in the told strips of level 1, which the old-time face terms read (theta != 1)
+  for (auto& Lv : h->lev)
+    for (double* ovl : {Lv.ovlb[0], Lv.ovlb[1]})
+      if ((rc = launch_halo_kernel(h, Lv, HALO_DIRICHLET, nullptr, ovl))) return rc;
+  LevelDev& L1 = h->lev[0];
+  if (L1.pc_old && (rc = launch_halo_kernel(h, L1, HALO_DIRICHLET, nullptr, L1.ovl_old))) return rc;
   // coarse-level agglomeration on part 0: first level whose GLOBAL size is small enough to be launch-bound
   if (nparts > 1 && h->level_offset == 0) {
     const char* e = getenv("PAMG_AGG_ELEMS");
@@ -1661,7 +1656,7 @@ int pamg_copy_field(pamg_handle* h, int level, int dst_field, int src_field) {
   if (dst_field == src_field) return PAMG_OK;
   if (dst_field == PAMG_TNEW && src_field == PAMG_TNONLIN) { L.tnew_alias = true; return PAMG_OK; }      // :550
   if (dst_field == PAMG_TNONLIN && src_field == PAMG_TNEW) {                                             // :327
-    if (!L.tnew_alias) { L.cur ^= 1; L.tnew_alias = true; L.strips_valid = false; L.cut_valid = false; L.stage_valid = false; }
+    if (!L.tnew_alias) { L.cur ^= 1; L.tnew_alias = true; field_changed(L); }
     return PAMG_OK;
   }
   int rc;
@@ -1707,7 +1702,7 @@ int pamg_update_overlaps(pamg_handle* h, int level) {
   FANOUT(h, q, pamg_update_overlaps(q, level));
   if (!valid_level(h, level)) return PAMG_ERR_ARG;
   CK(cudaSetDevice(h->device));
-  return launch_halo(h, level);
+  return launch_halo(h, level, HALO_ALL);
 }
 
 int pamg_build_rhs(pamg_handle* h) {
@@ -1778,7 +1773,7 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
   if (!valid_level(G[0], 1)) return PAMG_ERR_ARG;
   CK(cudaSetDevice(G[0]->device));
   int rc;
-  for (pamg_handle* q : G) { LevelDev& L = q->lev[0]; L.tnew_alias = true; L.strips_valid = false; L.cut_valid = false; L.stage_valid = false; }
+  for (pamg_handle* q : G) { LevelDev& L = q->lev[0]; L.tnew_alias = true; field_changed(L); }
   double r0 = 0, r = 0, dummy;
   GALL(G, h, q, do_residual(q, 1, &dummy, nullptr, nullptr, true));
   if ((rc = group_norms(G, h, &r0, nullptr, nullptr))) return rc;
@@ -1919,7 +1914,7 @@ int pamg_timestep_host(pamg_handle* h, const double* tnew_in, double* tnew_out, 
     const size_t bytes = (size_t)L.ndof * sizeof(double);
     CK_(q, cudaMemcpyAsync(L.T[L.cur], tnew_in + off, bytes, cudaMemcpyHostToDevice, q->stream));
     L.tnew_alias = true;
-    L.strips_valid = false; L.cut_valid = false; L.stage_valid = false;
+    field_changed(L);
     CK_(q, cudaMemcpyAsync(L.told, L.T[L.cur], bytes, cudaMemcpyDeviceToDevice, q->stream));
     L.rhs_valid = false;
     off += (size_t)L.ndof;
@@ -1995,7 +1990,7 @@ int pamg_smooth_host(pamg_handle* h, int solver, int nsweeps, const double* tnew
   if (!h->vc_graphs.empty()) { CK(cudaStreamSynchronize(h->stream)); for (auto& g : h->vc_graphs) for (auto e : g.exec) cudaGraphExecDestroy(e); h->vc_graphs.clear(); }
   std::swap(L.T[L.cur], L.spare);   // the uploaded field becomes the iterate; the previous result stays in `spare` for its download
   L.tnew_alias = true;              // tnew_nonlin = tnew = the uploaded field (transport_tri_semi.F90:317)
-  L.strips_valid = false; L.cut_valid = false; L.stage_valid = false;
+  field_changed(L);
   int rc = do_smooth(h, 1, solver, nsweeps);
   if (rc) return rc;
   CK(cudaEventRecord(h->ev_comp, h->stream));

@@ -41,7 +41,7 @@ enum { MODE_JACOBI = 0, MODE_RESID = 1, MODE_GS = 2, MODE_RICH = 3 };
 // Two kinds of kernels take part.  k_halo sends AND receives exchange n in one launch (after something other than a sweep
 // changed the field).  The sweep kernels with a producer warp (XCHG) SEND: as a tile is finished the producer warp stores the
 // new values of its children on cut faces straight into the peers' staging buffers as exchange n+1 (the NVLink trip hides
-// under the rest of the sweep) and the last CTA advances the exchange number; a small unpack launch (k_halo, what = 4) before
+// under the rest of the sweep) and the last CTA advances the exchange number; a small unpack launch (k_halo, HALO_UNPACK) before
 // the next sweep moves the values - long arrived - from the staging buffer into the strips.  The staging buffer has FOUR
 // slots indexed by the exchange number mod 4: a sending sweep that nobody unpacks (a prolongation came next; the level's
 // next visit starts with a k_halo exchange) lets a rank run two exchanges ahead of a peer that still has to unpack - two
@@ -1729,6 +1729,15 @@ __global__ void k_wait_flags(WaitArgs a) {
   __threadfence_system();
 }
 
+// what a k_halo launch writes (HaloArgs::what)
+enum HaloMode {
+  HALO_ALL = 0,        // everything: update_overlaps as written, tnew and told strips
+  HALO_DIRICHLET = 1,  // Dirichlet faces only
+  HALO_CUT = 2,        // faces cut by the GPU partition only (one thread per position of the faces listed in cut_lf)
+  HALO_SHARED = 3,     // every face shared by two parents (no Dirichlet data)
+  HALO_UNPACK = 4      // unpack the cut-face values a sweep's producer warps sent into my staging buffer
+};
+
 struct HaloArgs {
   P2PArgs x;                               // x.npeers > 0: cut-face strips go straight to the peers (fused exchange)
   const double* tnew; const double* told;
@@ -1737,11 +1746,9 @@ struct HaloArgs {
   const int32_t* dst_strip; const int32_t* rev; const int32_t* strip_of;
   double bc_scale;
   int U, s, with_old;
-  int what;   // 0 everything (update_overlaps as written); 1 Dirichlet faces only; 2 faces cut by the GPU partition only
-              // (one thread per position of the faces listed in cut_lf); 3 all faces between parents (no Dirichlet data);
-              // 4 unpack the cut-face values a sweep's producer warps sent into my staging buffer
+  int what;                                // a HaloMode
   int nstrips;
-  const int32_t* cut_lf; int ncut;         // what == 2: (u*3+mf) of the cut faces
+  const int32_t* cut_lf; int ncut;         // HALO_CUT: (u*3+mf) of the cut faces
   // Dirichlet data of domain-boundary faces per (u, side): kind 0 = sin(x+y) (splitting.F90:1246-1252), 1 = the constant
   // bc_val (update_overlaps' t_bc argument, :1210), 2 = open face, no data; nullptr = kind 0 everywhere
   const int32_t* bc_kind; const double* bc_val;
@@ -1766,16 +1773,16 @@ __device__ __forceinline__ void child_nodes(const double* __restrict__ xg, int s
 
 __global__ void __launch_bounds__(TPB) k_halo(HaloArgs a) {
   const int S = 1 << a.s, b = 2 << a.s;
-  const long long n = (a.what == 2 ? (long long)a.ncut : (long long)a.U * 3) * S;
+  const long long n = (a.what == HALO_CUT ? (long long)a.ncut : (long long)a.U * 3) * S;
   unsigned long long e64 = 0;
   if (a.x.npeers > 0) e64 = *(volatile unsigned long long*)(a.x.sync + P2P_EPOCH) + 1;
-  if (a.what == 4) {                       // the values of the current exchange sit in my staging buffer (a sweep's producer
+  if (a.what == HALO_UNPACK) {             // the values of the current exchange sit in my staging buffer (a sweep's producer
     p2p_receive(a.x, e64 - 1, false);      // warps sent them): unpack them into the strips, nothing to send
     return;
   }
   for (long long tid = (long long)blockIdx.x * TPB + threadIdx.x; tid < n; tid += (long long)gridDim.x * TPB) {
     const int i = (int)(tid & (S - 1));           // position - 1
-    const int lf = (a.what == 2) ? __ldg(a.cut_lf + (tid >> a.s)) : (int)(tid >> a.s);   // u*3 + mf
+    const int lf = (a.what == HALO_CUT) ? __ldg(a.cut_lf + (tid >> a.s)) : (int)(tid >> a.s);   // u*3 + mf
     const int u = lf / 3, mf = lf - 3 * u;
     const int pos = i + 1;
     int r, ipos;
@@ -1785,9 +1792,9 @@ __global__ void __launch_bounds__(TPB) k_halo(HaloArgs a) {
     const int ele = 1 + (r - 1) * (b + 1 - r) + ipos - 1;
     const int dst = __ldg(a.dst_strip + lf);
     const size_t S3 = (size_t)3 * S;
-    if (a.what == 1 && dst >= 0) continue;
-    if (a.what == 2 && dst < a.nstrips) continue;
-    if (a.what == 3 && dst < 0) continue;
+    if (a.what == HALO_DIRICHLET && dst >= 0) continue;
+    if (a.what == HALO_CUT && dst < a.nstrips) continue;
+    if (a.what == HALO_SHARED && dst < 0) continue;
     if (dst < 0) {
       // Dirichlet data at the two face nodes (:1246-1252,1287-1293,1344-1350): sin(x+y), or the constant t_bc of the face
       const int kind = a.bc_kind ? __ldg(a.bc_kind + lf) : 0;

@@ -18,7 +18,7 @@ def main():
     mesh = pamg.Mesh.synthetic(kp, world)
     per = 4 ** kp
     pf = np.arange(world + 1, dtype=np.int32) * per
-    # PAMG_TEST_THETA != 1: the told values of the cut faces travel too (old-time branch of get_RHS, exchange_told_cut)
+    # PAMG_TEST_THETA != 1: the told values of the cut faces travel too (old-time branch of get_RHS, exchange_told)
     params = pamg.default_params(n_split=n, multi_levels=n, u_x=0.9, u_y=0.3, theta=float(os.environ.get("PAMG_TEST_THETA", "1.0")))
     g = pamg.SemiImplicitIterative(params, mesh, device=local, nparts=world, part_first=pf, my_part=rank)
     ids = [pamg.get_unique_id() if rank == 0 else None]

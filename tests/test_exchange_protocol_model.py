@@ -22,8 +22,8 @@ import pytest
 
 
 def expand(program, in_sweep):
-    """program: string over H (halo exchange), W (sending sweep), U (unpack), X (field changed outside a sweep: no launch).
-    Returns the list of atomic steps of one rank: ('send', n) / ('wait', n) with the exchange numbers resolved."""
+    """program: string over H (halo exchange), W (sending sweep), U (unpack), X (field changed outside a sweep: no launch),
+    the strip-state transitions halo_exchanged, sweep_done, unpacked and field_changed of pamg_api.cu.  Returns the list of atomic steps of one rank: ('send', n) / ('wait', n) with the exchange numbers resolved."""
     steps, e = [], 0
     for op in program:
         if op == "H":
@@ -100,7 +100,7 @@ def shipped_programs(max_len):
             out.append(p); return
         # "XHH": told changed (or update_overlaps as written was called): the told values of the cut faces are exchanged by a
         # k_halo launch of their own, which leaves nothing to unpack, and a second one exchanges the tnew values
-        # (exchange_told_cut + ensure_strips, theta != 1; launch_halo what = 0)
+        # (exchange_told + ensure_strips, theta != 1; launch_halo with HALO_ALL)
         if pending:                       # a sweep has sent: unpack, or the field changes and k_halo exchanges afresh
             grow(p + "U", False)
             grow(p + "XH", False)

@@ -116,7 +116,7 @@ def test_crank_nicolson_time_steps_with_vcycles(meshes, solver):
 
 def test_partitioned_mesh_exchanges_the_told_strips():
     """three parts on one device: the told values of the cut faces travel into the neighbours' told strips before the
-    old-time pass (exchange_told_cut); result equal to the single handle's"""
+    old-time pass (exchange_told); result equal to the single handle's"""
     kp, n, theta = 2, 6, 0.5
     mesh = pamg.Mesh.synthetic(kp, 2)
     params = pamg.default_params(n_split=n, multi_levels=n, u_x=0.9, u_y=0.3, theta=theta)
