@@ -627,7 +627,7 @@ int configure_face(pamg_handle* h) {
   if ((rc = configure_one(h, k_element_win2<MODE_JACOBI, FACE>, WIN2_THREADS, WIN_SMEM_BYTES, h->kc.win2[f]))) return rc;
   if ((rc = configure_one(h, k_element_win2<MODE_RESID, FACE>, WIN2_THREADS, WIN_SMEM_BYTES, dummy))) return rc;
   if ((rc = configure_one(h, k_element_win2<MODE_RICH, FACE>, WIN2_THREADS, WIN_SMEM_BYTES, dummy))) return rc;
-  if (FACE) {
+  if constexpr (FACE) {   // (launch_element selects the XCHG and NORM kernels with face terms only)
     if ((rc = configure_one(h, k_element_win2<MODE_JACOBI, FACE, true>, WIN2_THREADS, WIN_SMEM_BYTES, h->kc.win2x))) return rc;
     if ((rc = configure_one(h, k_element_win2<MODE_JACOBI, FACE, false, true>, WIN2_THREADS, WIN_SMEM_BYTES, dummy))) return rc;
     if ((rc = configure_one(h, k_element_win2<MODE_JACOBI, FACE, true, true>, WIN2_THREADS, WIN_SMEM_BYTES, dummy))) return rc;
@@ -703,28 +703,29 @@ template <int MODE>
 int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout, int colour, int grid, bool use_strips,
                    bool write_next = false, bool xchg = false, bool norm = false, const ElemOverride* ov = nullptr) {
   ElemArgs a = elem_args(h, L, Tin, Tout, colour, use_strips, write_next);
-  if (MODE == MODE_RESID) xchg = false;     // a residual evaluation sends nothing
   if (ov) { a.ovl = ov->ovl; a.pc = ov->pc; a.rsign = ov->rsign; }
   const int f = h->p.face_terms ? 1 : 0;
-  // the in-place GS pass runs with face terms only on s >= 9 (do_smooth), so k_element_win and k_element_direct2 have
-  // no such instantiation
-  constexpr bool FACE_OK = MODE != MODE_GS;
   const bool prof = !ov && h->profiling && h->pev_used + 2 <= (int)h->pev.size();
   if (prof) CK(cudaEventRecord(h->pev[h->pev_used], h->stream));
+  // (the in-place GS pass never runs on a producer level, and with face terms only on s >= 9 (do_smooth): the branches
+  // below instantiate no GS kernel it cannot launch)
   if (MODE != MODE_GS && producer_level(L)) {
-    // window kernel with a producer warp (no CTA-wide barrier between tiles)
-    auto kern = xchg ? k_element_win2<MODE == MODE_RESID ? MODE_JACOBI : MODE, true, true>
-                     : h->p.face_terms ? k_element_win2<MODE, true> : k_element_win2<MODE, false>;
-    // a Jacobi sweep that also reduces the residual norms of the iterate it starts from (norm_fusable)
-    if (norm) kern = xchg ? k_element_win2<MODE == MODE_JACOBI ? MODE_JACOBI : MODE, true, true, MODE == MODE_JACOBI>
-                          : k_element_win2<MODE == MODE_JACOBI ? MODE_JACOBI : MODE, true, false, MODE == MODE_JACOBI>;
-    const int tgrid = (int)std::max(1ll, std::min(L.nelem / TPB, (long long)h->nsm * (xchg ? h->kc.win2x : h->kc.win2[f])));
-    kern<<<tgrid, WIN2_THREADS, WIN_SMEM_BYTES, h->stream>>>(a);
-    if (MODE == MODE_RESID || norm) h->last_partials = tgrid;
+    if constexpr (MODE != MODE_GS) {
+      // window kernel with a producer warp (no CTA-wide barrier between tiles)
+      const bool send = MODE != MODE_RESID && xchg;     // a residual evaluation sends nothing
+      void (*kern)(ElemArgs) = h->p.face_terms ? k_element_win2<MODE, true> : k_element_win2<MODE, false>;
+      if constexpr (MODE != MODE_RESID) if (send) kern = k_element_win2<MODE, true, true>;
+      // a Jacobi sweep that also reduces the residual norms of the iterate it starts from (norm_fusable)
+      if constexpr (MODE == MODE_JACOBI) if (norm) kern = send ? k_element_win2<MODE, true, true, true> : k_element_win2<MODE, true, false, true>;
+      const int tgrid = (int)std::max(1ll, std::min(L.nelem / TPB, (long long)h->nsm * (send ? h->kc.win2x : h->kc.win2[f])));
+      kern<<<tgrid, WIN2_THREADS, WIN_SMEM_BYTES, h->stream>>>(a);
+      if (MODE == MODE_RESID || norm) h->last_partials = tgrid;
+    }
   } else if (L.C >= TPB && L.s <= 8) {
     // (a vertical neighbour is up to 2^(s+1) children away: the 8-tile ring covers s <= 8)
     // window kernel: ring of 8 field tiles in shared memory, every neighbour value read from it
-    auto kern = h->p.face_terms && FACE_OK ? k_element_win<MODE, FACE_OK> : k_element_win<MODE, false>;
+    void (*kern)(ElemArgs) = k_element_win<MODE, false>;
+    if constexpr (MODE != MODE_GS) if (h->p.face_terms) kern = k_element_win<MODE, true>;
     const int tgrid = (int)std::max(1ll, std::min(L.nelem / TPB, (long long)h->nsm * h->kc.win[f]));
     kern<<<tgrid, TPB, WIN_SMEM_BYTES, h->stream>>>(a);
     if (MODE == MODE_RESID) h->last_partials = tgrid;
@@ -737,8 +738,9 @@ int launch_element(pamg_handle* h, LevelDev& L, const double* Tin, double* Tout,
   } else {
     // branch-free direct kernel (all loads of a child in flight at once): levels with fewer than 256 children per parent
     if (MODE == MODE_RESID) h->last_partials = grid;
-    if (h->p.face_terms && FACE_OK) k_element_direct2<MODE, FACE_OK><<<grid, TPB, 0, h->stream>>>(a);
-    else k_element_direct2<MODE, false><<<grid, TPB, 0, h->stream>>>(a);
+    void (*kern)(ElemArgs) = k_element_direct2<MODE, false>;
+    if constexpr (MODE != MODE_GS) if (h->p.face_terms) kern = k_element_direct2<MODE, true>;
+    kern<<<grid, TPB, 0, h->stream>>>(a);
   }
   if (prof) { CK(cudaEventRecord(h->pev[h->pev_used + 1], h->stream)); h->pev_used += 2; }
   h->launches++;

@@ -121,79 +121,31 @@ __host__ __device__ __forceinline__ void child_from_flat(int t, int s, int& r, i
 //   f1:(1,3)  f2:(3,2)  f3:(2,1)      (transport_tri_semi.F90:142-147), and the penalty coefficient of each face
 struct FaceIn { double n1a, n1b, n2a, n2b, n3a, n3b, pen1, pen2, pen3; };
 
-// One child: A x (get_A_x, transport_tri_semi.F90:412-448, theta = 1), the diagonal (get_diagonal :481-486)
-// and the update of the chosen solver.  Shared by the direct and the TMA-tiled kernels.
-template <int MODE, bool FACE>
-__device__ __forceinline__ void elem_apply(const double* __restrict__ pc, bool up, double T1, double T2, double T3,
-                                           const FaceIn& fi, double b1, double b2, double b3, double omega,
-                                           double rsign, double& o1, double& o2, double& o3) {
-  const double sg = up ? 1.0 : -1.0;
-  // ---- volume terms: (1/dt) M T - S T + K T
-  const double cm = __ldg(pc + PC_CM);
-  const double sumT = T1 + T2 + T3;
-  const double k11 = __ldg(pc + PC_K11), k12 = __ldg(pc + PC_K12), k13 = __ldg(pc + PC_K13);
-  const double k22 = __ldg(pc + PC_K22), k23 = __ldg(pc + PC_K23), k33 = __ldg(pc + PC_K33);
-  const double adv = sg * sumT;
-  const double mass1 = cm * (T1 + sumT), mass2 = cm * (T2 + sumT), mass3 = cm * (T3 + sumT);
-  const double st1 = __ldg(pc + PC_ADV + 0) * adv, st2 = __ldg(pc + PC_ADV + 1) * adv, st3 = __ldg(pc + PC_ADV + 2) * adv;
-  double ax1 = mass1 - st1 + (k11 * T1 + k12 * T2 + k13 * T3);
-  double ax2 = mass2 - st2 + (k12 * T1 + k22 * T2 + k23 * T3);
-  double ax3 = mass3 - st3 + (k13 * T1 + k23 * T2 + k33 * T3);
-  // ml/dt + K_ii (+ penalty diagonal below); ml = A/3 = 4 * A/12
-  double d1 = 4.0 * cm + k11, d2 = 4.0 * cm + k22, d3 = 4.0 * cm + k33;
-  double fx1 = 0.0, fx2 = 0.0, fx3 = 0.0;  // upwind flux, kept apart for Richardson (:516)
-  if (FACE) {
-    // penalty diffusion (k/dx) int sn_i (T - T2)  (matrices.F90:113-115, get_diff_surf_stencl :468-477):
-    // face mass (L/6)[[2,1],[1,2]] folded into pen = k (L/2) / (3 dx)
-    {
-      const double da = T1 - fi.n1a, db = T3 - fi.n1b;   // face 1: a = node 1, b = node 3
-      ax1 += fi.pen1 * (2.0 * da + db); ax3 += fi.pen1 * (da + 2.0 * db);
-      d1 += 2.0 * fi.pen1; d3 += 2.0 * fi.pen1;
-    }
-    {
-      const double da = T3 - fi.n2a, db = T2 - fi.n2b;   // face 2: a = node 3, b = node 2
-      ax3 += fi.pen2 * (2.0 * da + db); ax2 += fi.pen2 * (da + 2.0 * db);
-      d3 += 2.0 * fi.pen2; d2 += 2.0 * fi.pen2;
-    }
-    {
-      const double da = T2 - fi.n3a, db = T1 - fi.n3b;   // face 3: a = node 2, b = node 1
-      ax2 += fi.pen3 * (2.0 * da + db); ax1 += fi.pen3 * (da + 2.0 * db);
-      d2 += 2.0 * fi.pen3; d1 += 2.0 * fi.pen3;
-    }
-    // upwind flux: income = 1 when n.u < 0 (transport_tri_unstr.F90:729-738)
-    {
-      const double fl = sg * __ldg(pc + PC_FL + 0);
-      const bool in = fl < 0.0;
-      const double wa = in ? fi.n1a : T1, wb = in ? fi.n1b : T3;
-      fx1 += fl * (2.0 * wa + wb); fx3 += fl * (wa + 2.0 * wb);
-    }
-    {
-      const double fl = sg * __ldg(pc + PC_FL + 1);
-      const bool in = fl < 0.0;
-      const double wa = in ? fi.n2a : T3, wb = in ? fi.n2b : T2;
-      fx3 += fl * (2.0 * wa + wb); fx2 += fl * (wa + 2.0 * wb);
-    }
-    {
-      const double fl = sg * __ldg(pc + PC_FL + 2);
-      const bool in = fl < 0.0;
-      const double wa = in ? fi.n3a : T2, wb = in ? fi.n3b : T1;
-      fx2 += fl * (2.0 * wa + wb); fx1 += fl * (wa + 2.0 * wb);
-    }
-    ax1 += fx1; ax2 += fx2; ax3 += fx3;
-  }
-  if (MODE == MODE_RESID) {
-    o1 = rsign * (ax1 - b1); o2 = rsign * (ax2 - b2); o3 = rsign * (ax3 - b3);  // :869
-  } else if (MODE == MODE_RICH) {
-    // solve_Richardson (:511-518): omega * (b - (mass - stiff + flux))
-    o1 = T1 + omega * (b1 - (mass1 - st1 + fx1));
-    o2 = T2 + omega * (b2 - (mass2 - st2 + fx2));
-    o3 = T3 + omega * (b3 - (mass3 - st3 + fx3));
-  } else {
-    // solve_Jacobi (:491-497) / solve_Gauss_Seidel (:501-507)
-    o1 = T1 + omega / d1 * (b1 - ax1);
-    o2 = T2 + omega / d2 * (b2 - ax2);
-    o3 = T3 + omega / d3 * (b3 - ax3);
-  }
+// The in-parent neighbours of child c in row r (splitting.F90:749-769): across face 1 the child of the adjacent row (below
+// an up child, above a down child), whose index nbr1 returns; across face 2 the left child of an up child and the right
+// child of a down child (c -+ 1); across face 3 the other one of the two.
+__host__ __device__ __forceinline__ int nbr1(int c, bool up, int r, int b) { return up ? c - b - 2 + 2 * r : c + b - 2 * r; }
+
+// Which of that neighbour's nodes meet mine: across face F = 1, 2, 3 my face nodes (a, b) = (1,3), (3,2), (2,1) meet its
+// nodes (3,1), (2,3), (1,2).  ld(n) loads node n (0-based) of the neighbour's record.
+template <int F, class Ld>
+__device__ __forceinline__ void pair_face(Ld ld, double& va, double& vb) {
+  va = ld(F == 1 ? 2 : F == 2 ? 1 : 0);
+  vb = ld(F == 1 ? 0 : F == 2 ? 2 : 1);
+}
+// all three faces, the neighbours' records at v1, v2, v3
+__device__ __forceinline__ void pair_nodes(const double* v1, const double* v2, const double* v3, FaceIn& fi) {
+  pair_face<1>([&](int n) { return v1[n]; }, fi.n1a, fi.n1b);
+  pair_face<2>([&](int n) { return v2[n]; }, fi.n2a, fi.n2b);
+  pair_face<3>([&](int n) { return v3[n]; }, fi.n3a, fi.n3b);
+}
+
+// Up children on the parent boundary (surf_ele, splitting.F90:434-449): face 1 of a row-1 child lies on parent side 0 at
+// strip position ipos/2, face 2 of the first child of a row on side 2 and face 3 of the last child on side 1, both at
+// position r-1.  The apex child (len = 1) lies on both sides.
+__host__ __device__ __forceinline__ void face_on_side(int f, int r, int ipos, int& side, int& pos) {
+  side = f == 1 ? 0 : f == 2 ? 2 : 1;
+  pos = f == 1 ? ipos >> 1 : r - 1;
 }
 
 // Exterior values of a parent face WITHOUT a halo strip.  update_overlaps (splitting.F90:1255-1391) copies the nodal values
@@ -227,6 +179,14 @@ __device__ __forceinline__ void ext_pair(const ElemArgs& a, int d, int strip, in
 __device__ __forceinline__ void halo_pair(const ElemArgs& a, int u, int mf, int slot0, int S, double& va, double& vb) {
   const int d = a.nsrc ? __ldg(a.nsrc + u * 3 + mf) : -1;
   ext_pair(a, d, __ldg(a.strip_of + u * 3 + mf), __ldg(a.hmap + u * 3 + mf), slot0, S, va, vb);
+}
+
+// exterior values across face f of an up child on the parent boundary; ix(j): entry j of the parent's index table
+template <class Ix>
+__device__ __forceinline__ void ext_face(const ElemArgs& a, int f, int r, int ipos, int S, Ix ix, double& va, double& vb) {
+  int side, pos;
+  face_on_side(f, r, ipos, side, pos);
+  ext_pair(a, ix(8 + side), ix(side), ix(4 + side), pos, S, va, vb);
 }
 
 // a sweep that sent exchange e64 + 1 from its producer warps: the last CTA to finish advances the level's exchange number
@@ -296,6 +256,21 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+
+// the contiguous range of tiles [tbeg, tend) this CTA owns
+__device__ __forceinline__ void cta_tiles(long long ntiles, long long& tbeg, long long& tend) {
+  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;
+  tbeg = (long long)blockIdx.x * per;
+  tend = min(ntiles, tbeg + per);
+}
+
+// one tile (TPB children, 6 KB) of src into slot sl of a shared-memory ring, completing on bar[sl]
+constexpr uint32_t TILE_BYTES = 3 * TPB * sizeof(double);
+__device__ __forceinline__ void load_tile(double* ring, uint64_t* bar, int sl, const double* src, long long tile) {
+  mbar_expect_tx(&bar[sl], TILE_BYTES);
+  tma_load_1d(ring + sl * 3 * TPB, src + tile * 3 * TPB, TILE_BYTES, &bar[sl]);
+}
 
 // memory-order child index k (0-based) -> row, position.  Row r starts at m(b-m), m = r-1; the float sqrt
 // guess is off by at most one, fixed with two predicated corrections (no loops, no divergence).
@@ -332,14 +307,42 @@ struct ParentRegs {
   double px1, px2, px3;   // penalty coefficients of faces on the parent boundary
 };
 static_assert(sizeof(ParentRegs) == 22 * sizeof(double), "ParentRegs must mirror the pc table");
-__device__ __forceinline__ void load_parent(const double* __restrict__ pc, ParentRegs& P) {
-  double* d = reinterpret_cast<double*>(&P);
-#pragma unroll
-  for (int i = 0; i < 22; ++i) d[i] = __ldg(pc + i);
+
+// parent u's coefficients (NPC doubles) and, with sIdx, its index table (strip_of at 0..2, hmap at 4..6, nsrc at 8..10)
+// into shared memory, one entry per thread of the CTA
+__device__ __forceinline__ void load_parent_cta(const ElemArgs& a, int u, int tid, double* sPC, int* sIdx = nullptr) {
+  if (tid < NPC) sPC[tid] = __ldg(a.pc + (size_t)u * NPC + tid);
+  else if (sIdx) {
+    if (tid < NPC + 3) sIdx[tid - NPC] = __ldg(a.strip_of + u * 3 + (tid - NPC));
+    else if (tid < NPC + 6) sIdx[4 + tid - NPC - 3] = __ldg(a.hmap + u * 3 + (tid - NPC - 3));
+    else if (tid < NPC + 9) sIdx[8 + tid - NPC - 6] = a.nsrc ? __ldg(a.nsrc + u * 3 + (tid - NPC - 6)) : -1;
+  }
+}
+
+// An up child on parent faces (face_on_side) takes the exterior values of each such face, ext(f, side, pos, va, vb), and
+// its boundary penalty px instead of the in-parent neighbour's values and pi.  Returns the mask of those faces (bit f-1).
+template <class Ext>
+__device__ __forceinline__ int parent_faces(int r, int ipos, int len, const ParentRegs& P, Ext ext, FaceIn& fi) {
+  int bmask = 0, side, pos;
+  if (r == 1) { face_on_side(1, r, ipos, side, pos); ext(1, side, pos, fi.n1a, fi.n1b); fi.pen1 = P.px1; bmask |= 1; }
+  if (ipos == 1) { face_on_side(2, r, ipos, side, pos); ext(2, side, pos, fi.n2a, fi.n2b); fi.pen2 = P.px2; bmask |= 2; }
+  if (ipos == len) { face_on_side(3, r, ipos, side, pos); ext(3, side, pos, fi.n3a, fi.n3b); fi.pen3 = P.px3; bmask |= 4; }
+  return bmask;
+}
+// the same in a window kernel, which fetched the values a tile ahead (h1 across face 1, h2 across the side face); the apex
+// child lies on both sides and fetches side 1 now
+__device__ __forceinline__ int parent_faces_fetched(const ElemArgs& a, int u, int r, int ipos, int len, int S,
+                                                    const ParentRegs& P, double h1a, double h1b, double h2a, double h2b,
+                                                    FaceIn& fi) {
+  return parent_faces(r, ipos, len, P, [&](int f, int side, int pos, double& va, double& vb) {
+    if (f == 1) { va = h1a; vb = h1b; }
+    else if (f == 3 && len == 1) halo_pair(a, u, side, pos, S, va, vb);
+    else { va = h2a; vb = h2b; }
+  }, fi);
 }
 
 // Folded operator of a child whose three faces are inside the parent, one set per orientation (up / down).
-// Everything elem_apply adds up term by term is linear in (T, neighbour values), so for such children
+// Everything elem_apply_regs adds up term by term is linear in (T, neighbour values), so for such children
 //   (A x)_i = sum_j a_ij T_j + sum_f c_f [[2,1],[1,2]] (n_fa, n_fb)
 // with a_ij = mass + advection + diffusion + penalty + outflow flux and c_f = -pen_f (+ inflow flux).
 // The host folds the coefficients once per parent and level (fold_coefficients in pamg_api.cu); the kernels
@@ -379,7 +382,8 @@ __device__ __forceinline__ void elem_apply_folded(const Folded& F, const double*
   }
 }
 
-// Same arithmetic as elem_apply, coefficients from registers; `interior` children (no face on the parent
+// One child: A x (get_A_x, transport_tri_semi.F90:412-448, theta = 1), the diagonal (get_diagonal :481-486) and the
+// update of the chosen solver, term by term with the parent's coefficients; `interior` children (no face on the parent
 // boundary) use the precomputed omega / D.
 template <int MODE, bool FACE>
 __device__ __forceinline__ void elem_apply_regs(const ParentRegs& P, bool up, bool interior, double T1, double T2,
@@ -446,10 +450,6 @@ __device__ __forceinline__ void elem_apply_regs(const ParentRegs& P, bool up, bo
   }
 }
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
 // Pipelined 1-D TMA tile kernel.  Every CTA owns a CONTIGUOUS range of tiles (so it stays inside one parent
 // for hundreds of tiles and the vertical neighbours it needs were touched by itself a moment ago); NSTAGE
 // tiles are in flight through a ring of shared-memory stages, each filled by two bulk copies that complete
@@ -472,7 +472,7 @@ __global__ void __launch_bounds__(TPB, 3) k_element_tma(ElemArgs a) {
   double acc_sum = 0.0, acc_abs = 0.0, acc_max = 0.0;
   if (tid == 0) {
     for (int i = 0; i < NSTAGE; ++i) mbar_init(&bar[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   const long long ntiles = (a.nelem + TPB - 1) / TPB;
@@ -505,14 +505,16 @@ __global__ void __launch_bounds__(TPB, 3) k_element_tma(ElemArgs a) {
     child_from_ele0(k, s, p.r, p.ipos, p.len);
     p.up = p.ipos & 1;
     if (FACE && !(MODE == MODE_GS && (int)p.up != a.colour)) {
-      // vertical neighbour: child above for a down child, child below for an up child (splitting.F90:749-769);
-      // up children of row 1 sit on parent face 1 and read the halo strip instead
-      const int nb = p.up ? (k - b - 2 + 2 * p.r) : (k + b - 2 * p.r);       // 0-based child index
+      // the neighbour across face 1 is a global load: fetched a tile ahead; up children of row 1 sit on parent side 0
+      // and read the halo strip instead
+      const int nb = nbr1(k, p.up, p.r, b);                          // 0-based child index
       if (p.up && p.r == 1) {
-        halo_pair(a, p.u, 0, p.ipos >> 1, S, p.va, p.vb);
+        int side, pos;
+        face_on_side(1, p.r, p.ipos, side, pos);
+        halo_pair(a, p.u, side, pos, S, p.va, p.vb);
       } else {
         const unsigned o1 = ((unsigned)(g - k) + (unsigned)nb) * 3u;         // offsets in doubles fit 32 bits
-        p.va = __ldg(a.Tin + o1 + 2); p.vb = __ldg(a.Tin + o1);
+        pair_face<1>([&](int n) { return __ldg(a.Tin + o1 + n); }, p.va, p.vb);
       }
     }
   };
@@ -531,7 +533,7 @@ __global__ void __launch_bounds__(TPB, 3) k_element_tma(ElemArgs a) {
       const int u_tile = (int)(g0 >> twos);          // uniform over the CTA (a tile never spans two parents)
       if (u_tile != u_loaded) {
         __syncthreads();
-        if (tid < NPC) sPC[tid] = __ldg(a.pc + (size_t)u_tile * NPC + tid);
+        load_parent_cta(a, u_tile, tid, sPC);
         __syncthreads();
         u_loaded = u_tile;
       }
@@ -605,6 +607,15 @@ constexpr int WIN_NB = 4;                    // rhs / output tiles (power of two
 constexpr int WIN_CH = WIN_NT * TPB;
 constexpr size_t WIN_SMEM_BYTES = sizeof(double) * 3 * TPB * (WIN_NT + WIN_NB) + 8 * (WIN_NT + WIN_NB) + 64;
 __device__ __forceinline__ void tma_store_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
+__device__ __forceinline__ void tma_store_wait_read2() { asm volatile("cp.async.bulk.wait_group.read 2;" ::: "memory"); }
+
+// the in-parent neighbours (nbr1) of the child at ring index cw
+__device__ __forceinline__ void ring_nbrs(const double* sT, int cw, bool up, int r, int b, FaceIn& fi) {
+  const double* tv = sT + (nbr1(cw, up, r, b) & (WIN_CH - 1)) * 3;
+  const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
+  const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
+  pair_nodes(tv, up ? tl : tr, up ? tr : tl, fi);
+}
 
 template <int MODE, bool FACE>
 __global__ void __launch_bounds__(TPB, 3) k_element_win(ElemArgs a) {
@@ -618,28 +629,19 @@ __global__ void __launch_bounds__(TPB, 3) k_element_win(ElemArgs a) {
   const int s = a.s, twos = 2 * s, b = 2 << s, S = 1 << s;
   const long long Cmask = (1ll << twos) - 1;
   const int tid = threadIdx.x;
-  constexpr uint32_t TILE_BYTES = 3 * TPB * sizeof(double);
   double acc_sum = 0.0, acc_abs = 0.0, acc_max = 0.0;
   if (tid == 0) {
     for (int i = 0; i < WIN_NT + WIN_NB; ++i) mbar_init(&barT[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   const long long ntiles = a.nelem / TPB;                 // the host only launches this kernel when TPB | 4^s
-  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;
-  const long long tbeg = (long long)blockIdx.x * per, tend = min(ntiles, tbeg + per);
+  long long tbeg, tend;
+  cta_tiles(ntiles, tbeg, tend);
   const long long tlo = max(0ll, tbeg - 2), thi = min(ntiles, tend + 2);
 
-  auto issueT = [&](long long tile) {   // tid 0 only
-    const int sl = (int)(tile & (WIN_NT - 1));
-    mbar_expect_tx(&barT[sl], TILE_BYTES);
-    tma_load_1d(sT + sl * 3 * TPB, a.Tin + tile * 3 * TPB, TILE_BYTES, &barT[sl]);
-  };
-  auto issueB = [&](long long tile) {
-    const int sl = (int)((tile - tbeg) & (WIN_NB - 1));
-    mbar_expect_tx(&barB[sl], TILE_BYTES);
-    tma_load_1d(sB + sl * 3 * TPB, a.rhs + tile * 3 * TPB, TILE_BYTES, &barB[sl]);
-  };
+  auto issueT = [&](long long tile) { load_tile(sT, barT, (int)(tile & (WIN_NT - 1)), a.Tin, tile); };   // tid 0 only
+  auto issueB = [&](long long tile) { load_tile(sB, barB, (int)((tile - tbeg) & (WIN_NB - 1)), a.rhs, tile); };
   if (tid == 0 && tbeg < tend) {
     for (long long t = tlo; t < min(thi, tbeg + 5); ++t) issueT(t);
     for (long long t = tbeg; t < min(tend, tbeg + 2); ++t) issueB(t);
@@ -715,17 +717,7 @@ __global__ void __launch_bounds__(TPB, 3) k_element_win(ElemArgs a) {
         const ParentRegs& P = *reinterpret_cast<const ParentRegs*>(sPC);
         if (FACE) {
           fi.pen1 = P.pi1; fi.pen2 = P.pi2; fi.pen3 = P.pi3;
-          // vertical neighbour: child above for a down child, child below for an up child (splitting.F90:749-769)
-          const int dv = up ? (2 * cur.r - b - 2) : (b - 2 * cur.r);
-          const double* tv = sT + ((cw + dv) & (WIN_CH - 1)) * 3;
-          fi.n1a = tv[2]; fi.n1b = tv[0];
-          // face 2 looks left for an up child and right for a down child, face 3 the other way
-          const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-          const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-          const double* t2 = up ? tl : tr;
-          const double* t3 = up ? tr : tl;
-          fi.n2a = t2[1]; fi.n2b = t2[2];
-          fi.n3a = t3[0]; fi.n3b = t3[1];
+          ring_nbrs(sT, cw, up, cur.r, b, fi);
           if (up && (cur.r == 1 || cur.ipos == 1 || cur.ipos == cur.len)) {   // child on a parent face (rare)
             interior = false;
             if (cur.r == 1) { fi.n1a = cur.h1a; fi.n1b = cur.h1b; fi.pen1 = P.px1; bmask |= 1; }
@@ -856,16 +848,15 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_element_win2(ElemArgs a) {
   const int s = a.s, twos = 2 * s, b = 2 << s, S = 1 << s;
   const long long Cmask = (1ll << twos) - 1;
   const int tid = threadIdx.x;
-  constexpr uint32_t TILE_BYTES = 3 * TPB * sizeof(double);
   double acc_sum = 0.0, acc_abs = 0.0, acc_max = 0.0;
   if (tid == 0) {
     for (int i = 0; i < WIN_NT + WIN_NB; ++i) mbar_init(&barT[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   const long long ntiles = a.nelem / TPB;
-  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;
-  const long long tbeg = (long long)blockIdx.x * per, tend = min(ntiles, tbeg + per);
+  long long tbeg, tend;
+  cta_tiles(ntiles, tbeg, tend);
   const long long tlo = max(0ll, tbeg - 2), thi = min(ntiles, tend + 2);
 
   if (tid >= TPB) {
@@ -875,11 +866,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_element_win2(ElemArgs a) {
     // exchange number of the cut-face values this sweep READS (the sweep or k_halo before it sent them); it sends e64 + 1
     unsigned long long e64 = 0;
     if (XCHG) e64 = *(volatile unsigned long long*)(a.xsync + P2P_EPOCH);
-    auto issueT = [&](long long tile) {   // lane 0
-      const int sl = (int)(tile & (WIN_NT - 1));
-      mbar_expect_tx(&barT[sl], TILE_BYTES);
-      tma_load_1d(sT + sl * 3 * TPB, a.Tin + tile * 3 * TPB, TILE_BYTES, &barT[sl]);
-    };
+    auto issueT = [&](long long tile) { load_tile(sT, barT, (int)(tile & (WIN_NT - 1)), a.Tin, tile); };   // lane 0
     auto issueB = [&](long long tile) {   // whole warp: a new parent's coefficients go out with its first rhs tile
       const int u = (int)((tile * TPB) >> twos);
       if (u != u_loaded) {
@@ -891,11 +878,8 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_element_win2(ElemArgs a) {
         u_loaded = u;
         __syncwarp();
       }
-      if (lane == 0) {
-        const int sl = (int)((tile - tbeg) & (WIN_NB - 1));
-        mbar_expect_tx(&barB[sl], TILE_BYTES);    // release: the coefficient writes above are visible to whoever waits on it
-        tma_load_1d(sB + sl * 3 * TPB, a.rhs + tile * 3 * TPB, TILE_BYTES, &barB[sl]);
-      }
+      // (the expect_tx releases the coefficient writes above to whoever waits on the tile)
+      if (lane == 0) load_tile(sB, barB, (int)((tile - tbeg) & (WIN_NB - 1)), a.rhs, tile);
     };
     if (tbeg < tend) {
       if (lane == 0) for (long long t = tlo; t < min(thi, tbeg + 6); ++t) issueT(t);
@@ -984,15 +968,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_element_win2(ElemArgs a) {
         const ParentRegs& P = *reinterpret_cast<const ParentRegs*>(sPC);
         if (FACE) {
           fi.pen1 = P.pi1; fi.pen2 = P.pi2; fi.pen3 = P.pi3;
-          const int dv = up ? (2 * cur.r - b - 2) : (b - 2 * cur.r);
-          const double* tv = sT + ((cw + dv) & (WIN_CH - 1)) * 3;
-          fi.n1a = tv[2]; fi.n1b = tv[0];
-          const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-          const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-          const double* t2 = up ? tl : tr;
-          const double* t3 = up ? tr : tl;
-          fi.n2a = t2[1]; fi.n2b = t2[2];
-          fi.n3a = t3[0]; fi.n3b = t3[1];
+          ring_nbrs(sT, cw, up, cur.r, b, fi);
           if (up && (cur.r == 1 || cur.ipos == 1 || cur.ipos == cur.len)) {
             interior = false;
             if (cur.r == 1) { fi.n1a = cur.h1a; fi.n1b = cur.h1b; fi.pen1 = P.px1; bmask |= 1; }
@@ -1060,7 +1036,6 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_element_win2(ElemArgs a) {
 // halo strips) with 24 B/DOF of traffic instead of 48.  A CTA relaxes the down children of the two tiles before
 // and the one tile after its own range redundantly (in shared memory only) so that CTAs stay independent.
 constexpr size_t GSW_SMEM_BYTES = WIN_SMEM_BYTES;
-__device__ __forceinline__ void tma_store_wait_read2() { asm volatile("cp.async.bulk.wait_group.read 2;" ::: "memory"); }
 
 __global__ void __launch_bounds__(TPB, 3) k_gs_win(ElemArgs a) {
   extern __shared__ __align__(128) unsigned char dsm[];
@@ -1074,30 +1049,21 @@ __global__ void __launch_bounds__(TPB, 3) k_gs_win(ElemArgs a) {
   const int s = a.s, twos = 2 * s, b = 2 << s, S = 1 << s;
   const long long Cmask = (1ll << twos) - 1;
   const int tid = threadIdx.x;
-  constexpr uint32_t TILE_BYTES = 3 * TPB * sizeof(double);
   if (tid == 0) {
     for (int i = 0; i < WIN_NT + WIN_NB; ++i) mbar_init(&barT[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   const long long ntiles = a.nelem / TPB;
-  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;
-  const long long tbeg = (long long)blockIdx.x * per, tend = min(ntiles, tbeg + per);
+  long long tbeg, tend;
+  cta_tiles(ntiles, tbeg, tend);
   if (tbeg >= tend) return;
   const long long dlo = max(0ll, tbeg - 2), dhi = min(ntiles - 1, tend);       // tiles whose down children I relax
   const long long tlo = max(0ll, dlo - 1), thi = min(ntiles, dhi + 3);         // field tiles I load: [tlo, thi)
   const long long t0 = dlo - 2;                                                // first iteration
 
-  auto issueT = [&](long long tile) {
-    const int sl = (int)(tile & (WIN_NT - 1));
-    mbar_expect_tx(&barT[sl], TILE_BYTES);
-    tma_load_1d(sT + sl * 3 * TPB, a.Tin + tile * 3 * TPB, TILE_BYTES, &barT[sl]);
-  };
-  auto issueB = [&](long long tile) {
-    const int sl = (int)((tile - dlo) & (WIN_NB - 1));
-    mbar_expect_tx(&barB[sl], TILE_BYTES);
-    tma_load_1d(sB + sl * 3 * TPB, a.rhs + tile * 3 * TPB, TILE_BYTES, &barB[sl]);
-  };
+  auto issueT = [&](long long tile) { load_tile(sT, barT, (int)(tile & (WIN_NT - 1)), a.Tin, tile); };
+  auto issueB = [&](long long tile) { load_tile(sB, barB, (int)((tile - dlo) & (WIN_NB - 1)), a.rhs, tile); };
   auto waitT = [&](long long tile) { mbar_wait(&barT[tile & (WIN_NT - 1)], (uint32_t)(((tile - tlo) >> 3) & 1)); };
   auto waitB = [&](long long tile) { mbar_wait(&barB[(tile - dlo) & (WIN_NB - 1)], (uint32_t)(((tile - dlo) >> 2) & 1)); };
   if (tid == 0) {
@@ -1146,12 +1112,7 @@ __global__ void __launch_bounds__(TPB, 3) k_gs_win(ElemArgs a) {
       const int uu = doU ? (int)((tile * TPB) >> twos) : u_up;
       if (ud != u_dn || uu != u_up) {                    // uniform over the CTA
         __syncthreads();
-        if (uu != u_up) {
-          if (tid < NPC) sPC[tid] = __ldg(a.pc + (size_t)uu * NPC + tid);
-          else if (tid < NPC + 3) sIdx[tid - NPC] = __ldg(a.strip_of + uu * 3 + (tid - NPC));
-          else if (tid < NPC + 6) sIdx[4 + tid - NPC - 3] = __ldg(a.hmap + uu * 3 + (tid - NPC - 3));
-          else if (tid < NPC + 9) sIdx[8 + tid - NPC - 6] = a.nsrc ? __ldg(a.nsrc + uu * 3 + (tid - NPC - 6)) : -1;
-        }
+        if (uu != u_up) load_parent_cta(a, uu, tid, sPC, sIdx);
         if (ud != u_dn && tid >= 128 && tid < 144) sPD[tid - 128] = __ldg(a.pc + (size_t)ud * NPC + PC_FOLD + 16 + (tid - 128));
         __syncthreads();
         u_dn = ud; u_up = uu;
@@ -1173,12 +1134,7 @@ __global__ void __launch_bounds__(TPB, 3) k_gs_win(ElemArgs a) {
         double* t = sT + cw * 3;
         const double T1 = t[0], T2 = t[1], T3 = t[2];
         FaceIn fi;
-        const double* tv = sT + ((cw + b - 2 * r) & (WIN_CH - 1)) * 3;      // up child of the row above
-        fi.n1a = tv[2]; fi.n1b = tv[0];
-        const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-        const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-        fi.n2a = tr[1]; fi.n2b = tr[2];
-        fi.n3a = tl[0]; fi.n3b = tl[1];
+        ring_nbrs(sT, cw, false, r, b, fi);
         const double* bb = sB + ((td - dlo) & (WIN_NB - 1)) * 3 * TPB + tid * 3;
         const Folded& F = *reinterpret_cast<const Folded*>(sPD);
         double o1, o2, o3;
@@ -1194,21 +1150,10 @@ __global__ void __launch_bounds__(TPB, 3) k_gs_win(ElemArgs a) {
         const double T1 = t[0], T2 = t[1], T3 = t[2];
         FaceIn fi;
         int bmask = 0;
-        const double* tv = sT + ((cw + 2 * cur.r - b - 2) & (WIN_CH - 1)) * 3;   // down child of the row below
-        fi.n1a = tv[2]; fi.n1b = tv[0];
-        const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-        const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-        fi.n2a = tl[1]; fi.n2b = tl[2];
-        fi.n3a = tr[0]; fi.n3b = tr[1];
-        if (cur.r == 1 || cur.ipos == 1 || cur.ipos == cur.len) {               // child on a parent face (rare)
-          if (cur.r == 1) { fi.n1a = cur.h1a; fi.n1b = cur.h1b; bmask |= 1; }
-          if (cur.ipos == 1) { fi.n2a = cur.h2a; fi.n2b = cur.h2b; bmask |= 2; }
-          if (cur.ipos == cur.len) {
-            if (cur.len == 1) halo_pair(a, (int)((tile * TPB) >> twos), 1, cur.r - 1, S, fi.n3a, fi.n3b);
-            else { fi.n3a = cur.h2a; fi.n3b = cur.h2b; }
-            bmask |= 4;
-          }
-        }
+        ring_nbrs(sT, cw, true, cur.r, b, fi);
+        if (cur.r == 1 || cur.ipos == 1 || cur.ipos == cur.len)               // child on a parent face (rare)
+          bmask = parent_faces_fetched(a, (int)((tile * TPB) >> twos), cur.r, cur.ipos, cur.len, S,
+                                       *reinterpret_cast<const ParentRegs*>(sPC), cur.h1a, cur.h1b, cur.h2a, cur.h2b, fi);
         const double* bb = sB + ((tile - dlo) & (WIN_NB - 1)) * 3 * TPB + tid * 3;
         const Folded& F = *reinterpret_cast<const Folded*>(sPC + PC_FOLD);
         double o1, o2, o3;
@@ -1250,16 +1195,15 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
   const int s = a.s, twos = 2 * s, b = 2 << s, S = 1 << s;
   const long long Cmask = (1ll << twos) - 1;
   const int tid = threadIdx.x;
-  constexpr uint32_t TILE_BYTES = 3 * TPB * sizeof(double);
   if (tid == 0) {
     for (int i = 0; i < WIN_NT + WIN_NB; ++i) mbar_init(&barT[i], 1);
     for (int i = 0; i < 4; ++i) mbar_init(&doneD[i], TPB / 64);   // the four down warps
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   __syncthreads();
   const long long ntiles = a.nelem / TPB;
-  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;
-  const long long tbeg = (long long)blockIdx.x * per, tend = min(ntiles, tbeg + per);
+  long long tbeg, tend;
+  cta_tiles(ntiles, tbeg, tend);
   if (tbeg >= tend) {
     if (XCHG && tid == TPB) p2p_advance(a.xsync, *(volatile unsigned long long*)(a.xsync + P2P_EPOCH));
     return;
@@ -1274,11 +1218,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
     int u_loaded = -1;
     unsigned long long e64 = 0;                          // exchange number this sweep reads (see k_element_win2)
     if (XCHG) e64 = *(volatile unsigned long long*)(a.xsync + P2P_EPOCH);
-    auto issueT = [&](long long tile) {
-      const int sl = (int)(tile & (WIN_NT - 1));
-      mbar_expect_tx(&barT[sl], TILE_BYTES);
-      tma_load_1d(sT + sl * 3 * TPB, a.Tin + tile * 3 * TPB, TILE_BYTES, &barT[sl]);
-    };
+    auto issueT = [&](long long tile) { load_tile(sT, barT, (int)(tile & (WIN_NT - 1)), a.Tin, tile); };
     auto issueB = [&](long long tile) {   // whole warp
       const int u = (int)((tile * TPB) >> twos);
       if (u != u_loaded) {
@@ -1290,11 +1230,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
         u_loaded = u;
         __syncwarp();
       }
-      if (lane == 0) {
-        const int sl = (int)((tile - dlo) & (WIN_NB - 1));
-        mbar_expect_tx(&barB[sl], TILE_BYTES);
-        tma_load_1d(sB + sl * 3 * TPB, a.rhs + tile * 3 * TPB, TILE_BYTES, &barB[sl]);
-      }
+      if (lane == 0) load_tile(sB, barB, (int)((tile - dlo) & (WIN_NB - 1)), a.rhs, tile);
     };
     if (lane == 0) for (long long t = tlo; t < min(thi, t0 + 6); ++t) issueT(t);
     for (long long t = dlo; t <= min(dhi, dlo + 3); ++t) issueB(t);
@@ -1309,7 +1245,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
           tma_store_commit();
         }
         // ring slot of tile-2: nobody is behind iteration tile+1; its store (two groups ago) has been read
-        if (tile + 6 < thi) { asm volatile("cp.async.bulk.wait_group.read 2;" ::: "memory"); issueT(tile + 6); }
+        if (tile + 6 < thi) { tma_store_wait_read2(); issueT(tile + 6); }
       }
       __syncwarp();
       if (tile + 4 >= dlo + 4 && tile + 4 <= dhi) issueB(tile + 4);   // rhs slot of tile: consumed by its up children
@@ -1345,12 +1281,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
       const double T1 = t[0], T2 = t[1], T3 = t[2];
       FaceIn fi;
       int bmask = 0;
-      const double* tv = sT + ((cw + 2 * rr - b - 2) & (WIN_CH - 1)) * 3;
-      fi.n1a = tv[2]; fi.n1b = tv[0];
-      const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-      const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-      fi.n2a = tl[1]; fi.n2b = tl[2];
-      fi.n3a = tr[0]; fi.n3b = tr[1];
+      ring_nbrs(sT, cw, true, rr, b, fi);
       if (rr == 1 || ip == 1 || ip == ln) {
         if (rr == 1) { fi.n1a = h1a; fi.n1b = h1b; bmask |= 1; }
         if (ip == 1) { fi.n2a = h2a; fi.n2b = h2b; bmask |= 2; }
@@ -1397,12 +1328,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
             double* t = sT + cw * 3;
             const double T1 = t[0], T2 = t[1], T3 = t[2];
             FaceIn fi;
-            const double* tv = sT + ((cw + b - 2 * r) & (WIN_CH - 1)) * 3;
-            fi.n1a = tv[2]; fi.n1b = tv[0];
-            const double* tr = sT + ((cw + 1) & (WIN_CH - 1)) * 3;
-            const double* tl = sT + ((cw - 1) & (WIN_CH - 1)) * 3;
-            fi.n2a = tr[1]; fi.n2b = tr[2];
-            fi.n3a = tl[0]; fi.n3b = tl[1];
+            ring_nbrs(sT, cw, false, r, b, fi);
             const double* bb = sB + ((td - dloi) & (WIN_NB - 1)) * (3 * TPB) + (j2 + off) * 3;
             const double* pd = sPC2[(td >> pshift) & 1] + PC_FOLD + 16;
             const Folded& F = *reinterpret_cast<const Folded*>(pd);
@@ -1411,7 +1337,7 @@ __global__ void __launch_bounds__(WIN2_THREADS, 3) k_gs_win2(ElemArgs a) {
             t[0] = o1; t[1] = o2; t[2] = o3;
           } else if (td >= tbegi && td < tendi) {
             const int* ix = sIdx2[(td >> pshift) & 1];
-            ext_pair(a, ix[10], ix[2], ix[6], r, S, nsec_a, nsec_b);   // side 3 at the position of row r+1
+            ext_face(a, 2, r + 1, 1, S, [&](int j) { return ix[j]; }, nsec_a, nsec_b);   // first child of row r+1
             nsec = true;
           }
         }
@@ -1503,15 +1429,15 @@ __device__ __forceinline__ void child_update(const ElemArgs& a, int u, int r, in
   if (FACE) {
     const unsigned o1 = (pbase + (unsigned)(nb1 - 1)) * 3u, o2 = (pbase + (unsigned)(nb2 - 1)) * 3u,
                    o3 = (pbase + (unsigned)(nb3 - 1)) * 3u;
-    fi.n1a = ldT(o1 + 2); fi.n1b = ldT(o1);        // my node 1 <-> its node 3, my node 3 <-> its node 1
-    fi.n2a = ldT(o2 + 1); fi.n2b = ldT(o2 + 2);    // my 3 <-> its 2, my 2 <-> its 3
-    fi.n3a = ldT(o3); fi.n3b = ldT(o3 + 1);        // my 2 <-> its 1, my 1 <-> its 2
+    pair_face<1>([&](int n) { return ldT(o1 + n); }, fi.n1a, fi.n1b);
+    pair_face<2>([&](int n) { return ldT(o2 + n); }, fi.n2a, fi.n2b);
+    pair_face<3>([&](int n) { return ldT(o3 + n); }, fi.n3a, fi.n3b);
     fi.pen1 = P.pi1; fi.pen2 = P.pi2; fi.pen3 = P.pi3;
     if (up && (r == 1 || ipos == 1 || ipos == len)) {   // child on a parent face (rare): halo strips
       interior = false;
-      if (r == 1) { halo_pair(a, u, 0, ipos >> 1, S, fi.n1a, fi.n1b); fi.pen1 = P.px1; bmask |= 1; }
-      if (ipos == 1) { halo_pair(a, u, 2, r - 1, S, fi.n2a, fi.n2b); fi.pen2 = P.px2; bmask |= 2; }
-      if (ipos == len) { halo_pair(a, u, 1, r - 1, S, fi.n3a, fi.n3b); fi.pen3 = P.px3; bmask |= 4; }
+      bmask = parent_faces(r, ipos, len, P, [&](int, int side, int pos, double& va, double& vb) {
+        halo_pair(a, u, side, pos, S, va, vb);
+      }, fi);
     }
   }
   double o1v, o2v, o3v;
@@ -1586,12 +1512,7 @@ __global__ void __launch_bounds__(TPB) k_gs_small(ElemArgs a) {
     const double* P0 = sT + (lu << twos) * 3;           // my parent's children
     if (active && !up) {
       const double T1 = t[0], T2 = t[1], T3 = t[2];
-      const double* tv = P0 + (k + b - 2 * r) * 3;
-      const double* tr = P0 + (k + 1) * 3;
-      const double* tl = P0 + (k - 1) * 3;
-      fi.n1a = tv[2]; fi.n1b = tv[0];
-      fi.n2a = tr[1]; fi.n2b = tr[2];
-      fi.n3a = tl[0]; fi.n3b = tl[1];
+      pair_nodes(P0 + nbr1(k, false, r, b) * 3, P0 + (k + 1) * 3, P0 + (k - 1) * 3, fi);
       const Folded& F = *reinterpret_cast<const Folded*>(pcu + PC_FOLD + 16);
       double o1, o2, o3;
       elem_apply_folded<MODE_GS>(F, pcu + PC_DPEN, 0, T1, T2, T3, fi, b1, b2, b3, a.rsign, o1, o2, o3);
