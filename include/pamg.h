@@ -195,6 +195,16 @@ int pamg_comm_init(pamg_handle* h, const char* id128, int nranks, int rank);
 int pamg_halo_peer_count(const pamg_handle* h, int* npeers);
 int pamg_halo_peer_info(const pamg_handle* h, int idx, int* peer_part, int* nfaces);
 
+/* host-only: flow levels of an upwind graph (the function pamg_implicit_set_precond's sweep uses).  Edge c -> e for every face
+ * f of e with bit f of inflow_mask[e] set and a neighbour c = neig[e][f] - 1 (neig [E][3], 1-based, 0 = boundary).  level[e] =
+ * the longest upwind path ending at e (Kahn's algorithm, O(E)); order [E] = the elements sorted by (level, index).  A cycle:
+ * when no element is left whose upstream neighbours all have a level, the lowest-index element left gets 1 + the largest
+ * level of its upstream neighbours that have one (0 if none), and its other upstream edges are lagged.  lagged = the number
+ * of edges (c, e) with level[c] >= level[e]: 0 for an acyclic graph.  nlevels = 1 + the largest level; nlevels and lagged
+ * may be NULL. */
+int pamg_flow_levels(int E, const int32_t* neig, const int32_t* inflow_mask, int32_t* level, int32_t* order,
+                     int32_t* nlevels, int64_t* lagged);
+
 /* ---- unstructured explicit DG step (unstr_explicit, transport_tri_unstr.F90:588-795) ------------ */
 int pamg_set_unstructured(pamg_handle* h, int E, const double* X, const int32_t* neig, const int32_t* fneig);
 int pamg_unstr_upload(pamg_handle* h, const double* tnew /* (3,E) */);
@@ -227,14 +237,40 @@ int pamg_implicit_assemble(pamg_handle* h, double dt, double u_x, double u_y, in
 int pamg_implicit_assemble_diffusion(pamg_handle* h, double dt, double u_x, double u_y, double k, int use_dir);
 int pamg_implicit_get_bsr(pamg_handle* h, double* val /* [E][4][9] or NULL */, int32_t* col /* [E][4], 0-based, -1 = none, or NULL */);
 int pamg_implicit_apply(pamg_handle* h, const double* x /* host (3,E) */, double* y /* host: (lhs + flux) x */);
-/* ntime x nits passes of: told = tnew ; solve (lhs + flux) tnew = (M/dt) told by block-Jacobi-preconditioned
- * BiCGStab to ||r|| <= tol ||rhs|| (at most max_iters iterations per solve).  iters_total / relres (worst solve)
- * may be NULL. */
+/* ntime x nits passes of: told = tnew ; solve (lhs + flux) tnew = (M/dt) told by BiCGStab, right-preconditioned with the
+ * preconditioner of pamg_implicit_set_precond (block Jacobi by default), to ||r|| <= tol ||rhs|| (at most max_iters
+ * iterations per solve).  iters_total / relres (worst solve) may be NULL. */
 int pamg_implicit_step(pamg_handle* h, int ntime, int nits, double tol, int max_iters, int* iters_total, double* relres);
 /* measurement aids: average device time (ms) of `reps` block-CSR products; host synchronisations of the Krylov solves so far
  * (the scalars of the recurrence live on the device: one look at the convergence flag per 16 iterations) */
 int pamg_implicit_spmv_time(pamg_handle* h, int reps, float* ms);
 int pamg_implicit_host_syncs(pamg_handle* h, int64_t* n);
+
+/* ---- preconditioner of the implicit solve ------------------------------------------------------------------------------
+ * PAMG_PREC_BLOCK_JACOBI (default): the inverse diagonal 3x3 blocks.  PAMG_PREC_FLOW_GS: one block Gauss-Seidel pass in flow
+ * order (a transport sweep), M = D + L with L = every stored off-diagonal block (e, c) whose column element c has a lower
+ * flow level than e.  Levels come from the upwind graph of the assembled velocity: e depends on its neighbour c across face
+ * f when a Gauss point of f is inflow for e (the assembly's upwind rule) with a non-zero flux; level[e] = the longest upwind
+ * path ending at e.  With pure advection and an acyclic graph M is the operator itself and BiCGStab stops after one
+ * iteration; diffusion blocks to neighbours of the same or a higher level, and the edges that close a cycle of a nodal
+ * field, are lagged (left out of M).  One sweep is one kernel launch whose cost grows with the number of levels.
+ * Needs pamg_set_unstructured first (else PAMG_ERR_STATE); an unknown kind is PAMG_ERR_ARG.  May be called before or after
+ * assembly; the choice survives pamg_set_unstructured.  The levels are built when first needed (the next
+ * pamg_implicit_step, _precond_apply or _flow_levels) and rebuilt after pamg_set_unstructured, pamg_unstr_set_velocity, an
+ * assembly with a different u_x / u_y (uniform velocity) or, with a field, a different use_dir; dt, k and the
+ * stabilisation keep them.  On a multi-GPU handle it acts on part 0 like every unstructured entry. */
+#define PAMG_PREC_BLOCK_JACOBI 0
+#define PAMG_PREC_FLOW_GS 1
+int pamg_implicit_set_precond(pamg_handle* h, int kind);
+/* y = M^-1 x with the selected preconditioner, once (x, y host (3,E)); a timed-out sweep returns PAMG_ERR_CUDA and
+ * pamg_last_error names k_flow_sweep.  Needs an assembled operator (else PAMG_ERR_STATE). */
+int pamg_implicit_precond_apply(pamg_handle* h, const double* x, double* y);
+/* the flow levels of the assembled velocity (built here if stale): level [E] (may be NULL), the number of levels and the
+ * number of lagged upwind edges.  Needs an assembled operator (else PAMG_ERR_STATE). */
+int pamg_implicit_flow_levels(pamg_handle* h, int32_t* level, int32_t* nlevels, int64_t* lagged);
+/* measurement aid: average device time (ms) of `reps` flow sweeps on the work vectors, and the host time (ms) of the last
+ * level build: setup_ms[0] mask kernel + download, [1] pamg_flow_levels, [2] upload (setup_ms may be NULL) */
+int pamg_implicit_flow_time(pamg_handle* h, int reps, float* ms, double* setup_ms);
 
 /* ---- Petrov-Galerkin residual-based stabilisation (transport_tri_unstr.F90:239-267,278; semi_str_implicit.F90:290-318) --
  * diff_coe(gi) and stab(iloc,jloc) of every element from tnew = the field of pamg_unstr_upload and the given told.

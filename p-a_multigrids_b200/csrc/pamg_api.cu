@@ -2261,6 +2261,90 @@ int pamg_implicit_host_syncs(pamg_handle* h, int64_t* n) {
   return PAMG_OK;
 }
 
+// ---- preconditioner of the implicit solve ----------------------------------------------------------------------------
+int pamg_implicit_set_precond(pamg_handle* h, int kind) {
+  ON_PART0(h);
+  if (!h || (kind != PAMG_PREC_BLOCK_JACOBI && kind != PAMG_PREC_FLOW_GS)) return PAMG_ERR_ARG;
+  if (h->un.E < 1) return fail(h, PAMG_ERR_STATE, "pamg_set_unstructured has not been called");
+  h->un.precond = kind;
+  return PAMG_OK;
+}
+
+int pamg_implicit_precond_apply(pamg_handle* h, const double* x, double* y) {
+  ON_PART0(h);
+  if (!h || h->un.E < 1 || !x || !y) return PAMG_ERR_ARG;
+  if (!h->un.assembled) return fail(h, PAMG_ERR_STATE, "pamg_implicit_assemble has not been called");
+  CK(cudaSetDevice(h->device));
+  UnstrDev& u = h->un;
+  const size_t nb = (size_t)u.E * 3 * sizeof(double);
+  double *W = u.work, *Y = u.work + (size_t)u.E * 3;
+  std::string e;
+  CK(cudaMemcpyAsync(W, x, nb, cudaMemcpyHostToDevice, h->stream));
+  if (u.precond == PAMG_PREC_FLOW_GS) {
+    int rc = flow_prepare(u, h->nsm, h->stream, e);
+    if (rc) return fail(h, rc, e);
+    CK(cudaMemsetAsync(u.dots + KS_FLOW_ERR, 0, sizeof(double), h->stream));
+    k_flow_sweep<<<stream_grid(k_flow_sweep, u.occ_flow, u.E, h->nsm), TPB, 0, h->stream>>>(flow_args(u, W, Y, 0));
+  } else {
+    k_block_apply<<<stream_grid(k_block_apply, u.occ_apply, u.E, h->nsm), TPB, 0, h->stream>>>(u.dinv, u.mdt, W, Y, u.E, u.ld, 0);
+  }
+  h->launches++;
+  CK(cudaGetLastError());
+  double ferr = 0.0;
+  CK(cudaMemcpyAsync(y, Y, nb, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(&ferr, u.dots + KS_FLOW_ERR, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  if (u.precond == PAMG_PREC_FLOW_GS && ferr != 0.0)
+    return fail(h, PAMG_ERR_CUDA, "k_flow_sweep: a dependency wait saw no progress for 2 s");
+  return PAMG_OK;
+}
+
+int pamg_implicit_flow_levels(pamg_handle* h, int32_t* level, int32_t* nlevels, int64_t* lagged) {
+  ON_PART0(h);
+  if (!h || h->un.E < 1) return PAMG_ERR_ARG;
+  if (!h->un.assembled) return fail(h, PAMG_ERR_STATE, "pamg_implicit_assemble has not been called");
+  CK(cudaSetDevice(h->device));
+  std::string e;
+  int rc = flow_prepare(h->un, h->nsm, h->stream, e);
+  if (rc) return fail(h, rc, e);
+  if (level) std::memcpy(level, h->un.flow_level_host.data(), (size_t)h->un.E * sizeof(int32_t));
+  if (nlevels) *nlevels = h->un.flow_nlevels;
+  if (lagged) *lagged = h->un.flow_lagged;
+  return PAMG_OK;
+}
+
+int pamg_implicit_flow_time(pamg_handle* h, int reps, float* ms, double* setup_ms) {
+  ON_PART0(h);
+  if (!h || h->un.E < 1 || reps < 1 || !ms) return PAMG_ERR_ARG;
+  if (!h->un.assembled) return fail(h, PAMG_ERR_STATE, "pamg_implicit_assemble has not been called");
+  CK(cudaSetDevice(h->device));
+  UnstrDev& u = h->un;
+  std::string e;
+  int rc = flow_prepare(u, h->nsm, h->stream, e);
+  if (rc) return fail(h, rc, e);
+  const size_t n = (size_t)u.E * 3;
+  double *W = u.work, *Y = u.work + n;
+  const int grid = stream_grid(k_flow_sweep, u.occ_flow, u.E, h->nsm);
+  const FlowArgs fa = flow_args(u, W, Y, 0);
+  CK(cudaMemcpyAsync(W, u.T[u.cur], n * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+  CK(cudaMemsetAsync(u.dots + KS_FLOW_ERR, 0, sizeof(double), h->stream));
+  k_flow_sweep<<<grid, TPB, 0, h->stream>>>(fa);
+  CK(cudaEventRecord(h->ev[14], h->stream));
+  for (int i = 0; i < reps; ++i) k_flow_sweep<<<grid, TPB, 0, h->stream>>>(fa);
+  CK(cudaEventRecord(h->ev[15], h->stream));
+  h->launches += reps + 1;
+  CK(cudaGetLastError());
+  double ferr = 0.0;
+  CK(cudaMemcpyAsync(&ferr, u.dots + KS_FLOW_ERR, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaEventSynchronize(h->ev[15]));
+  CK(cudaStreamSynchronize(h->stream));
+  if (ferr != 0.0) return fail(h, PAMG_ERR_CUDA, "k_flow_sweep: a dependency wait saw no progress for 2 s");
+  CK(cudaEventElapsedTime(ms, h->ev[14], h->ev[15]));
+  *ms /= (float)reps;
+  if (setup_ms) for (int i = 0; i < 3; ++i) setup_ms[i] = u.flow_setup_ms[i];
+  return PAMG_OK;
+}
+
 // ---- trans_rec front-end (transport_rect.F90:7) -------------------------------------------------------------
 int pamg_trans_rec(pamg_handle* h, double CFL, int no_ele_row, int no_ele_col, double x_length, double y_length, double u_x,
                    double u_y, double time, int nits, int njac_its, int direct_solver, int volume_term, double* x_all,

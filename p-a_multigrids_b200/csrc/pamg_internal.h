@@ -40,5 +40,9 @@ struct HaloPlan {
 int build_halo_plan(int U_global, const double* X, const int32_t* neig, const int32_t* fneig, const int32_t* dir,
                     int halo_rule, int nparts, const int32_t* part_first, int my_part, HaloPlan& plan);
 
+// flow levels of the upwind graph (pamg_flow_levels, pamg_plan.cpp)
+int flow_levels(int E, const int32_t* neig, const int32_t* inflow_mask, int32_t* level, int32_t* order, int32_t* nlevels,
+                int64_t* lagged);
+
 }  // namespace pamg
 #endif

@@ -144,3 +144,74 @@ extern "C" int pamg_halo_plan(int U_global, const double* X, const int32_t* neig
   if (counts) { counts[0] = (int32_t)p.peers.size(); counts[1] = p.nstrips; counts[2] = p.nsend; counts[3] = p.U_local; counts[4] = p.first; }
   return PAMG_OK;
 }
+
+// ---- flow levels of the upwind graph (the order of the flow-ordered block Gauss-Seidel preconditioner) -----------------
+// Edge c -> e for every face f of e with bit f of inflow_mask[e] set and a neighbour c = neig[e][f] - 1.  level[e] = the
+// longest upwind path ending at e (Kahn's algorithm, O(E)).  When the queue runs dry before every element has a level, the
+// graph has a cycle: the lowest-index element left gets 1 + the largest level of its already levelled upstream neighbours (0
+// if it has none) and enters the queue.  lagged = the edges whose source level is not below their target's: the sweep
+// treats those blocks as zero.  order = the elements sorted by (level, index).
+int pamg::flow_levels(int E, const int32_t* neig, const int32_t* inflow_mask, int32_t* level, int32_t* order,
+                      int32_t* nlevels, int64_t* lagged) {
+  if (E < 1 || !neig || !inflow_mask || !level || !order) return PAMG_ERR_ARG;
+  std::vector<int32_t> indeg((size_t)E, 0), first((size_t)E + 1, 0), succ;
+  for (int e = 0; e < E; ++e)
+    for (int f = 0; f < 3; ++f) {
+      const int q = neig[(size_t)e * 3 + f];
+      if (q < 0 || q > E) return PAMG_ERR_ARG;
+      if (q != 0 && ((inflow_mask[e] >> f) & 1)) { ++indeg[e]; ++first[q]; }
+    }
+  for (int e = 0; e < E; ++e) first[e + 1] += first[e];
+  succ.resize((size_t)first[E]);
+  {
+    std::vector<int32_t> fill(first.begin(), first.end() - 1);
+    for (int e = 0; e < E; ++e)
+      for (int f = 0; f < 3; ++f) {
+        const int q = neig[(size_t)e * 3 + f];
+        if (q != 0 && ((inflow_mask[e] >> f) & 1)) succ[(size_t)fill[q - 1]++] = e;
+      }
+  }
+  std::vector<int32_t> queue;
+  queue.reserve((size_t)E);
+  std::vector<char> placed((size_t)E, 0);
+  for (int e = 0; e < E; ++e) {
+    level[e] = 0;
+    if (indeg[e] == 0) { queue.push_back(e); placed[e] = 1; }
+  }
+  size_t head = 0;
+  int next_free = 0;                       // every element below it is placed
+  while (queue.size() < (size_t)E || head < queue.size()) {
+    if (head == queue.size()) {            // cycle: the lowest-index element left; level[] already holds 1 + max upstream
+      while (placed[next_free]) ++next_free;
+      queue.push_back(next_free); placed[next_free] = 1;
+    }
+    const int c = queue[head++];
+    for (int32_t i = first[c]; i < first[c + 1]; ++i) {
+      const int e = succ[(size_t)i];
+      if (placed[e]) continue;             // an edge into an element placed earlier by the cycle rule
+      level[e] = std::max(level[e], level[c] + 1);
+      if (--indeg[e] == 0) { queue.push_back(e); placed[e] = 1; }
+    }
+  }
+  int32_t nl = 0;
+  int64_t lag = 0;
+  for (int e = 0; e < E; ++e) {
+    nl = std::max(nl, level[e] + 1);
+    for (int f = 0; f < 3; ++f) {
+      const int q = neig[(size_t)e * 3 + f];
+      if (q != 0 && ((inflow_mask[e] >> f) & 1) && level[q - 1] >= level[e]) ++lag;
+    }
+  }
+  std::vector<int32_t> start((size_t)nl + 1, 0);
+  for (int e = 0; e < E; ++e) ++start[(size_t)level[e] + 1];
+  for (int l = 0; l < nl; ++l) start[(size_t)l + 1] += start[(size_t)l];
+  for (int e = 0; e < E; ++e) order[start[(size_t)level[e]]++] = e;
+  if (nlevels) *nlevels = nl;
+  if (lagged) *lagged = lag;
+  return PAMG_OK;
+}
+
+extern "C" int pamg_flow_levels(int E, const int32_t* neig, const int32_t* inflow_mask, int32_t* level, int32_t* order,
+                                int32_t* nlevels, int64_t* lagged) {
+  return pamg::flow_levels(E, neig, inflow_mask, level, order, nlevels, lagged);
+}

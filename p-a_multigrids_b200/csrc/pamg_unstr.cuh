@@ -14,12 +14,15 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <string>
 #include <vector>
 
 #include "pamg.h"
+#include "pamg_internal.h"
 #include "pamg_kernels.cuh"
 
 namespace pamg {
@@ -59,6 +62,23 @@ struct UnstrDev {
   int occ_explicit = 0, occ_assemble = 0, occ_spmv = 0, occ_apply = 0, occ_stab = 0, occ_kry[6] = {0, 0, 0, 0, 0, 0};   // resident CTAs
                               // per SM of the streaming kernels (this device)
   int occ_explicit_f = 0, occ_assemble_f = 0, occ_stab_f = 0;   // the same for the velocity-field instantiations
+  int use_dir = 0;             // pairing rule of the last assembly
+  // flow-ordered block Gauss-Seidel preconditioner (pamg_implicit_set_precond): the levels of the upwind graph of the
+  // assembled velocity, built when first needed and kept until the mesh, the field, the uniform velocity or (with a field)
+  // the pairing rule changes
+  int precond = PAMG_PREC_BLOCK_JACOBI;
+  bool flow_valid = false;
+  double flow_ux = 0.0, flow_uy = 0.0; int flow_use_dir = 0;
+  int32_t* flow_order = nullptr;     // [E] elements sorted by (level, index)
+  int32_t* flow_level = nullptr;     // [E]
+  unsigned* flow_done = nullptr;     // [E] number of the sweep application that last published the element (never cleared)
+  unsigned* flow_ctl = nullptr;      // [3] ticket counter, CTAs finished, applications so far
+  uint8_t* flow_mask = nullptr;      // [E] inflow faces of every element (k_flow_mask)
+  int flow_nlevels = 0; long long flow_lagged = 0;
+  double flow_setup_ms[3] = {0.0, 0.0, 0.0};   // host time of the last build: mask (kernel + download), levels, upload
+  int occ_flow = 0, occ_flow_vec = 0;
+  std::vector<int32_t> neig_host;    // [E][3] as given to pamg_set_unstructured (the level computation runs on the host)
+  std::vector<int32_t> flow_level_host;
 };
 
 inline size_t plane_stride(int E) {
@@ -139,6 +159,8 @@ __device__ __forceinline__ FaceVel2 neighbour_vel(const double* __restrict__ U, 
   }
   return v;
 }
+// income = 1/2 + 1/2 sign(1, -c) == 1 for c = sdetwei n.u (sign(1, -0) = 1: a face with c = -0 is inflow)
+__device__ __forceinline__ bool upwind_in(double c) { return signbit(-c) == 0; }
 // sdetwei n.u of both traces at Gauss point s and the upwind choice income(s) = 1/2 + 1/2 sign(1, -n.(us + us2)/2), the
 // sign taken from the element's own trace alone where sn2 = 0
 struct GaussFlux { double c, c2; bool in; };
@@ -147,7 +169,7 @@ __device__ __forceinline__ GaussFlux gauss_flux(const TriEdges& g, int l1, int l
   GaussFlux r;
   r.c = face_flux(g, l1, l2, l3, a1 * ux[l1] + a2 * ux[l2], a1 * uy[l1] + a2 * uy[l2]);
   r.c2 = v.own ? r.c : face_flux(g, l1, l2, l3, a1 * v.ax + a2 * v.bx, a1 * v.ay + a2 * v.by);
-  r.in = signbit(-(ns >= 1 ? r.c + r.c2 : r.c)) == 0;
+  r.in = upwind_in(ns >= 1 ? r.c + r.c2 : r.c);
   return r;
 }
 
@@ -272,7 +294,7 @@ __global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OC
       const double c = face_flux(g, l1, l2, L3[f], a.ux, a.uy);   // sdetwei * n . u
       const bool has2 = (enc[f] & 3) >= 1;
       // income = 0.5 + 0.5 sign(1, -n.(u + u2)/2) (:731); u2 = 0 when sn2 = 0 (Nside = 0) does not change the sign
-      const bool in = signbit(-c) == 0;
+      const bool in = upwind_in(c);
       double ca, cb;
       if (in) { const double f2 = has2 ? c : 0.0; ca = f2 * (w2 * T2a[f] + w1 * T2b[f]); cb = f2 * (w1 * T2a[f] + w2 * T2b[f]); }
       else { ca = c * (w2 * T[l1] + w1 * T[l2]); cb = c * (w1 * T[l1] + w2 * T[l2]); }
@@ -331,6 +353,7 @@ inline void unstr_free(UnstrDev& u) {
   cudaFree(u.X); cudaFree(u.U); cudaFree(u.neig); cudaFree(u.nside); cudaFree(u.pen); cudaFree(u.T[0]); cudaFree(u.T[1]); cudaFree(u.told);
   cudaFree(u.bsr_val); cudaFree(u.bsr_col); cudaFree(u.dinv); cudaFree(u.mdt); cudaFree(u.work); cudaFree(u.dots); cudaFree(u.diag0); cudaFree(u.stab);
   cudaFree(u.xfer);
+  cudaFree(u.flow_order); cudaFree(u.flow_level); cudaFree(u.flow_done); cudaFree(u.flow_ctl); cudaFree(u.flow_mask);
   if (u.dots_host) cudaFreeHost(u.dots_host);
   u = UnstrDev();
 }
@@ -359,7 +382,9 @@ inline int stream_grid(K kernel, int& occ_cache, int E, int nsm) {
 
 inline int unstr_setup(UnstrDev& u, int E, const double* X, const int32_t* neig, const int32_t* fneig,
                        cudaStream_t st, std::string& err) {
+  const int precond = u.precond;   // a solver choice, kept across meshes
   unstr_free(u);
+  u.precond = precond;
   // geometric pairing flag per face: does the neighbour node that get_unstr_sn2 pairs with my first face
   // node actually coincide with it?  (SURVEY B-9: the reference ignores Dir here)
   // penalty length of the diffusion face term (get_d_center Msh2Tri.F90:349-385, add_diffusion_surf matrices.F90:84-110)
@@ -395,6 +420,7 @@ inline int unstr_setup(UnstrDev& u, int E, const double* X, const int32_t* neig,
     }
   }
   u.E = E; u.ld = ld;
+  u.neig_host.assign(neig, neig + (size_t)E * 3);
   UCK(cudaMalloc(&u.X, ld * 6 * sizeof(double)));
   UCK(cudaMalloc(&u.neig, ld * 3 * sizeof(int32_t)));
   UCK(cudaMalloc(&u.nside, ld * 3 * sizeof(int32_t)));
@@ -417,6 +443,7 @@ inline int unstr_setup(UnstrDev& u, int E, const double* X, const int32_t* neig,
 inline int unstr_set_velocity(UnstrDev& u, const double* u_ele, int nsm, cudaStream_t st, std::string& err) {
   u.assembled = false;
   u.with_stab = false;
+  u.flow_valid = false;
   if (!u_ele) { cudaFree(u.U); u.U = nullptr; return PAMG_OK; }
   const size_t E = (size_t)u.E;
   if (!u.U) UCK(cudaMalloc(&u.U, u.ld * 6 * sizeof(double)));
@@ -555,7 +582,7 @@ __global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_ASSEMBLE_FIELD : PAMG_OC
       const int l1 = L1[f], l2 = L2[f];
       const double c = face_flux(g, l1, l2, L3[f], a.ux, a.uy);   // sdetwei * n . u
       const int ns = enc[f] & 3;
-      const bool in = signbit(-c) == 0;
+      const bool in = upwind_in(c);
       // neighbour nodes coincident with (l1, l2): as in get_unstr_sn2, or the geometric pairing with use_dir
       int m1 = (ns == 1) ? 2 : (ns == 2 ? 0 : 1), m2 = (ns == 1) ? 0 : (ns == 2 ? 1 : 2);
       if (a.use_dir && (enc[f] >> 2)) { const int t = m1; m1 = m2; m2 = t; }
@@ -918,6 +945,254 @@ __global__ void __launch_bounds__(TPB, 6) k_kry_x(KryArgs a) {   // (unbounded t
   }
 }
 
+// ---- flow-ordered block Gauss-Seidel preconditioner (a "transport sweep") --------------------------------------------
+// With pure advection and upwind fluxes element e is coupled only to its inflow neighbours, so in flow order the operator is
+// block lower-triangular and one block Gauss-Seidel pass in that order solves it exactly.  M = D + L, L = every stored
+// off-diagonal block (e, c) with level[c] < level[e]; blocks to the same or a higher level (diffusion: downstream and
+// crosswind neighbours; a cycle of a nodal field) are lagged, i.e. treated as zero.
+constexpr int KS_FLOW_ERR = 10;   // Krylov scalar slot: != 0 after a dependency wait of k_flow_sweep timed out
+
+// inflow faces of every element: bit f when a Gauss point of face f is inflow (the assembly's upwind rule) with a non-zero
+// flux and the face has a neighbour, i.e. exactly where k_assemble_bsr puts a non-zero advective block into the neighbour's
+// columns.  A tangential face (c = -0, n.u = 0) couples nothing and orders nothing: counting it would make a 2-cycle.
+struct MaskArgs {
+  const double* X; const int32_t* neig; const int32_t* nside; const double* U; uint8_t* mask;
+  double ux, uy;
+  size_t ld;
+  int E, use_dir;
+};
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB) k_flow_mask(MaskArgs a) {
+  const double al = 0.78867513459481288, be = 0.21132486540518712;
+  const size_t ld = a.ld;
+  const int L1[3] = {0, 1, 2}, L2[3] = {2, 0, 1}, L3[3] = {1, 2, 0};
+  for (int e = blockIdx.x * TPB + threadIdx.x; e < a.E; e += gridDim.x * TPB) {
+    TriEdges g;
+    tri_edges(a.X, ld, (size_t)e, g);
+    double ux[3], uy[3];
+    if constexpr (FIELD) load_vel(a.U, ld, (size_t)e, ux, uy);
+    unsigned m = 0;
+#pragma unroll
+    for (int f = 0; f < 3; ++f) {
+      const int q = __ldg(a.neig + (size_t)f * ld + e), enc = __ldg(a.nside + (size_t)f * ld + e);
+      const int ns = enc & 3;
+      if (ns < 1 || q == 0) continue;
+      const int l1 = L1[f], l2 = L2[f];
+      if constexpr (FIELD) {
+        int m1 = (ns == 1) ? 2 : (ns == 2 ? 0 : 1), m2 = (ns == 1) ? 0 : (ns == 2 ? 1 : 2);
+        if (a.use_dir && (enc >> 2)) { const int t = m1; m1 = m2; m2 = t; }
+        const FaceVel2 v2 = neighbour_vel(a.U, ld, q, ns, m1, m2);
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const GaussFlux r = gauss_flux(g, l1, l2, L3[f], s == 0 ? al : be, s == 0 ? be : al, ux, uy, v2, ns);
+          if (r.in && r.c2 != 0.0) m |= 1u << f;
+        }
+      } else {
+        const double c = face_flux(g, l1, l2, L3[f], a.ux, a.uy);
+        if (upwind_in(c) && c != 0.0) m |= 1u << f;
+      }
+    }
+    a.mask[e] = (uint8_t)m;
+  }
+}
+
+__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
+  unsigned v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void st_release(unsigned* p, unsigned v) {
+  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long global_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+
+struct FlowArgs {
+  const double* val; const int32_t* col; const double* dinv; const int32_t* level; const int32_t* order;
+  const double* x; double* y;
+  unsigned* done; unsigned* ctl; double* ks;
+  size_t ld;
+  int E, krylov;   // krylov: a step of the solve (nothing to do once the solve has stopped)
+};
+enum { FLOW_TICKET = 0, FLOW_EXITED, FLOW_APPS };
+constexpr unsigned long long FLOW_WAIT_NS = 2000000000ull;   // a warp that sees no progress for 2 s gives up
+
+// y = M^-1 x, y_e = dinv_e (x_e - sum_{level[c] < level[e]} B_ec y_c), in one launch without grid synchronisation.  Warps take
+// chunks of 32 consecutive entries of `order` from a ticket counter, so chunks are handed out in flow order; an element waits
+// for the done flags of the (at most 3) neighbours it uses.  Deadlock-free: the warp holding the smallest unfinished ticket
+// waits only for finished elements.  A chunk may straddle a level boundary, so a lane never spins on its own: every lane
+// whose dependencies are published computes and publishes, and the warp repeats until all its lanes are done.  Each element
+// sums its neighbour terms in face order once all have arrived: two applications are bit-identical.  Flags carry the
+// application number (device memory), so they are never cleared; the last CTA to leave resets the ticket counter and
+// advances the number, with no host round trip.  The elements of a chunk are not contiguous, so records are gathered per
+// lane instead of through warp_load3 / warp_store3; the matrix stays in its planes.  A wait that sees no progress for
+// FLOW_WAIT_NS sets KS_FLOW_ERR (and stops the solve) instead of hanging the device.
+__global__ void __launch_bounds__(TPB) k_flow_sweep(FlowArgs a) {
+  __shared__ unsigned s_app;
+  if (threadIdx.x == 0) s_app = *(volatile unsigned*)(a.ctl + FLOW_APPS) + 1u;
+  __syncthreads();
+  const unsigned app = s_app;
+  const int lane = threadIdx.x & 31;
+  const size_t ld = a.ld;
+  const int nchunks = (a.E + 31) >> 5;
+  volatile double* err = a.ks + KS_FLOW_ERR;
+  bool run = !(a.krylov && a.ks[KS_DONE] != 0.0);
+  while (run) {
+    int t = 0;
+    if (lane == 0) t = (*err != 0.0) ? nchunks : (int)atomicAdd(a.ctl + FLOW_TICKET, 1u);
+    t = __shfl_sync(0xffffffffu, t, 0);
+    if (t >= nchunks) break;
+    const int pos = t * 32 + lane;
+    const bool valid = pos < a.E;
+    const int e = valid ? __ldg(a.order + pos) : 0;
+    double x0 = 0.0, x1 = 0.0, x2 = 0.0, d[9], B[3][9], yc[3][3];
+    int c[3];
+    unsigned wait = 0;
+    if (valid) {
+      const int lev = __ldg(a.level + e);
+#pragma unroll
+      for (int f = 0; f < 3; ++f) {
+        c[f] = __ldg(a.col + (size_t)(1 + f) * ld + e);
+        if (c[f] >= 0 && __ldg(a.level + c[f]) < lev) wait |= 1u << f;
+      }
+      x0 = __ldg(a.x + (size_t)e * 3); x1 = __ldg(a.x + (size_t)e * 3 + 1); x2 = __ldg(a.x + (size_t)e * 3 + 2);
+#pragma unroll
+      for (int k = 0; k < 9; ++k) d[k] = __ldg(a.dinv + (size_t)k * ld + e);
+#pragma unroll
+      for (int f = 0; f < 3; ++f)
+#pragma unroll
+        for (int k = 0; k < 9; ++k) B[f][k] = ((wait >> f) & 1) ? __ldg(a.val + (size_t)((1 + f) * 9 + k) * ld + e) : 0.0;
+    }
+    const unsigned use = wait;
+    bool pending = valid;
+    unsigned long long t_last = lane == 0 ? global_ns() : 0ull;
+    unsigned idle = 0;
+    bool failed = false;
+    while (__any_sync(0xffffffffu, pending)) {
+      bool moved = false;
+      if (pending) {
+#pragma unroll
+        for (int f = 0; f < 3; ++f)
+          if (((wait >> f) & 1) && ld_acquire(a.done + c[f]) == app) {
+            const double* yp = a.y + (size_t)c[f] * 3;
+            yc[f][0] = __ldcg(yp); yc[f][1] = __ldcg(yp + 1); yc[f][2] = __ldcg(yp + 2);
+            wait &= ~(1u << f); moved = true;
+          }
+        if (wait == 0) {
+          double r0 = x0, r1 = x1, r2 = x2;
+#pragma unroll
+          for (int f = 0; f < 3; ++f)
+            if ((use >> f) & 1) {
+              r0 -= B[f][0] * yc[f][0] + B[f][1] * yc[f][1] + B[f][2] * yc[f][2];
+              r1 -= B[f][3] * yc[f][0] + B[f][4] * yc[f][1] + B[f][5] * yc[f][2];
+              r2 -= B[f][6] * yc[f][0] + B[f][7] * yc[f][1] + B[f][8] * yc[f][2];
+            }
+          double* yp = a.y + (size_t)e * 3;
+          __stcg(yp, d[0] * r0 + d[1] * r1 + d[2] * r2);
+          __stcg(yp + 1, d[3] * r0 + d[4] * r1 + d[5] * r2);
+          __stcg(yp + 2, d[6] * r0 + d[7] * r1 + d[8] * r2);
+          st_release(a.done + e, app);
+          pending = false; moved = true;
+        }
+      }
+      if (__any_sync(0xffffffffu, moved)) { idle = 0; if (lane == 0) t_last = global_ns(); continue; }
+      __nanosleep(32);
+      if ((++idle & 1023) == 0) {
+        int give_up = 0;
+        if (lane == 0) {
+          give_up = *err != 0.0;
+          if (!give_up && global_ns() - t_last > FLOW_WAIT_NS) {
+            *err = 1.0;
+            if (a.krylov) a.ks[KS_DONE] = 3.0;
+            give_up = 1;
+          }
+        }
+        if (__shfl_sync(0xffffffffu, give_up, 0)) { failed = true; break; }
+      }
+    }
+    if (failed) break;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0 && atomicAdd(a.ctl + FLOW_EXITED, 1u) == gridDim.x - 1) {
+    a.ctl[FLOW_TICKET] = 0u; a.ctl[FLOW_EXITED] = 0u; a.ctl[FLOW_APPS] = app;
+  }
+}
+
+// the vector updates of k_kry_p / k_kry_s without their block-Jacobi products: with the flow preconditioner y = M^-1 p and
+// z = M^-1 s come from k_flow_sweep.  p = r + beta (p - omega v) ; s = r - alpha v
+template <int WHICH>
+__global__ void __launch_bounds__(TPB) k_kry_vec(KryArgs a) {
+  if (a.ks[KS_DONE] != 0.0) return;
+  const long long n = 3LL * a.E;
+  if (WHICH == 0) {
+    const double rho_new = a.ks[KS_RHONEW], rho = a.ks[KS_RHO], alpha = a.ks[KS_ALPHA], omega = a.ks[KS_OMEGA];
+    const double beta = (rho_new / rho) * (alpha / omega);
+    for (long long i = (long long)blockIdx.x * TPB + threadIdx.x; i < n; i += (long long)gridDim.x * TPB)
+      a.p[i] = a.r[i] + beta * a.p[i] + (-beta * omega) * a.v[i];
+  } else {
+    const double alpha = a.ks[KS_ALPHA];
+    for (long long i = (long long)blockIdx.x * TPB + threadIdx.x; i < n; i += (long long)gridDim.x * TPB)
+      a.s[i] = a.r[i] - alpha * a.v[i];
+  }
+}
+
+inline FlowArgs flow_args(const UnstrDev& u, const double* x, double* y, int krylov) {
+  FlowArgs f;
+  f.val = u.bsr_val; f.col = u.bsr_col; f.dinv = u.dinv; f.level = u.flow_level; f.order = u.flow_order;
+  f.x = x; f.y = y; f.done = u.flow_done; f.ctl = u.flow_ctl; f.ks = u.dots; f.ld = u.ld; f.E = u.E; f.krylov = krylov;
+  return f;
+}
+
+// levels of the upwind graph of the assembled velocity: k_flow_mask, one byte per element down, pamg::flow_levels on the host,
+// order and level up.  Kept while the velocity is the same (pamg_unstr_set_velocity clears them; dt, k and the stabilisation
+// do not change the graph).
+inline int flow_prepare(UnstrDev& u, int nsm, cudaStream_t st, std::string& err) {
+  if (u.flow_valid && (u.U ? u.flow_use_dir == u.use_dir : (u.flow_ux == u.ux && u.flow_uy == u.uy))) return PAMG_OK;
+  const size_t E = (size_t)u.E;
+  if (!u.flow_order) {
+    UCK(cudaMalloc(&u.flow_order, E * sizeof(int32_t)));
+    UCK(cudaMalloc(&u.flow_level, E * sizeof(int32_t)));
+    UCK(cudaMalloc(&u.flow_done, E * sizeof(unsigned)));
+    UCK(cudaMalloc(&u.flow_ctl, 4 * sizeof(unsigned)));
+    UCK(cudaMalloc(&u.flow_mask, E));
+    UCK(cudaMemsetAsync(u.flow_done, 0, E * sizeof(unsigned), st));
+    UCK(cudaMemsetAsync(u.flow_ctl, 0, 4 * sizeof(unsigned), st));
+  }
+  using clk = std::chrono::steady_clock;
+  const auto t0 = clk::now();
+  MaskArgs m;
+  m.X = u.X; m.neig = u.neig; m.nside = u.nside; m.U = u.U; m.mask = u.flow_mask; m.ux = u.ux; m.uy = u.uy; m.ld = u.ld;
+  m.E = u.E; m.use_dir = u.use_dir;
+  const int grid = std::max(1, std::min((u.E + TPB - 1) / TPB, nsm * 8));
+  if (u.U) k_flow_mask<true><<<grid, TPB, 0, st>>>(m);
+  else k_flow_mask<false><<<grid, TPB, 0, st>>>(m);
+  UCK(cudaGetLastError());
+  std::vector<uint8_t> m8(E);
+  UCK(cudaMemcpyAsync(m8.data(), u.flow_mask, E, cudaMemcpyDeviceToHost, st));
+  UCK(cudaStreamSynchronize(st));
+  const auto t1 = clk::now();
+  std::vector<int32_t> mask(m8.begin(), m8.end()), order(E);
+  u.flow_level_host.resize(E);
+  int32_t nl = 0;
+  int64_t lag = 0;
+  const int rc = flow_levels(u.E, u.neig_host.data(), mask.data(), u.flow_level_host.data(), order.data(), &nl, &lag);
+  if (rc != PAMG_OK) { err = "pamg::flow_levels failed"; return rc; }
+  const auto t2 = clk::now();
+  UCK(cudaMemcpyAsync(u.flow_order, order.data(), E * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  UCK(cudaMemcpyAsync(u.flow_level, u.flow_level_host.data(), E * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  UCK(cudaStreamSynchronize(st));
+  const auto t3 = clk::now();
+  u.flow_setup_ms[0] = std::chrono::duration<double, std::milli>(t1 - t0).count();
+  u.flow_setup_ms[1] = std::chrono::duration<double, std::milli>(t2 - t1).count();
+  u.flow_setup_ms[2] = std::chrono::duration<double, std::milli>(t3 - t2).count();
+  u.flow_nlevels = nl; u.flow_lagged = lag;
+  u.flow_valid = true; u.flow_ux = u.ux; u.flow_uy = u.uy; u.flow_use_dir = u.use_dir;
+  return PAMG_OK;
+}
+
 // Petrov-Galerkin residual-based stabilisation (transport_tri_unstr.F90:239-267,278): one thread per element.
 // For P1 the gradient of T and inv_jac are constant over the element; rgi differs per Gauss point through T(gi).
 // mode 0: write diff_coe (3 per element) and stab (9 per element), both in ABI order [E][..].
@@ -1023,7 +1298,7 @@ inline int implicit_assemble(UnstrDev& u, double dt, double ux, double uy, doubl
   else k_assemble_bsr<false><<<stream_grid(k_assemble_bsr<false>, u.occ_assemble, u.E, nsm), TPB, 0, st>>>(a);
   nlaunch++;
   UCK(cudaGetLastError());
-  u.assembled = true; u.dt = dt; u.ux = ux; u.uy = uy; u.kdiff = kdiff;
+  u.assembled = true; u.dt = dt; u.ux = ux; u.uy = uy; u.kdiff = kdiff; u.use_dir = use_dir;
   return PAMG_OK;
 }
 
@@ -1045,6 +1320,18 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
   a.val = u.bsr_val; a.col = u.bsr_col; a.dinv = u.dinv; a.ks = u.dots; a.E = E; a.ld = u.ld;
   a.b = W; a.r = W + n; a.rh = W + 2 * n; a.p = W + 3 * n; a.v = W + 4 * n; a.s = W + 5 * n; a.t = W + 6 * n; a.y = W + 7 * n;
   a.z = W + 8 * n;
+  // flow preconditioner: y = M^-1 p and z = M^-1 s by k_flow_sweep between the vector updates and the products
+  const bool flow = u.precond == PAMG_PREC_FLOW_GS;
+  int g_vec = 0, g_flow = 0;
+  FlowArgs fp{}, fs{};
+  if (flow) {
+    const int rc = flow_prepare(u, nsm, st, err);
+    if (rc != PAMG_OK) return rc;
+    g_vec = stream_grid(k_kry_vec<0>, u.occ_flow_vec, E, nsm);
+    g_flow = stream_grid(k_flow_sweep, u.occ_flow, E, nsm);
+    fp = flow_args(u, a.p, a.y, 1); fs = flow_args(u, a.s, a.z, 1);
+    UCK(cudaMemsetAsync(u.dots + KS_FLOW_ERR, 0, sizeof(double), st));
+  }
   int total = 0;
   double worst = 0.0;
   const double maxit = (double)max_iters;
@@ -1069,7 +1356,17 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
       UCK(cudaMemcpyAsync(u.dots + KS_MAXIT, &maxit, sizeof(double), cudaMemcpyHostToDevice, st));
       k_kry_init<<<g_init, TPB, 0, st>>>(a, tol); nlaunch++;
       for (;;) {
-        for (int j = 0; j < KRY_BATCH; ++j) {
+        for (int j = 0; j < KRY_BATCH && flow; ++j) {
+          k_kry_vec<0><<<g_vec, TPB, 0, st>>>(a);
+          k_flow_sweep<<<g_flow, TPB, 0, st>>>(fp);
+          k_kry_spmv<0><<<g_v, TPB, 0, st>>>(a);
+          k_kry_vec<1><<<g_vec, TPB, 0, st>>>(a);
+          k_flow_sweep<<<g_flow, TPB, 0, st>>>(fs);
+          k_kry_spmv<1><<<g_t, TPB, 0, st>>>(a);
+          k_kry_x<<<g_x, TPB, 0, st>>>(a);
+          nlaunch += 7;
+        }
+        for (int j = 0; j < KRY_BATCH && !flow; ++j) {
           k_kry_p<<<g_p, TPB, 0, st>>>(a);
           k_kry_spmv<0><<<g_v, TPB, 0, st>>>(a);
           k_kry_s<<<g_s, TPB, 0, st>>>(a);
@@ -1083,6 +1380,10 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
         if (u.dots_host[KS_DONE] != 0.0) break;
       }
       UCK(cudaGetLastError());
+      if (flow && u.dots_host[KS_FLOW_ERR] != 0.0) {
+        err = "k_flow_sweep: a dependency wait saw no progress for 2 s; the solve was stopped";
+        return PAMG_ERR_CUDA;
+      }
       total += (int)u.dots_host[KS_ITER];
       const double bb = u.dots_host[KS_BB], rr = u.dots_host[KS_RR];
       const double rel = bb > 0.0 ? sqrt(rr / bb) : 0.0;

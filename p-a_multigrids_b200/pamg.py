@@ -17,6 +17,8 @@ LIB_PATH = os.environ.get("PAMG_LIB") or os.path.join(_HERE, "lib", "libpamg_cud
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_IO, ERR_SINGULAR, ERR_UNSUPPORTED = 0, -1, -2, -3, -4, -5, -6
 TNEW, TOLD, RHS, RES, TNONLIN = 0, 1, 2, 3, 5
 JACOBI, RICHARDSON, GAUSS_SEIDEL = 1, 2, 3
+PREC_BLOCK_JACOBI, PREC_FLOW_GS = 0, 1
+PRECONDITIONERS = {"block_jacobi": PREC_BLOCK_JACOBI, "flow_gs": PREC_FLOW_GS}
 
 _f64 = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
 _i32 = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
@@ -117,6 +119,11 @@ def lib():
         "pamg_implicit_step": (ci, [vp, ci, ci, cd, ci, pint, pdbl]),
         "pamg_unstr_stab": (ci, [vp, _f64, cd, cd, cd, vp, vp]),
         "pamg_implicit_set_stab": (ci, [vp, ci]),
+        "pamg_implicit_set_precond": (ci, [vp, ci]),
+        "pamg_implicit_precond_apply": (ci, [vp, _f64, _f64]),
+        "pamg_implicit_flow_levels": (ci, [vp, vp, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
+        "pamg_implicit_flow_time": (ci, [vp, ci, C.POINTER(C.c_float), vp]),
+        "pamg_flow_levels": (ci, [ci, _i32, _i32, _i32, _i32, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
         "pamg_trans_rec": (ci, [vp, cd, ci, ci, cd, cd, cd, cd, cd, ci, ci, ci, ci, vp, vp, pint]),
         "pamg_apply_local_minv": (ci, [vp, ci, ci, _f64, vp, vp, vp, vp]),
         "pamg_output_fields": (ci, [vp, vp, vp, vp]),
@@ -270,6 +277,22 @@ def parent_table(params, mesh, parent, s, theta_weight=None, with_mass=True, bc_
     if rc != OK:
         raise PamgError(rc, "pamg_parent_table")
     return out
+
+
+def flow_levels(neig, inflow_mask):
+    """Host-only: flow levels of the upwind graph given by (E,3) 1-based neighbours and per-element inflow-face bits
+    (pamg_flow_levels).  Returns (level [E], order [E], nlevels, lagged)."""
+    neig = np.ascontiguousarray(neig, np.int32)
+    mask = np.ascontiguousarray(inflow_mask, np.int32).reshape(-1)
+    E = mask.shape[0]
+    if neig.shape != (E, 3):
+        raise ValueError(f"neig must have shape (E, 3) = ({E}, 3), got {neig.shape}")
+    level = np.zeros(E, np.int32); order = np.zeros(E, np.int32)
+    nl = C.c_int32(0); lag = C.c_int64(0)
+    rc = lib().pamg_flow_levels(E, neig, mask, level, order, C.byref(nl), C.byref(lag))
+    if rc != OK:
+        raise PamgError(rc, "pamg_flow_levels")
+    return level, order, nl.value, lag.value
 
 
 # ------------------------------------------------------------------------------ solver handle
@@ -533,9 +556,37 @@ class SemiImplicitIterative:
         self._ck(self.L.pamg_unstr_stab(self.h, o, dt, u_x, u_y, _ptr(dc), _ptr(st)))
         return dc, st
 
-    def unstr_implicit(self, tnew, dt, u_x, u_y, ntime=2, nits=1, use_dir=False, tol=1e-13, max_iters=500, with_stab=False):
-        """Time loop of unstr_implicit; returns (tnew, Krylov iterations in total, worst relative residual)."""
+    def implicit_set_precond(self, kind):
+        """Preconditioner of the implicit solve: "block_jacobi" (default) or "flow_gs", one block Gauss-Seidel pass in
+        flow order (pamg_implicit_set_precond)."""
+        if kind not in PRECONDITIONERS:
+            raise ValueError(f"unknown preconditioner {kind!r}: one of {sorted(PRECONDITIONERS)}")
+        self._ck(self.L.pamg_implicit_set_precond(self.h, PRECONDITIONERS[kind]))
+
+    def implicit_precond_apply(self, x):
+        """y = M^-1 x with the selected preconditioner, once; x is (E, 3)."""
+        x = np.ascontiguousarray(x, np.float64); y = np.empty_like(x)
+        self._ck(self.L.pamg_implicit_precond_apply(self.h, x, y))
+        return y
+
+    def implicit_flow_levels(self):
+        """(level [E], nlevels, lagged) of the upwind graph of the assembled velocity."""
+        level = np.zeros(self._E, np.int32); nl = C.c_int32(0); lag = C.c_int64(0)
+        self._ck(self.L.pamg_implicit_flow_levels(self.h, _ptr(level), C.byref(nl), C.byref(lag)))
+        return level, nl.value, lag.value
+
+    def implicit_flow_time(self, reps=5):
+        """(ms per flow sweep, host ms of the last level build: [mask, levels, upload])."""
+        ms = C.c_float(); setup = np.zeros(3)
+        self._ck(self.L.pamg_implicit_flow_time(self.h, reps, C.byref(ms), _ptr(setup)))
+        return ms.value, setup
+
+    def unstr_implicit(self, tnew, dt, u_x, u_y, ntime=2, nits=1, use_dir=False, tol=1e-13, max_iters=500, with_stab=False,
+                       precond="block_jacobi"):
+        """Time loop of unstr_implicit; returns (tnew, Krylov iterations in total, worst relative residual).  precond:
+        "block_jacobi" or "flow_gs" (implicit_set_precond)."""
         t = np.ascontiguousarray(tnew, np.float64)
+        self.implicit_set_precond(precond)
         self.implicit_assemble(dt, u_x, u_y, use_dir)
         if with_stab:
             self._ck(self.L.pamg_implicit_set_stab(self.h, 1))

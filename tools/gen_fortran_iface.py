@@ -17,7 +17,7 @@ OUT = os.path.join(ROOT, "p-a_multigrids_b200", "host", "pamg_iface.F90")
 
 # pointer arguments that are ONE value written by the library (everything else with a '*' is an array)
 SCALAR_OUT = {"n", "U", "ndof", "l2", "linf", "conv", "cycles", "relres", "npeers", "peer_part", "nfaces", "iters_total",
-              "ntime", "ms", "total_ms", "launches"}
+              "ntime", "ms", "total_ms", "launches", "nlevels", "lagged"}
 # array arguments the header documents as optional (NULL allowed): passed as type(c_ptr) so that c_null_ptr can be given
 NULLABLE = {"part_first", "region", "devices", "bc_value", "val", "col", "diff_coe", "stab", "x_all", "analytical", "error",
             "Minv", "status", "rhs", "x", "hist", "strip_of", "dst_strip", "rev", "hmap", "peers", "counts", "X_out", "bc_kind",
@@ -33,7 +33,8 @@ NULLABLE_IN = {"pamg_mesh_get": {"X", "neig", "fneig", "dir", "region"},
                "pamg_vcycle_solve": {"cycles", "hist"}, "pamg_residual": {"l2", "linf"},
                "pamg_timestep_host": {"cycles", "relres"}, "pamg_implicit_step": {"iters_total", "relres"},
                "pamg_halo_peer_info": {"peer_part", "nfaces"}, "pamg_parent_table": {"bc_kind"},
-               "pamg_unstr_set_velocity": {"u_ele"}}
+               "pamg_unstr_set_velocity": {"u_ele"}, "pamg_implicit_flow_levels": {"level"},
+               "pamg_implicit_flow_time": {"setup_ms"}}
 
 FTYPE = {"int": "integer(c_int)", "int32_t": "integer(c_int32_t)", "int64_t": "integer(c_int64_t)", "double": "real(c_double)",
          "float": "real(c_float)"}
