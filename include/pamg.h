@@ -218,6 +218,25 @@ int pamg_unstr_download(pamg_handle* h, double* tnew);
  * (income(s) = 1/2 + 1/2 sign(1, -n.(u + u2)/2)); where n.u changes sign along a face, the inflow point's part goes into the
  * neighbour's columns and the outflow point's into the element's own (HEAD picks one block per face from income(1)). */
 int pamg_unstr_set_velocity(pamg_handle* h, const double* u_ele);
+/* Boundary data of the domain-boundary faces (neig == 0) of the unstructured mesh, [E][3] in gmsh face order.  The codes are
+ * those of pamg_set_boundary_data: bc_kind 0 = sin(x+y) at the face's two nodes, 1 = the values bc_value[e][f][0..1] at the
+ * face nodes (l1, l2) = (1,3), (2,1), (3,2), linear along the face (NULL = zeros), 2 = open (no data, no penalty term; refused
+ * where a Gauss point of the face has inflow with a non-zero flux).  Entries of interior faces are ignored.  bc_kind = NULL
+ * returns to HEAD (no exterior trace on boundary faces: sn2 = 0).  With data, the face term of pamg_explicit_step and of the
+ * implicit operator takes its exterior trace g_s = sn(s,1) g1 + sn(s,2) g2 from the data and its exterior velocity from the
+ * element (u_bc = u_ele): an inflow Gauss point (the assembly's upwind rule) adds -c_s sn(s,.) g_s, c_s = sdetwei n.u_s, and
+ * with k > 0 the penalty adds k (L/2)/dx sum_s sn(s,.) g_s, both to the right-hand side of the implicit solve (computed by
+ * the assembly, added to (M/dt) told every time step) or to rhs of the explicit step.  An open face has no penalty term in
+ * the operator either.  t_bc of pamg_explicit_step stays the exterior value of the faces without data (a boundary face given
+ * fNeig >= 1 keeps HEAD's treatment too).
+ * Needs pamg_set_unstructured first (else PAMG_ERR_STATE), which clears the data.  E must be the mesh's E and every kind
+ * on a boundary face 0..2 (else PAMG_ERR_ARG, nothing changed).  Setting or clearing the data makes the assembled operator
+ * stale like pamg_unstr_set_velocity: pamg_implicit_step, _apply, _get_bsr, _set_stab, _precond_apply and _flow_levels
+ * return PAMG_ERR_STATE until the next pamg_implicit_assemble*.  An open face with inflow is refused with
+ * PAMG_ERR_UNSUPPORTED by the next assembly (the operator stays unassembled) or explicit step; pamg_last_error names the
+ * element and face.  The data adds no upwind edges: the flow levels of pamg_implicit_set_precond do not change.  On a
+ * multi-GPU handle it acts on part 0 like every unstructured entry. */
+int pamg_unstr_set_boundary(pamg_handle* h, int E, const int32_t* bc_kind, const double* bc_value);
 /* ntime x nits nonlinear iterations; njac_its Jacobi iterations on M x = M told + dt rhs, or the exact
  * register-resident local inverse when use_exact_minv != 0 (transport_rect.F90:277-291) */
 int pamg_explicit_step(pamg_handle* h, double dt, double u_x, double u_y, double t_bc, int ntime, int nits,

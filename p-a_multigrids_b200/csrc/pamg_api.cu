@@ -2079,6 +2079,20 @@ int pamg_unstr_set_velocity(pamg_handle* h, const double* u_ele) {
   return PAMG_OK;
 }
 
+int pamg_unstr_set_boundary(pamg_handle* h, int E, const int32_t* bc_kind, const double* bc_value) {
+  ON_PART0(h);
+  if (!h) return PAMG_ERR_ARG;
+  if (h->un.E < 1) return fail(h, PAMG_ERR_STATE, "pamg_set_unstructured has not been called");
+  if (E != h->un.E) return fail(h, PAMG_ERR_ARG, "pamg_unstr_set_boundary: E = " + std::to_string(E) + ", the mesh has " + std::to_string(h->un.E));
+  CK(cudaSetDevice(h->device));
+  std::string e;
+  long long nl = 0;
+  int rc = unstr_set_boundary(h->un, bc_kind, bc_value, h->nsm, h->stream, nl, e);
+  h->launches += nl;
+  if (rc) return fail(h, rc, e);
+  return PAMG_OK;
+}
+
 int pamg_unstr_upload(pamg_handle* h, const double* tnew) {
   ON_PART0(h);
   if (!h || !tnew || h->un.E < 1) return PAMG_ERR_ARG;

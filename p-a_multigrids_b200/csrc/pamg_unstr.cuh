@@ -78,7 +78,19 @@ struct UnstrDev {
   double flow_setup_ms[3] = {0.0, 0.0, 0.0};   // host time of the last build: mask (kernel + download), levels, upload
   int occ_flow = 0, occ_flow_vec = 0;
   std::vector<int32_t> neig_host;    // [E][3] as given to pamg_set_unstructured (the level computation runs on the host)
+  std::vector<int32_t> fneig_host;   // [E][3]
   std::vector<int32_t> flow_level_host;
+  // boundary data of the faces without an exterior trace (Nside = 0, i.e. neig = 0; pamg_unstr_set_boundary).  nbc = 0 and
+  // every pointer null: HEAD (sn2 = 0 on those faces).  Everything but bc_g is sized by the boundary elements.
+  int nbc = 0;                       // elements with at least one such face
+  double* bc_g = nullptr;            // [6][ld] exterior trace at the face nodes (l1, l2) of face f: planes 2f, 2f+1 (0 on an
+                                     //         open face); read only at faces with Nside = 0.  Allocated while data is set
+  int32_t* bc_list = nullptr;        // [nbc] those elements, ascending
+  int32_t* bc_open = nullptr;        // [nbc] bit f: face f is open (kind 2)
+  double* bc_pen = nullptr;          // [nbc][3] the penalty planes of these elements as built by the mesh (open faces get 0 in
+                                     //          `pen` while the data is set; restored from here when it is cleared)
+  double* bc_rhs = nullptr;          // [nbc][3] g_bc of the last assembly: inflow and penalty terms of the data
+  int32_t* bc_bad = nullptr;         // [1] lowest 3 e + f of an open face with inflow, INT32_MAX = none
 };
 
 inline size_t plane_stride(int E) {
@@ -180,6 +192,7 @@ struct UnstrArgs {
   size_t ld;
   int E, njac, exact, use_dir;
   const double* U;   // velocity planes (FIELD instantiation only); last, so the uniform kernel's parameter offsets stay put
+  const double* bcg; // boundary data planes (k_unstr_explicit_bc only); after U for the same reason
 };
 
 // unstr_explicit element loop (transport_tri_unstr.F90:600-791).  One warp = 32 consecutive elements per trip: all the
@@ -200,11 +213,16 @@ struct UnstrArgs {
 // FIELD: the velocity is the nodal field a.U (u_ele); the volume term takes ugi(g) = sum_i n(g,i) u(:,i) at the three
 // Gauss points and every face Gauss point its own upwind choice from the two traces.  The uniform instantiation is the
 // kernel as it was before the field existed.
+// BC: a face with Nside = 0 takes its exterior trace from the data planes a.bcg (pamg_unstr_set_boundary) and lets it in at
+// its inflow points; the exterior velocity is the element's own trace (u_bc = u_ele, :93).  Only such faces read the planes:
+// an interior element loads nothing more than without data.  Open faces hold 0 there; an open face with inflow was refused
+// before the launch (k_bc_rhs).
 #ifndef PAMG_OCC_EXPLICIT_FIELD
 #define PAMG_OCC_EXPLICIT_FIELD 2
 #endif
-template <bool FIELD>
-__global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OCC_EXPLICIT) k_unstr_explicit(UnstrArgs a) {
+template <bool FIELD, bool BC>
+__device__ __forceinline__ void unstr_explicit_body(const UnstrArgs& a) {
+  __builtin_assume(threadIdx.x < TPB);   // what __launch_bounds__ tells the kernel that inlines this
   __shared__ double smw[TPB / 32][2][96];
   const double al = 0.78867513459481288, be = 0.21132486540518712;  // sn_orig, ShapFun.F90:1100-1111
   // weights of int sn_c * trace over the face: (2/3, 1/3) -- exact products of the 2-point Gauss rule
@@ -301,6 +319,31 @@ __global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OC
       rhs[l1] -= ca; rhs[l2] -= cb;                     // :742-746
     }
     }
+    if constexpr (BC) {
+      // the data's inflow term, after HEAD's face loop (which gives these faces nothing: sn2 = 0), so that every other
+      // operation rounds as in k_unstr_explicit: zero data reproduces it bit for bit.  One branch for the whole element:
+      // interior elements (all but O(sqrt E)) skip it instead of predicating the face fluxes.  The data is loaded here, not
+      // with the other streaming loads: held across the flux loop it made the uniform kernel spill
+      const bool bnd = ((enc[0] & 3) == 0) | ((enc[1] & 3) == 0) | ((enc[2] & 3) == 0);
+      if (bnd)
+#pragma unroll
+      for (int f = 0; f < 3; ++f) {
+        if ((enc[f] & 3) != 0) continue;
+        const int l1 = L1[f], l2 = L2[f];
+        const double gA = __ldg(a.bcg + (size_t)(2 * f) * ld + e), gB = __ldg(a.bcg + (size_t)(2 * f + 1) * ld + e);
+        if constexpr (FIELD) {
+#pragma unroll
+          for (int s = 0; s < 2; ++s) {
+            const double a1 = s == 0 ? al : be, a2 = s == 0 ? be : al;
+            const double c = face_flux(g, l1, l2, L3[f], a1 * ux[l1] + a2 * ux[l2], a1 * uy[l1] + a2 * uy[l2]);
+            if (upwind_in(c)) { const double fl = c * (a1 * gA + a2 * gB); rhs[l1] -= a1 * fl; rhs[l2] -= a2 * fl; }
+          }
+        } else {
+          const double c = face_flux(g, l1, l2, L3[f], a.ux, a.uy);
+          if (upwind_in(c)) { rhs[l1] -= c * (w2 * gA + w1 * gB); rhs[l2] -= c * (w1 * gA + w2 * gB); }
+        }
+      }
+    }
     const double area = 0.5 * fabs(g.detj);
     const double m12 = area * (1.0 / 12.0);
     const double iarea = 1.0 / area;
@@ -336,6 +379,111 @@ __global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OC
     __syncwarp();
   }
 }
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OCC_EXPLICIT) k_unstr_explicit(UnstrArgs a) {
+  unstr_explicit_body<FIELD, false>(a);
+}
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB, FIELD ? PAMG_OCC_EXPLICIT_FIELD : PAMG_OCC_EXPLICIT) k_unstr_explicit_bc(UnstrArgs a) {
+  unstr_explicit_body<FIELD, true>(a);
+}
+
+// ---- boundary data (pamg_unstr_set_boundary) ------------------------------------------------------------------------------
+// Per element of the compact list bc_list, the data's part of the face term, with the exterior trace g_s = sn(s,1) g1 +
+// sn(s,2) g2 on a face with Nside = 0 and the exterior velocity the element's own trace:
+//   inflow Gauss point (the assembly's upwind_in of c_s = sdetwei n.u_s):  -c_s sn(s, .) g_s
+//   penalty (k > 0, face not open):                                        +k pen sum_s sn(s, .) g_s
+// i.e. exactly what k_assemble_bsr leaves out of the matrix on such a face ("sn2 = 0 -> no block", "only the own part
+// stays").  rhs = null: only the check.  An open face with an inflow point of non-zero flux (k_flow_mask's rule) sets *bad
+// to the lowest 3 e + f.  One thread per element (an element may have two boundary faces): no atomics on rhs.
+struct BcArgs {
+  const double* X; const int32_t* nside; const double* pen; const double* U; const double* g;
+  const int32_t* list; const int32_t* open; double* rhs; int32_t* bad;
+  double ux, uy, kdiff;
+  size_t ld;
+  int n;
+};
+template <bool FIELD>
+__global__ void __launch_bounds__(TPB) k_bc_rhs(BcArgs a) {
+  const double al = 0.78867513459481288, be = 0.21132486540518712;
+  const double w2 = al * al + be * be, w1 = 2.0 * al * be;
+  const size_t ld = a.ld;
+  const int L1[3] = {0, 1, 2}, L2[3] = {2, 0, 1}, L3[3] = {1, 2, 0};
+  for (int j = blockIdx.x * TPB + threadIdx.x; j < a.n; j += gridDim.x * TPB) {
+    const int e = __ldg(a.list + j), om = __ldg(a.open + j);
+    TriEdges g;
+    tri_edges(a.X, ld, (size_t)e, g);
+    double ux[3], uy[3];
+    if constexpr (FIELD) load_vel(a.U, ld, (size_t)e, ux, uy);
+    double r[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+    for (int f = 0; f < 3; ++f) {
+      if ((__ldg(a.nside + (size_t)f * ld + e) & 3) != 0) continue;
+      const int l1 = L1[f], l2 = L2[f];
+      const bool open = (om >> f) & 1;
+      const double g1 = __ldg(a.g + (size_t)(2 * f) * ld + e), g2 = __ldg(a.g + (size_t)(2 * f + 1) * ld + e);
+      bool inflow = false;
+      if constexpr (FIELD) {
+#pragma unroll
+        for (int s = 0; s < 2; ++s) {
+          const double a1 = s == 0 ? al : be, a2 = s == 0 ? be : al;
+          const double c = face_flux(g, l1, l2, L3[f], a1 * ux[l1] + a2 * ux[l2], a1 * uy[l1] + a2 * uy[l2]);
+          if (!upwind_in(c)) continue;
+          inflow |= c != 0.0;
+          const double gs = c * (a1 * g1 + a2 * g2);
+          r[l1] -= a1 * gs; r[l2] -= a2 * gs;
+        }
+      } else {
+        const double c = face_flux(g, l1, l2, L3[f], a.ux, a.uy);
+        if (upwind_in(c)) {
+          inflow = c != 0.0;
+          r[l1] -= c * (w2 * g1 + w1 * g2); r[l2] -= c * (w1 * g1 + w2 * g2);
+        }
+      }
+      if (open && inflow) atomicMin(a.bad, 3 * e + f);
+      if (!open && a.kdiff != 0.0) {
+        const double kp = a.kdiff * __ldg(a.pen + (size_t)f * ld + e);
+        r[l1] += kp * (w2 * g1 + w1 * g2); r[l2] += kp * (w1 * g1 + w2 * g2);
+      }
+    }
+    if (a.rhs) { a.rhs[(size_t)j * 3] = r[0]; a.rhs[(size_t)j * 3 + 1] = r[1]; a.rhs[(size_t)j * 3 + 2] = r[2]; }
+  }
+}
+// b += g_bc on the listed elements (one launch per time step of the implicit solve)
+__global__ void __launch_bounds__(TPB) k_bc_scatter(const int32_t* __restrict__ list, const double* __restrict__ rhs,
+                                                    double* __restrict__ b, int n) {
+  for (int j = blockIdx.x * TPB + threadIdx.x; j < n; j += gridDim.x * TPB) {
+    double* p = b + (size_t)__ldg(list + j) * 3;
+    p[0] += __ldg(rhs + (size_t)j * 3); p[1] += __ldg(rhs + (size_t)j * 3 + 1); p[2] += __ldg(rhs + (size_t)j * 3 + 2);
+  }
+}
+// set (restore = 0): keep the listed elements' penalty planes in `saved`, write the data into the planes bcg - vals[n][6], or
+// sin(x+y) at the face nodes where bit 3 + f of code[j] is set (kind 0) - and 0 into the penalty of open faces (bit f).
+// restore = 1: the penalty planes back from `saved`.
+__global__ void __launch_bounds__(TPB) k_bc_planes(const int32_t* __restrict__ list, const int32_t* __restrict__ code,
+                                                   const double* __restrict__ vals, double* __restrict__ bcg,
+                                                   const double* __restrict__ X, double* __restrict__ pen,
+                                                   double* __restrict__ saved, size_t ld, int n, int restore) {
+  for (int j = blockIdx.x * TPB + threadIdx.x; j < n; j += gridDim.x * TPB) {
+    const size_t e = (size_t)list[j];
+    if (restore) {
+      for (int f = 0; f < 3; ++f) pen[(size_t)f * ld + e] = saved[(size_t)j * 3 + f];
+      continue;
+    }
+    const int c = code[j];
+#pragma unroll
+    for (int f = 0; f < 3; ++f) {
+      saved[(size_t)j * 3 + f] = pen[(size_t)f * ld + e];
+      if ((c >> f) & 1) pen[(size_t)f * ld + e] = 0.0;
+      const int l[2] = {f, (f + 2) % 3};   // face nodes (l1, l2) = (1,3), (2,1), (3,2)
+#pragma unroll
+      for (int i = 0; i < 2; ++i)
+        bcg[(size_t)(2 * f + i) * ld + e] = ((c >> (3 + f)) & 1)
+                                              ? sin(X[(size_t)(2 * l[i]) * ld + e] + X[(size_t)(2 * l[i] + 1) * ld + e])
+                                              : vals[(size_t)j * 6 + 2 * f + i];
+    }
+  }
+}
 
 // [E][K] (ABI order) <-> [K][ld] planes; one thread per element (set-up and read-back only)
 template <typename Tp>
@@ -354,6 +502,7 @@ inline void unstr_free(UnstrDev& u) {
   cudaFree(u.bsr_val); cudaFree(u.bsr_col); cudaFree(u.dinv); cudaFree(u.mdt); cudaFree(u.work); cudaFree(u.dots); cudaFree(u.diag0); cudaFree(u.stab);
   cudaFree(u.xfer);
   cudaFree(u.flow_order); cudaFree(u.flow_level); cudaFree(u.flow_done); cudaFree(u.flow_ctl); cudaFree(u.flow_mask);
+  cudaFree(u.bc_g); cudaFree(u.bc_list); cudaFree(u.bc_open); cudaFree(u.bc_pen); cudaFree(u.bc_rhs); cudaFree(u.bc_bad);
   if (u.dots_host) cudaFreeHost(u.dots_host);
   u = UnstrDev();
 }
@@ -421,6 +570,7 @@ inline int unstr_setup(UnstrDev& u, int E, const double* X, const int32_t* neig,
   }
   u.E = E; u.ld = ld;
   u.neig_host.assign(neig, neig + (size_t)E * 3);
+  u.fneig_host.assign(fneig, fneig + (size_t)E * 3);
   UCK(cudaMalloc(&u.X, ld * 6 * sizeof(double)));
   UCK(cudaMalloc(&u.neig, ld * 3 * sizeof(int32_t)));
   UCK(cudaMalloc(&u.nside, ld * 3 * sizeof(int32_t)));
@@ -462,19 +612,128 @@ inline int unstr_set_velocity(UnstrDev& u, const double* u_ele, int nsm, cudaStr
   return rc;
 }
 
+// Boundary data of the faces with Nside = 0 (pamg_unstr_set_boundary), kind [E][3] / value [E][3][2] in the ABI's order;
+// kind = null clears it.  The kinds are checked before anything changes; the operator assembled before is stale either way.
+constexpr int32_t BC_NONE = 0x7f7f7f7f;   // *bc_bad when no open face has inflow (a memset of 0x7f bytes)
+inline void bc_free(UnstrDev& u) {
+  cudaFree(u.bc_g); cudaFree(u.bc_list); cudaFree(u.bc_open); cudaFree(u.bc_pen); cudaFree(u.bc_rhs); cudaFree(u.bc_bad);
+  u.bc_g = nullptr; u.bc_pen = u.bc_rhs = nullptr; u.bc_list = u.bc_open = u.bc_bad = nullptr;
+  u.nbc = 0;
+}
+inline int unstr_set_boundary(UnstrDev& u, const int32_t* kind, const double* value, int nsm, cudaStream_t st,
+                              long long& nlaunch, std::string& err) {
+  const int E = u.E;
+  std::vector<int32_t> list, code;
+  std::vector<double> vals;
+  if (kind) {
+    for (int e = 0; e < E; ++e) {
+      int c = 0;
+      bool any = false;
+      double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+      for (int f = 0; f < 3; ++f) {
+        const size_t i = (size_t)e * 3 + f;
+        if (u.neig_host[i] != 0) continue;
+        const int k = kind[i];
+        if (k < 0 || k > 2) {
+          err = "bc_kind[" + std::to_string(e) + "][" + std::to_string(f) + "] = " + std::to_string(k) +
+                " on a boundary face: 0 (sin(x+y)), 1 (values) or 2 (open)";
+          return PAMG_ERR_ARG;
+        }
+        if (u.fneig_host[i] != 0) continue;   // a boundary face the caller paired (Nside >= 1) keeps HEAD's treatment
+        any = true;
+        if (k == 2) c |= 1 << f;
+        else if (k == 0) c |= 8 << f;
+        else if (value) { v[2 * f] = value[i * 2]; v[2 * f + 1] = value[i * 2 + 1]; }
+      }
+      if (any) { list.push_back(e); code.push_back(c); vals.insert(vals.end(), v, v + 6); }
+    }
+  }
+  u.assembled = false;
+  u.with_stab = false;
+  if (u.nbc > 0) {   // the mesh's penalty planes back first
+    k_bc_planes<<<std::max(1, std::min((u.nbc + TPB - 1) / TPB, nsm * 8)), TPB, 0, st>>>(u.bc_list, u.bc_open, nullptr, nullptr,
+                                                                                        u.X, u.pen, u.bc_pen, u.ld, u.nbc, 1);
+    nlaunch++;
+    UCK(cudaGetLastError());
+    UCK(cudaStreamSynchronize(st));
+  }
+  bc_free(u);
+  if (list.empty()) return PAMG_OK;
+  const int n = (int)list.size();
+  double* d_vals = nullptr;
+  int rc = PAMG_OK;
+  auto ck = [&](cudaError_t e1) {
+    if (e1 != cudaSuccess && rc == PAMG_OK) { err = std::string("pamg_unstr_set_boundary: ") + cudaGetErrorString(e1); rc = PAMG_ERR_CUDA; }
+    return rc == PAMG_OK;
+  };
+  ck(cudaMalloc(&u.bc_g, u.ld * 6 * sizeof(double))) && ck(cudaMalloc(&u.bc_list, n * sizeof(int32_t))) &&
+      ck(cudaMalloc(&u.bc_open, n * sizeof(int32_t))) && ck(cudaMalloc(&u.bc_pen, (size_t)n * 3 * sizeof(double))) &&
+      ck(cudaMalloc(&u.bc_rhs, (size_t)n * 3 * sizeof(double))) && ck(cudaMalloc(&u.bc_bad, sizeof(int32_t))) &&
+      ck(cudaMalloc(&d_vals, (size_t)n * 6 * sizeof(double))) &&
+      ck(cudaMemsetAsync(u.bc_g, 0, u.ld * 6 * sizeof(double), st)) &&
+      ck(cudaMemsetAsync(u.bc_rhs, 0, (size_t)n * 3 * sizeof(double), st)) &&
+      ck(cudaMemcpyAsync(u.bc_list, list.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st)) &&
+      ck(cudaMemcpyAsync(u.bc_open, code.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st)) &&
+      ck(cudaMemcpyAsync(d_vals, vals.data(), (size_t)n * 6 * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (rc == PAMG_OK) {
+    k_bc_planes<<<std::max(1, std::min((n + TPB - 1) / TPB, nsm * 8)), TPB, 0, st>>>(u.bc_list, u.bc_open, d_vals, u.bc_g, u.X,
+                                                                                    u.pen, u.bc_pen, u.ld, n, 0);
+    nlaunch++;
+    ck(cudaGetLastError()) && ck(cudaStreamSynchronize(st));
+  }
+  cudaFree(d_vals);
+  if (rc != PAMG_OK) { bc_free(u); return rc; }   // (the penalty planes are only written by a kernel that ran to the end)
+  u.nbc = n;
+  return PAMG_OK;
+}
+
+// k_bc_rhs on the current velocity: rhs = u.bc_rhs (assembly) or null (the open-face check of an explicit step).  The verdict
+// is read by bc_verdict after the next synchronisation.
+inline int bc_launch(UnstrDev& u, double ux, double uy, double kdiff, bool with_rhs, int nsm, cudaStream_t st,
+                     long long& nlaunch, std::string& err) {
+  UCK(cudaMemsetAsync(u.bc_bad, 0x7f, sizeof(int32_t), st));
+  BcArgs b;
+  b.X = u.X; b.nside = u.nside; b.pen = u.pen; b.U = u.U; b.g = u.bc_g; b.list = u.bc_list; b.open = u.bc_open;
+  b.rhs = with_rhs ? u.bc_rhs : nullptr; b.bad = u.bc_bad; b.ux = ux; b.uy = uy; b.kdiff = kdiff; b.ld = u.ld; b.n = u.nbc;
+  const int grid = std::max(1, std::min((u.nbc + TPB - 1) / TPB, nsm * 8));
+  if (u.U) k_bc_rhs<true><<<grid, TPB, 0, st>>>(b);
+  else k_bc_rhs<false><<<grid, TPB, 0, st>>>(b);
+  nlaunch++;
+  UCK(cudaGetLastError());
+  return PAMG_OK;
+}
+inline int bc_verdict(UnstrDev& u, cudaStream_t st, std::string& err) {
+  int32_t bad = BC_NONE;
+  UCK(cudaMemcpyAsync(&bad, u.bc_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  UCK(cudaStreamSynchronize(st));
+  if (bad == BC_NONE) return PAMG_OK;
+  err = "open boundary face with inflow: element " + std::to_string(bad / 3) + " (0-based), face " + std::to_string(bad % 3 + 1) +
+        " (gmsh order); an inflow face needs data (bc_kind 0 or 1)";
+  return PAMG_ERR_UNSUPPORTED;
+}
+
 // time loop of unstr_explicit (:588-795): told = tnew ; nits x { tnew = tnew_nonlin ; element loop }
 inline int unstr_step(UnstrDev& u, double dt, double ux, double uy, double t_bc, int ntime, int nits, int njac,
                       int exact, int use_dir, int nsm, cudaStream_t st, long long& nlaunch, std::string& err) {
   const int grid = u.U ? stream_grid(k_unstr_explicit<true>, u.occ_explicit_f, u.E, nsm)
                        : stream_grid(k_unstr_explicit<false>, u.occ_explicit, u.E, nsm);
+  const bool bc = u.nbc > 0;   // (the data instantiations have the same launch bounds and resources per CTA)
+  if (bc) {   // open faces with inflow: once per call, the velocity does not change inside it
+    int rc = bc_launch(u, ux, uy, 0.0, false, nsm, st, nlaunch, err);
+    if (rc == PAMG_OK) rc = bc_verdict(u, st, err);
+    if (rc != PAMG_OK) return rc;
+  }
   for (int it = 0; it < ntime; ++it) {
     UCK(cudaMemcpyAsync(u.told, u.T[u.cur], (size_t)u.E * 3 * sizeof(double), cudaMemcpyDeviceToDevice, st));
     for (int k = 0; k < nits; ++k) {
       UnstrArgs a;
       a.X = u.X; a.neig = u.neig; a.nside = u.nside; a.Tin = u.T[u.cur]; a.told = u.told; a.Tout = u.T[u.cur ^ 1];
       a.dt = dt; a.ux = ux; a.uy = uy; a.t_bc = t_bc; a.ld = u.ld; a.E = u.E; a.njac = njac; a.exact = exact; a.use_dir = use_dir;
-      a.U = u.U;
-      if (u.U) k_unstr_explicit<true><<<grid, TPB, 0, st>>>(a);
+      a.U = u.U; a.bcg = u.bc_g;
+      if (bc) {
+        if (u.U) k_unstr_explicit_bc<true><<<grid, TPB, 0, st>>>(a);
+        else k_unstr_explicit_bc<false><<<grid, TPB, 0, st>>>(a);
+      } else if (u.U) k_unstr_explicit<true><<<grid, TPB, 0, st>>>(a);
       else k_unstr_explicit<false><<<grid, TPB, 0, st>>>(a);
       nlaunch++;
       UCK(cudaGetLastError());
@@ -1294,10 +1553,16 @@ inline int implicit_assemble(UnstrDev& u, double dt, double ux, double uy, doubl
   a.X = u.X; a.neig = u.neig; a.nside = u.nside; a.pen = u.pen; a.val = u.bsr_val; a.col = u.bsr_col; a.dinv = u.dinv;
   a.mdt = u.mdt;
   a.inv24dt = 1.0 / (24.0 * dt); a.ux = ux; a.uy = uy; a.kdiff = kdiff; a.ld = ld; a.E = u.E; a.use_dir = use_dir; a.U = u.U;
+  u.assembled = false;
   if (u.U) k_assemble_bsr<true><<<stream_grid(k_assemble_bsr<true>, u.occ_assemble_f, u.E, nsm), TPB, 0, st>>>(a);
   else k_assemble_bsr<false><<<stream_grid(k_assemble_bsr<false>, u.occ_assemble, u.E, nsm), TPB, 0, st>>>(a);
   nlaunch++;
   UCK(cudaGetLastError());
+  if (u.nbc > 0) {   // g_bc of this velocity, k and data; refused (operator left unassembled) for an open face with inflow
+    int rc = bc_launch(u, ux, uy, kdiff, true, nsm, st, nlaunch, err);
+    if (rc == PAMG_OK) rc = bc_verdict(u, st, err);
+    if (rc != PAMG_OK) return rc;
+  }
   u.assembled = true; u.dt = dt; u.ux = ux; u.uy = uy; u.kdiff = kdiff; u.use_dir = use_dir;
   return PAMG_OK;
 }
@@ -1343,6 +1608,10 @@ inline int implicit_step(UnstrDev& u, int ntime, int nits, double tol, int max_i
       if (k == 0) {
         UCK(cudaMemcpyAsync(u.told, a.x, (size_t)n * sizeof(double), cudaMemcpyDeviceToDevice, st));
         k_block_apply<<<g_apply, TPB, 0, st>>>(u.dinv, u.mdt, u.told, a.b, E, u.ld, 1); nlaunch++;
+        if (u.nbc > 0) {   // + g_bc of the boundary data (pamg_unstr_set_boundary)
+          k_bc_scatter<<<std::max(1, std::min((u.nbc + TPB - 1) / TPB, nsm * 8)), TPB, 0, st>>>(u.bc_list, u.bc_rhs, a.b, u.nbc);
+          nlaunch++;
+        }
       }
       if (u.with_stab) {   // INTENDED use (:367-368 commented at HEAD): diagonal blocks += stab(tnew_nonlin, told)
         StabArgs sa;

@@ -107,6 +107,7 @@ def lib():
         "pamg_halo_peer_info": (ci, [vp, ci, pint, pint]),
         "pamg_set_unstructured": (ci, [vp, ci, _f64, _i32, _i32]),
         "pamg_unstr_set_velocity": (ci, [vp, vp]),
+        "pamg_unstr_set_boundary": (ci, [vp, ci, vp, vp]),
         "pamg_unstr_upload": (ci, [vp, _f64]),
         "pamg_unstr_download": (ci, [vp, _f64]),
         "pamg_explicit_step": (ci, [vp, cd, cd, cd, cd, ci, ci, ci, ci, ci]),
@@ -511,6 +512,24 @@ class SemiImplicitIterative:
             raise ValueError(f"u_ele must have shape (E, 3, 2) = ({self._E}, 3, 2), got {u.shape}")
         self._ck(self.L.pamg_unstr_set_velocity(self.h, _ptr(u)))
 
+    def set_unstructured_boundary(self, bc_kind, bc_value=None):
+        """Boundary data of the domain-boundary faces of the unstructured mesh (pamg_unstr_set_boundary): bc_kind (E, 3) in
+        gmsh face order, 0 = sin(x+y) at the face nodes, 1 = bc_value[e, f] = (value at l1, value at l2) with (l1, l2) = (1,3),
+        (2,1), (3,2), 2 = open (no data, no penalty; refused where the face has inflow); bc_value (E, 3, 2) or None (zeros).
+        Entries of interior faces are ignored.  None returns to no exterior trace on boundary faces (HEAD).  Call
+        implicit_assemble again before the implicit entries: the operator assembled before is stale."""
+        if bc_kind is None:
+            self._ck(self.L.pamg_unstr_set_boundary(self.h, getattr(self, "_E", 0), None, None))
+            return
+        kind = np.ascontiguousarray(bc_kind, np.int32)
+        val = None if bc_value is None else np.ascontiguousarray(bc_value, np.float64)
+        if hasattr(self, "_E"):                                     # (without a mesh the library answers ERR_STATE)
+            if kind.shape != (self._E, 3):
+                raise ValueError(f"bc_kind must have shape (E, 3) = ({self._E}, 3), got {kind.shape}")
+            if val is not None and val.shape != (self._E, 3, 2):
+                raise ValueError(f"bc_value must have shape (E, 3, 2) = ({self._E}, 3, 2), got {val.shape}")
+        self._ck(self.L.pamg_unstr_set_boundary(self.h, kind.shape[0] if kind.ndim else 0, _ptr(kind), _ptr(val)))
+
     def unstr_explicit(self, tnew, dt, u_x, u_y, ntime=2, nits=2, njac_its=10, t_bc=0.0, exact_minv=False,
                        use_dir=False):
         t = np.ascontiguousarray(tnew, np.float64)
@@ -582,12 +601,12 @@ class SemiImplicitIterative:
         return ms.value, setup
 
     def unstr_implicit(self, tnew, dt, u_x, u_y, ntime=2, nits=1, use_dir=False, tol=1e-13, max_iters=500, with_stab=False,
-                       precond="block_jacobi"):
+                       precond="block_jacobi", k=0.0):
         """Time loop of unstr_implicit; returns (tnew, Krylov iterations in total, worst relative residual).  precond:
-        "block_jacobi" or "flow_gs" (implicit_set_precond)."""
+        "block_jacobi" or "flow_gs" (implicit_set_precond); k > 0 adds the diffusion operator (implicit_assemble)."""
         t = np.ascontiguousarray(tnew, np.float64)
         self.implicit_set_precond(precond)
-        self.implicit_assemble(dt, u_x, u_y, use_dir)
+        self.implicit_assemble(dt, u_x, u_y, use_dir, k)
         if with_stab:
             self._ck(self.L.pamg_implicit_set_stab(self.h, 1))
         self._ck(self.L.pamg_unstr_upload(self.h, t))

@@ -34,7 +34,7 @@ NULLABLE_IN = {"pamg_mesh_get": {"X", "neig", "fneig", "dir", "region"},
                "pamg_timestep_host": {"cycles", "relres"}, "pamg_implicit_step": {"iters_total", "relres"},
                "pamg_halo_peer_info": {"peer_part", "nfaces"}, "pamg_parent_table": {"bc_kind"},
                "pamg_unstr_set_velocity": {"u_ele"}, "pamg_implicit_flow_levels": {"level"},
-               "pamg_implicit_flow_time": {"setup_ms"}}
+               "pamg_implicit_flow_time": {"setup_ms"}, "pamg_unstr_set_boundary": {"bc_kind", "bc_value"}}
 
 FTYPE = {"int": "integer(c_int)", "int32_t": "integer(c_int32_t)", "int64_t": "integer(c_int64_t)", "double": "real(c_double)",
          "float": "real(c_float)"}
