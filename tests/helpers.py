@@ -70,6 +70,56 @@ def strip_mesh(nsq=15):
     return np.array(X, np.float64)
 
 
+PERMUTATIONS = ((0, 1, 2), (0, 2, 1), (1, 0, 2), (1, 2, 0), (2, 0, 1), (2, 1, 0))
+
+
+def random_parent_triangulation(seed, m=4, jitter=0.3):
+    """(pts, simplices, neighbours) of a jittered (m+1) x (m+1) grid on the unit square: interior points moved by up to
+    jitter/m in x and y (MT19937(seed)), Delaunay triangles, the vertices of each triangle in a random one of the 6 orders.
+    neighbours[:, i] is the triangle opposite vertex i of the reordered simplex (-1: domain boundary), as in Delaunay."""
+    from scipy.spatial import Delaunay
+    assert 0.0 <= jitter < 0.5
+    rng = np.random.Generator(np.random.MT19937(seed))
+    g = np.linspace(0.0, 1.0, m + 1)
+    pts = np.stack(np.meshgrid(g, g, indexing="ij"), axis=-1).reshape(-1, 2)
+    inner = np.all((pts > 0.0) & (pts < 1.0), axis=1)
+    pts[inner] += (jitter / m) * (2.0 * rng.random((int(inner.sum()), 2)) - 1.0)
+    tri = Delaunay(pts)
+    order = np.array(PERMUTATIONS)[rng.integers(0, len(PERMUTATIONS), len(tri.simplices))]
+    return pts, np.take_along_axis(tri.simplices, order, axis=1), np.take_along_axis(tri.neighbors, order, axis=1)
+
+
+def random_parent_mesh(seed, m=4, jitter=0.3):
+    """Parents X[U,3,2] of random_parent_triangulation.  The vertex order decides which gmsh side of a parent a face is and
+    its orientation, so such a mesh pairs every parent side with every neighbour side in both reversal senses (see
+    face_combinations), which meshes built with one orientation rule, or flipped by one fixed swap, never do.  jitter < 1/2
+    keeps the triangles well shaped: the minimum angle is asserted to be at least 15 degrees."""
+    pts, simplices, _ = random_parent_triangulation(seed, m, jitter)
+    X = np.ascontiguousarray(pts[simplices])
+    assert min_angle_deg(X) >= 15.0, (seed, min_angle_deg(X))
+    return X
+
+
+def min_angle_deg(X):
+    ang = []
+    for i in range(3):
+        a = X[:, (i + 1) % 3] - X[:, i]
+        b = X[:, (i + 2) % 3] - X[:, i]
+        c = np.sum(a * b, axis=1) / (np.linalg.norm(a, axis=1) * np.linalg.norm(b, axis=1))
+        ang.append(np.degrees(np.arccos(np.clip(c, -1.0, 1.0))))
+    return float(np.min(ang))
+
+
+def face_combinations(neig, fneig, dirv):
+    """{(s, ns, dir)} over the interior faces: my gmsh side s (1-3), the neighbour's side ns = fNeig (1-3) and the reversal
+    flag Dir (0/1) of the face.  These three pick the branch of the halo tables a face takes; there are 18 of them."""
+    u, f = np.nonzero(np.asarray(neig) != 0)
+    return {(int(f_ + 1), int(fneig[a, f_]), int(dirv[a, f_])) for a, f_ in zip(u, f)}
+
+
+ALL_FACE_COMBINATIONS = {(s, ns, d) for s in (1, 2, 3) for ns in (1, 2, 3) for d in (0, 1)}
+
+
 def write_msh_triangles(X, path, region=1):
     """gmsh 2.2 ASCII file of free-standing triangles X[U,3,2] (coincident vertices are merged)."""
     ids, nodes, tris = {}, [], []

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import oracle_api as orc
-from helpers import child_coordinates, write_msh
+from helpers import child_coordinates, random_parent_mesh, write_msh
 from pamg_pkg import pamg
 
 SIDE_FACE_NODES = [(0, 2), (1, 0), (2, 1)]      # parent gmsh side 1, 2, 3 = child face f1 (1,3), f3 (2,1), f2 (3,2)
@@ -78,16 +78,24 @@ def test_cut_faces_of_a_partition_keep_their_strips():
                     assert src[u - first, mf].max() < (last - first) * 4 ** n * 3
 
 
-@pytest.mark.parametrize("seed,npts", [(2, 14), (7, 60)])
-@pytest.mark.parametrize("rule", [0, 1])
-def test_exterior_values_on_random_triangulations_with_mixed_orientation(seed, npts, rule):
+def random_triangles(seed, npts):
+    """X[U,3,2]: npts random points with half the triangles flipped by one swap, or (npts None) the jittered grid with every
+    triangle in a random vertex order, which holds all 18 (side, neighbour side, Dir) pairings (helpers.random_parent_mesh)."""
+    if npts is None:
+        return random_parent_mesh(seed)
     from scipy.spatial import Delaunay
     rng = np.random.Generator(np.random.MT19937(seed))
     pts = rng.random((npts, 2))
     simplices = Delaunay(pts).simplices.copy()
     flip = rng.random(len(simplices)) < 0.5
     simplices[flip] = simplices[flip][:, [0, 2, 1]]
-    m = pamg.Mesh.from_arrays(pts[simplices])
+    return pts[simplices]
+
+
+@pytest.mark.parametrize("seed,npts", [(2, 14), (7, 60), pytest.param(2, None, id="permuted-grid-2")])
+@pytest.mark.parametrize("rule", [0, 1])
+def test_exterior_values_on_random_triangulations_with_mixed_orientation(seed, npts, rule):
+    m = pamg.Mesh.from_arrays(random_triangles(seed, npts))
     n = 2
     S = 2 ** n
     T = continuous_field(child_coordinates(orc, m.X, n))
@@ -96,6 +104,14 @@ def test_exterior_values_on_random_triangulations_with_mixed_orientation(seed, n
     orc.lib().orc_surf_ele(n, surf)
     surf = surf.reshape(3, S)
     src = pamg.halo_sources(m, n, halo_rule=rule)
+    # the strips as the reference fills them (its reversal table under halo_rule 0, geometry under 1)
+    p = orc.intended_params(n, 1)
+    p.halo_rule = rule
+    s = orc.Semi(p, m.X, m.neig, m.fneig, m.dir)
+    s.field(orc.TNEW, 1)[:] = T
+    s.update_overlaps(1)
+    ovl = s.overlap(1)
+    hmap = pamg.halo_plan(m, halo_rule=rule)["hmap"].reshape(m.U, 3)
     for u in range(m.U):
         for mf in range(3):
             if m.neig[u, mf] == 0:
@@ -104,3 +120,6 @@ def test_exterior_values_on_random_triangulations_with_mixed_orientation(seed, n
             own = T[u, surf[mf] - 1]
             assert np.abs(flat[src[u, mf, :, 0]] - own[:, a]).max() <= 1e-12
             assert np.abs(flat[src[u, mf, :, 1]] - own[:, b]).max() <= 1e-12
+            hm = int(hmap[u, mf])
+            assert np.array_equal(flat[src[u, mf, :, 0]], ovl[u, mf, :, hm & 3])
+            assert np.array_equal(flat[src[u, mf, :, 1]], ovl[u, mf, :, hm >> 2])

@@ -9,15 +9,18 @@ import pytest
 from scipy.spatial import Delaunay
 
 import oracle_api as orc
-from helpers import write_msh_triangles
+from helpers import random_parent_triangulation, write_msh_triangles
 from pamg_pkg import pamg
 
 OPPOSITE = [1, 2, 0]                     # gmsh side 1, 2, 3 -> the vertex (0-based) it lies opposite
 SIDE_NODES = [(0, 2), (0, 1), (1, 2)]
 
 
-@pytest.mark.parametrize("seed,npts", [(1, 12), (2, 40), (3, 150), (4, 600)])
-def test_edge_hash_neighbours_equal_delaunay_and_the_reference_search(seed, npts, tmp_path):
+def triangulation(seed, npts):
+    """(pts, simplices, neighbours): npts random points with half the triangles flipped, or (npts None) the permuted jittered
+    grid of helpers.random_parent_triangulation, which pairs every gmsh side with every other in both reversal senses."""
+    if npts is None:
+        return random_parent_triangulation(seed)
     rng = np.random.Generator(np.random.MT19937(seed))
     pts = rng.random((npts, 2))
     tri = Delaunay(pts)
@@ -26,6 +29,12 @@ def test_edge_hash_neighbours_equal_delaunay_and_the_reference_search(seed, npts
     simplices[flip] = simplices[flip][:, [0, 2, 1]]
     nbrs = tri.neighbors.copy()
     nbrs[flip] = nbrs[flip][:, [0, 2, 1]]
+    return pts, simplices, nbrs
+
+
+@pytest.mark.parametrize("seed,npts", [(1, 12), (2, 40), (3, 150), (4, 600), pytest.param(2, None, id="permuted-grid-2")])
+def test_edge_hash_neighbours_equal_delaunay_and_the_reference_search(seed, npts, tmp_path):
+    pts, simplices, nbrs = triangulation(seed, npts)
     X = pts[simplices]
     m = pamg.Mesh.from_arrays(X)
     U = len(simplices)

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 import oracle_api as orc
-from helpers import rng_field, write_msh
+from helpers import random_parent_mesh, rng_field, write_msh
 from pamg_pkg import pamg
 
 FACE_NODES = [(0, 2), (2, 1), (1, 0)]        # child faces f1 (1,3), f2 (3,2), f3 (2,1): transport_tri_semi.F90:142-147
@@ -146,16 +146,21 @@ def test_parent_table_argument_errors(tmp_path):
     assert codes == {pamg.OK, pamg.ERR_UNSUPPORTED}
 
 
-@pytest.mark.parametrize("seed,npts", [(1, 8), (5, 20)])
+@pytest.mark.parametrize("seed,npts", [(1, 8), (5, 20), pytest.param(2, None, id="permuted-grid-2")])
 @pytest.mark.parametrize("theta", [1.0, 0.5])
 def test_folded_table_on_random_triangulations_with_mixed_orientation(seed, npts, theta, tmp_path):
-    from scipy.spatial import Delaunay
-    rng = np.random.Generator(np.random.MT19937(seed))
-    pts = rng.random((npts, 2))
-    simplices = Delaunay(pts).simplices.copy()
-    flip = rng.random(len(simplices)) < 0.5
-    simplices[flip] = simplices[flip][:, [0, 2, 1]]
-    mesh = pamg.Mesh.from_arrays(pts[simplices])
+    """npts None: the jittered grid with every triangle in a random vertex order (all 18 face pairings)."""
+    if npts is None:
+        X = random_parent_mesh(seed)
+    else:
+        from scipy.spatial import Delaunay
+        rng = np.random.Generator(np.random.MT19937(seed))
+        pts = rng.random((npts, 2))
+        simplices = Delaunay(pts).simplices.copy()
+        flip = rng.random(len(simplices)) < 0.5
+        simplices[flip] = simplices[flip][:, [0, 2, 1]]
+        X = pts[simplices]
+    mesh = pamg.Mesh.from_arrays(X)
     n = 2
     op = orc.intended_params(n, 1, dt=1e-2, k=0.05, u=(0.6, -0.3))
     op.theta = theta
