@@ -6,6 +6,7 @@
 #include <dlfcn.h>
 
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -116,8 +117,13 @@ struct pamg_handle {
   // resident CTAs per SM of the shared-memory kernels on THIS device ([face_terms]); set once per handle in configure_kernels
   struct KernelCfg { int win2[2] = {0, 0}, win2x = 0, win[2] = {0, 0}, tma[2] = {0, 0}, gs2 = 0, gs2x = 0, gs = 0, halo = 0; bool done = false; } kc;
   bool capturing = false;   // stream capture in progress: no synchronisation, no per-launch error polling
-  struct VcGraph { long long key; std::vector<cudaGraphExec_t> exec; std::vector<long long> launches; };   // one graph per GPU of the group
-  std::vector<VcGraph> vc_graphs;   // a few cached V-cycle graphs (solver / sweep counts / buffer parity)
+  // one graph per GPU of the group, and exactly what it was captured for: the schedule (solver, nu1, nu2, ncoarse, fuse) and
+  // the (cur, ovl_cur) of every level of every part and of the agglomerated coarse problem (vc_parity) at its start and end
+  struct VcGraph {
+    std::array<int, 5> sched; std::vector<int> parity, parity_end;
+    std::vector<cudaGraphExec_t> exec; std::vector<long long> launches;
+  };
+  std::vector<VcGraph> vc_graphs;   // a few cached V-cycle graphs
   bool graph_nccl = true;       // try to capture NCCL calls into the V-cycle graph (cleared when the library refuses)
   // per-kernel timing (element kernels only)
   bool profiling = false;
@@ -1137,6 +1143,23 @@ int vcycle_body(const Group& G, pamg_handle* owner, int solver, int nu1, int nu2
   return PAMG_OK;
 }
 
+// (cur, ovl_cur) of every level of every part, then of the coarse problem agglomerated on a part: the buffer choices a
+// captured V-cycle bakes in
+Group vc_handles(const Group& G) {
+  Group hs = G;
+  for (pamg_handle* q : G) if (q->agg) hs.push_back(q->agg);
+  return hs;
+}
+std::vector<int> vc_parity(const Group& G) {
+  std::vector<int> v;
+  for (pamg_handle* q : vc_handles(G)) for (const LevelDev& L : q->lev) { v.push_back(L.cur); v.push_back(L.ovl_cur); }
+  return v;
+}
+void set_vc_parity(const Group& G, const std::vector<int>& v) {
+  size_t i = 0;
+  for (pamg_handle* q : vc_handles(G)) for (LevelDev& L : q->lev) { L.cur = v[i++]; L.ovl_cur = v[i++]; }
+}
+
 // take back the norm sweep at the end of a fused body: the iterate it started from still sits in the other T buffer, and
 // the strips it read (local, unpacked cut faces) in the other strip buffer
 int undo_norm_sweep(pamg_handle* h) {
@@ -1795,20 +1818,18 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
     GALL(G, h, q, do_residual(q, 1, nullptr, nullptr, nullptr));      // leaves tracer%residuale of the final iterate, as before
     return PAMG_OK;
   };
-  const long long key0 = (((((long long)solver * 64 + nu1) * 64 + nu2) * 64 + ncoarse) * 2 + (fuse ? 1 : 0));
+  const std::array<int, 5> sched = {solver, nu1, nu2, ncoarse, fuse ? 1 : 0};
   // with NCCL in the cycle (halo exchange fallback, coarse gather/scatter) the capture is attempted once; if the library
   // refuses, the handle falls back to eager launches for good
   bool graph_ok = true;
   for (pamg_handle* q : G) graph_ok = graph_ok && !q->profiling && (!q->comm || q->graph_nccl);
   for (int c = 1; c <= max_cycles; ++c) {
     if (c >= 2 && graph_ok) {
-      // the graph bakes in which of the two T buffers holds the iterate and which strip buffer is current, on every level of
-      // every part (a hash: the product of the factors does not fit 64 bits for a group of GPUs)
-      unsigned long long hk = (unsigned long long)key0;
-      for (pamg_handle* q : G) for (auto& Lv : q->lev) hk = hk * 1000003ull + (unsigned long long)(Lv.cur * 2 + Lv.ovl_cur + 1);
-      const long long key = (long long)hk;
+      // the graph bakes in the schedule, and which of the two T buffers holds the iterate and which strip buffer is current,
+      // on every level of every part: a graph is replayed only when all of them are equal
+      const std::vector<int> parity = vc_parity(G);
       pamg_handle::VcGraph* vg = nullptr;
-      for (auto& g : h->vc_graphs) if (g.key == key) vg = &g;
+      for (auto& g : h->vc_graphs) if (g.sched == sched && g.parity == parity) vg = &g;
       if (!vg) {
         if (h->vc_graphs.size() >= 8) { for (auto e : h->vc_graphs.front().exec) cudaGraphExecDestroy(e); h->vc_graphs.erase(h->vc_graphs.begin()); }
         std::vector<long long> l0(G.size());
@@ -1824,7 +1845,8 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
         }
         rc = (ce == cudaSuccess) ? vcycle_body(G, h, solver, nu1, nu2, ncoarse, fuse, false) : PAMG_ERR_CUDA;
         pamg_handle::VcGraph ng;
-        ng.key = key;
+        ng.sched = sched;
+        ng.parity = parity;
         for (size_t i = 0; i < begun; ++i) {
           pamg_handle* q = G[i];
           if (q->in_group) cudaSetDevice(q->device);
@@ -1854,6 +1876,7 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
           if ((rc = vcycle_body(G, h, solver, nu1, nu2, ncoarse, fuse, false))) return rc;
           goto cycle_done;
         }
+        ng.parity_end = vc_parity(G);
         h->vc_graphs.push_back(ng);
         vg = &h->vc_graphs.back();
       }
@@ -1862,6 +1885,9 @@ int pamg_vcycle_solve(pamg_handle* h, int solver, int nu1, int nu2, int ncoarse,
         CK(cudaGraphLaunch(vg->exec[i], G[i]->stream));
         G[i]->launches += vg->launches[i];
       }
+      // a replay moves the buffers as the captured cycle did (with an odd sweep count on a level that is not normalised -
+      // level 1 of a fused solve, the strips of a producer level - the parity alternates and two graphs take turns)
+      set_vc_parity(G, vg->parity_end);
     } else {
       if ((rc = vcycle_body(G, h, solver, nu1, nu2, ncoarse, fuse, c == 1))) return rc;
     }
