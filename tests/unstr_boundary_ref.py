@@ -12,7 +12,7 @@ Kinds as in pamg_set_boundary_data: 0 = sin(x+y) at the face nodes, 1 = given va
 so the own penalty part leaves the matrix too)."""
 import numpy as np
 
-from velocity_field_ref import FACES, SN, Geometry, advection_rhs, implicit_matrix
+from velocity_field_ref import FACES, SN, Geometry, _assemble, advection_rhs, implicit_matrix
 
 OPEN = 2
 
@@ -71,21 +71,15 @@ def boundary_rhs(G, u, g, has, open_, k=0.0):
 
 def open_penalty(G, open_, k, sparse=False):
     """The own penalty blocks of the open faces that implicit_matrix contains and the library leaves out: (3E)^2."""
-    import scipy.sparse as sp
-    rows, cols, vals = [], [], []
-    if k != 0.0:
-        for f, (l1, l2) in enumerate(FACES):
-            kd = (k / _dx_boundary(G, f)) * G.sdet[:, f]
-            for e in np.nonzero(open_[:, f])[0]:
-                sn = np.zeros((2, 3))
-                for s in range(2):
-                    sn[s, l1], sn[s, l2] = SN[s]
-                b = kd[e] * sum(np.outer(sn[s], sn[s]) for s in range(2))
-                for i in range(3):
-                    for j in range(3):
-                        rows.append(3 * e + i); cols.append(3 * e + j); vals.append(b[i, j])
-    P = sp.csr_matrix((vals, (rows, cols)), shape=(3 * G.E, 3 * G.E))
-    return P if sparse else P.toarray()
+    P = []
+    for f, (l1, l2) in enumerate(FACES):
+        sn = np.zeros((2, 3))
+        for s in range(2):
+            sn[s, l1], sn[s, l2] = SN[s]
+        kd = (k / _dx_boundary(G, f)) * G.sdet[:, f] if k != 0.0 else np.zeros(G.E)
+        P.append(np.where(open_[:, f, None, None], kd[:, None, None] * sum(np.outer(sn[s], sn[s]) for s in range(2)), 0.0))
+    ar = np.arange(G.E)
+    return _assemble(ar, ar, P[0] + P[1] + P[2], 3 * G.E, sparse)
 
 
 def uniform(E, u):

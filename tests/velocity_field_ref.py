@@ -127,71 +127,68 @@ def implicit_matrix(X, neig, fneig, u, dt, k=0.0, use_dir=True, literal=False, s
     G = Geometry(X, neig, fneig, use_dir)
     u = np.asarray(u, np.float64)
     E = G.E
-    N = 3 * E
-    blocks, mblocks = {}, {}                                         # (row element, column element) -> 3x3
-
-    def add(store, e, c, b):
-        store[(e, c)] = store.get((e, c), 0.0) + b
+    ar = np.arange(E)
     cen = G.X.mean(axis=1)
     Mloc = (np.ones((3, 3)) + np.eye(3)) / 12.0
-    for e in range(E):
-        r = slice(3 * e, 3 * e + 3)
-        m = G.area[e] * Mloc / dt
-        stiff = np.zeros((3, 3))
-        for g, (i0, i1) in enumerate(GAUSS):
-            ug = 0.5 * (u[e, i0] + u[e, i1])
-            ng = np.zeros(3); ng[i0] = ng[i1] = 0.5
-            stiff += np.outer(G.grad[e] @ ug, ng) * G.area[e] / 3.0
-        add(mblocks, e, e, m)
-        add(blocks, e, e, m - stiff + k * G.area[e] * G.grad[e] @ G.grad[e].T)
+    m = G.area[:, None, None] * Mloc / dt
+    stiff = np.zeros((E, 3, 3))
+    for g, (i0, i1) in enumerate(GAUSS):
+        ug = 0.5 * (u[:, i0] + u[:, i1])
+        ng = np.zeros(3); ng[i0] = ng[i1] = 0.5
+        stiff += np.einsum("ei,j->eij", np.einsum("eid,ed->ei", G.grad, ug), ng) * G.area[:, None, None] / 3.0
+    diag = m - stiff + (k * G.area[:, None, None] * G.grad) @ G.grad.transpose(0, 2, 1)
+    off = np.zeros((3, E, 3, 3))                                     # block (e, neig[e, f] - 1) of face f
     for f, (l1, l2) in enumerate(FACES):
-        tr = [G.traces(u, f, s) for s in range(2)]
-        inc = [G.income(f, *tr[s]) for s in range(2)]
+        q, ns = G.neig[:, f], G.fneig[:, f]
+        inner = q != 0
+        m1, m2 = G.m[:, f, 0], G.m[:, f, 1]
+        sn = np.zeros((2, 3)); sn2 = np.zeros((E, 2, 3))
+        has = ar[ns >= 1]
+        for s in range(2):
+            sn[s, l1], sn[s, l2] = SN[s]
+            sn2[has, s, m1[has]], sn2[has, s, m2[has]] = SN[s]
         n = G.normal[:, f]
-        for e in range(E):
-            q, ns = int(G.neig[e, f]), int(G.fneig[e, f])
-            m1, m2 = G.m[e, f]
-            sn = np.zeros((2, 3)); sn2 = np.zeros((2, 3))
-            for s in range(2):
-                sn[s, l1], sn[s, l2] = SN[s]
-                if ns >= 1:
-                    sn2[s, m1], sn2[s, m2] = SN[s]
-            own = np.zeros((3, 3)); nbr = np.zeros((3, 3))
-            for s in range(2):
-                c = G.sdet[e, f] * (n[e] @ tr[s][0][e]); c2 = G.sdet[e, f] * (n[e] @ tr[s][1][e])
-                own += (1.0 - inc[s][e]) * c * np.outer(sn[s], sn[s])
-                nbr += inc[s][e] * c2 * np.outer(sn[s], sn2[s])
-            if literal:
-                target = (e + 1) if inc[0][e] == 0.0 else q
-                if target == 0:
-                    target = e + 1
-                add(blocks, e, target - 1, own + nbr)
-            else:
-                add(blocks, e, e, own)
-                add(blocks, e, (q - 1) if q != 0 else e, nbr)
-            if k != 0.0:
-                if q != 0:
-                    dx = np.linalg.norm(cen[e] - cen[q - 1])
-                else:
-                    dx = np.linalg.norm(cen[e] - 0.5 * (G.X[e, l1] + G.X[e, l2]))
-                add(blocks, e, e, (k / dx) * G.sdet[e, f] * sum(np.outer(sn[s], sn[s]) for s in range(2)))
-                if q != 0:
-                    add(blocks, e, q - 1, -(k / dx) * G.sdet[e, f] * sum(np.outer(sn[s], sn2[s]) for s in range(2)))
-    return _assemble(blocks, N, sparse), _assemble(mblocks, N, sparse)
+        own = np.zeros((E, 3, 3)); nbr = np.zeros((E, 3, 3))
+        for s in range(2):
+            us, us2 = G.traces(u, f, s)
+            inc = G.income(f, us, us2)
+            c = G.sdet[:, f] * np.einsum("ed,ed->e", n, us); c2 = G.sdet[:, f] * np.einsum("ed,ed->e", n, us2)
+            own += ((1.0 - inc) * c)[:, None, None] * np.outer(sn[s], sn[s])
+            nbr += (inc * c2)[:, None, None] * np.einsum("i,ej->eij", sn[s], sn2[:, s])
+            if s == 0:
+                to_own = (inc == 0.0) | ~inner                       # literal: the target of the whole face block
+        if literal:
+            diag[to_own] += (own + nbr)[to_own]
+            off[f, ~to_own] += (own + nbr)[~to_own]
+        else:
+            diag += own
+            diag[~inner] += nbr[~inner]
+            off[f, inner] += nbr[inner]
+        if k != 0.0:
+            nb = np.maximum(q - 1, 0)
+            dx = np.where(inner, np.linalg.norm(cen - cen[nb], axis=1),
+                          np.linalg.norm(cen - 0.5 * (G.X[:, l1] + G.X[:, l2]), axis=1))
+            kd = (k / dx) * G.sdet[:, f]
+            diag += kd[:, None, None] * sum(np.outer(sn[s], sn[s]) for s in range(2))
+            pen = -kd[:, None, None] * sum(np.einsum("i,ej->eij", sn[s], sn2[:, s]) for s in range(2))
+            off[f, inner] += pen[inner]
+    re = [ar] + [ar[G.neig[:, f] != 0] for f in range(3)]
+    ce = [ar] + [G.neig[G.neig[:, f] != 0, f] - 1 for f in range(3)]
+    vb = [diag] + [off[f, G.neig[:, f] != 0] for f in range(3)]
+    N = 3 * E
+    return _assemble(np.concatenate(re), np.concatenate(ce), np.concatenate(vb), N, sparse), _assemble(ar, ar, m, N, sparse)
 
 
-def _assemble(blocks, N, sparse):
+def _assemble(re, ce, v, N, sparse):
+    """(3E)^2 matrix, dense or scipy CSR, of the 3x3 blocks v[i] at block (re[i], ce[i]); repeated blocks add up."""
+    r = np.broadcast_to((3 * re)[:, None, None] + np.arange(3)[None, :, None], v.shape).ravel()
+    c = np.broadcast_to((3 * ce)[:, None, None] + np.arange(3)[None, None, :], v.shape).ravel()
     if not sparse:
         A = np.zeros((N, N))
-        for (e, c), b in blocks.items():
-            A[3 * e: 3 * e + 3, 3 * c: 3 * c + 3] += b
+        np.add.at(A, (r, c), v.ravel())
         return A
     import scipy.sparse as sp
-    keys = list(blocks)
-    r = np.array([e for e, _ in keys])[:, None, None] * 3 + np.arange(3)[None, :, None]
-    c = np.array([c for _, c in keys])[:, None, None] * 3 + np.arange(3)[None, None, :]
-    v = np.array([blocks[key] for key in keys])
-    return sp.csr_matrix((v.ravel(), (np.broadcast_to(r, v.shape).ravel(), np.broadcast_to(c, v.shape).ravel())), shape=(N, N))
+    return sp.csr_matrix((v.ravel(), (r, c)), shape=(N, N))
 
 
 def stab(X, u, tnew, told, dt):
@@ -253,10 +250,6 @@ def implicit_solve(X, neig, fneig, u, T, dt, ntime, nits, use_dir=True, with_sta
 def bsr_to_dense(val, col, sparse=False):
     """(val[E,4,3,3], col[E,4]) of pamg_implicit_get_bsr -> (3E)^2, dense or scipy CSR."""
     E = val.shape[0]
-    blocks = {}
-    for e in range(E):
-        for b in range(4):
-            c = int(col[e, b])
-            if c >= 0:
-                blocks[(e, c)] = blocks.get((e, c), 0.0) + val[e, b]
-    return _assemble(blocks, 3 * E, sparse)
+    ok = np.asarray(col) >= 0
+    re = np.broadcast_to(np.arange(E)[:, None], ok.shape)[ok]
+    return _assemble(re, np.asarray(col)[ok].astype(np.int64), np.asarray(val)[ok], 3 * E, sparse)
